@@ -28,6 +28,12 @@ the seed changes per step).
              the HBM view (algorithmic queue bytes) and the FP32 view (SURVEY 8(d) flop model) ride along.
   cpu_baseline / --impl reference : oracle/ (f64 C++ port of the reference, octree traversal, live NEE) on the
              host cores, bounded sample of the same frame.
+
+--dump-outputs DIR (rtb200 arm): after the timed steps, rank 0 writes the RGB8 frame of the last timed step, in scan-line
+order, as DIR/frame.npy (float32 [height, width, 3]).  A frame above 64 MB in float32 (the N > 1 frame) is written as a
+fixed seeded sample of its pixels instead: DIR/frame_pixels.npy (float64 flat pixel indices y * width + x, ascending) and
+DIR/frame_sample.npy (float32 [n, 3]).  The scene and the per-step seeds depend only on the arguments, so two builds run
+with the same arguments can be compared output for output (up to the last-level rounding of float atomics).
 """
 from __future__ import annotations
 
@@ -57,6 +63,8 @@ UNIT = "samples/s"
 SHADE_B_VERTEX, SHADE_B_EXT, SHADE_B_SHQ, SHADE_B_RED = 56.0, 56.0, 48.0, 16.0
 TRAV_B_EXT, TRAV_B_SH = 48.0, 64.0
 STRONG_FRAME = (3840, 2160, 256)     # the fixed frame of the N > 1 runs
+DUMP_BYTES = 64 << 20                # budget of --dump-outputs
+DUMP_SAMPLE_PIXELS = 1 << 21         # pixels kept from a frame over budget: 2 Mi x (12 + 8) B = 40 MB
 
 
 def workload(n_gpus: int):
@@ -150,7 +158,7 @@ def run_reference(args):
     if rank != 0:
         return 0
     wl = workload(args.gpus)
-    steps = max(1, args.steps)
+    steps = args.steps
     per_step = max(3.0, min(20.0, 90.0 / (steps + args.warmup)))
     if os.environ.get("RTB_BENCH_CPU_SECONDS"):   # test hook (tests/test_bench_contract.py): a shorter CPU sample
         per_step = float(os.environ["RTB_BENCH_CPU_SECONDS"])
@@ -184,6 +192,20 @@ def psnr(a, b):
 
     mse = np.mean((a.astype(np.float64) - b.astype(np.float64)) ** 2)
     return 99.0 if mse == 0 else float(10 * np.log10(255.0 ** 2 / mse))
+
+
+def dump_frame(out_dir, frame):
+    """--dump-outputs: frame (uint8 [h, w, 3], scan-line order) -> out_dir/frame.npy, or a seeded pixel sample when over budget."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    if frame.size * 4 <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, "frame.npy"), frame.astype(np.float32))
+        return
+    px = frame.reshape(-1, 3)
+    idx = np.sort(np.random.default_rng(0).choice(px.shape[0], DUMP_SAMPLE_PIXELS, replace=False))
+    np.save(os.path.join(out_dir, "frame_pixels.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "frame_sample.npy"), px[idx].astype(np.float32))
 
 
 def measure_configs(R, device, full_c4=True):
@@ -288,7 +310,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the configs / scaling_reference / weak / c4_full blocks")
     ap.add_argument("--spp", type=int, default=0, help="override spp (debug only; invalidates the bench line)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step to DIR (rtb200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the rtb200 arm (the reference arm renders a timing-sized row sample)")
     _stdout_for_json_only()
     if args.impl == "reference":
         return run_reference(args)
@@ -419,6 +446,9 @@ def main():
         clocks.start()
     elapsed, job, totals = timed(fr, SPP, args.steps, 0, 1000 + args.warmup)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # before anything else renders into fr
+        dump_frame(args.dump_outputs, fr.frame.cpu().numpy() if world > 1 else
+                   sharding.untile_numpy(fr.shard.cpu().numpy()[None], W, H, 1))
     value = job["samples"] / elapsed
     rays = job["rays_primary"] + job["rays_extension"] + job["rays_shadow"]
 

@@ -29,6 +29,35 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert p.returncode == 0 and p.stdout.strip() == ""
 
 
+def test_steps_and_dump_arguments_are_checked(tmp_path):
+    # no step count is silently replaced; the reference arm's row sample is sized by timing, so it has no reproducible output
+    for extra in (["--steps", "0"], ["--impl", "reference", "--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120, cwd=tmp_path)
+        assert p.returncode == 2 and p.stdout == "" and list(tmp_path.iterdir()) == [], extra
+
+
+def test_dump_of_a_large_frame_is_a_fixed_sample(tmp_path):
+    # the N > 1 frame (3840x2160) is over the 64 MB budget in float32: the same seeded pixel sample on every run
+    import numpy as np
+
+    import bench
+
+    frame = np.random.default_rng(1).integers(0, 256, (2160, 3840, 3), dtype=np.uint8)
+    for d in ("a", "b"):
+        bench.dump_frame(str(tmp_path / d), frame)
+    assert sorted(os.listdir(tmp_path / "a")) == ["frame_pixels.npy", "frame_sample.npy"]
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64 << 20
+    idx, px = np.load(tmp_path / "a" / "frame_pixels.npy"), np.load(tmp_path / "a" / "frame_sample.npy")
+    assert idx.dtype == np.float64 and px.dtype == np.float32 and px.shape == (idx.size, 3)
+    assert (np.diff(idx) > 0).all() and idx[0] >= 0 and idx[-1] < 3840 * 2160
+    assert np.array_equal(px, frame.reshape(-1, 3)[idx.astype(np.int64)])
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "frame_pixels.npy"))
+    small = frame[:1080, :1920]
+    bench.dump_frame(str(tmp_path / "c"), small)
+    assert sorted(os.listdir(tmp_path / "c")) == ["frame.npy"]
+    assert np.array_equal(np.load(tmp_path / "c" / "frame.npy"), small.astype(np.float32))
+
+
 import pytest
 
 
@@ -49,3 +78,20 @@ def test_rtb200_arm_line_has_the_contract_keys():
     r = d["roofline"]
     assert r["bound"] == "issue" and 0 < r["frac"] < 1 and abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-9 and r["traffic"] > 0
     assert set(d["config"]) >= {"workload", "width", "height", "spp"}
+
+
+@pytest.mark.gpu
+def test_rtb200_arm_dumps_the_last_timed_frame(gpu_scene, tmp_path):
+    # timed step i renders seed 1000 + warmup + i; the dump is the last one's RGB8 frame, untiled into scan-line order
+    import numpy as np
+
+    out = tmp_path / "dump"
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--spp", "8", "--no-configs", "--no-cpu-baseline",
+                        "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+    assert p.returncode == 0, p.stderr[-2000:]
+    assert json.loads(p.stdout)["steps"] == 2
+    assert os.listdir(out) == ["frame.npy"]
+    got = np.load(out / "frame.npy")
+    assert got.dtype == np.float32 and got.shape == (1080, 1920, 3)
+    want = gpu_scene("flying_unicorn").render(1920, 1080, 8, seed=1000 + 1 + 1)
+    assert np.abs(got - want).max() <= 1
