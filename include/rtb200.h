@@ -207,6 +207,33 @@ const char* rtb_last_error(void);
  * RTB_ECANCELLED if it became non-zero (src/server.rs:170, 198). */
 int rtb_render(rtb_scene* scene, const rtb_params* params, uint8_t* rgb8_out, volatile int* cancel);
 
+/* ---- adaptive sampling (not in the reference): stop rendering a 32x32 tile once its noise is below a target ----------
+ * params.spp is the BUDGET.  Passes add pass_spp samples per pixel to every tile still active; pass p covers the samples
+ * ks in [p * pass_spp, (p + 1) * pass_spp) of the budget frame's numbering (sample id sub * (spp/4) + k, ks = 4k + sub),
+ * exactly like pass p of a progressive job with passes = spp / pass_spp.  A tile that received n samples per pixel
+ * therefore holds a PREFIX of the budget frame's samples and is resolved with n (the bytes of that progressive job's
+ * pass n / pass_spp - 1, up to the order of the fp32 sums).
+ * Statistic, per pixel after every pass: for each sub-pixel s the pass's mean luminance
+ * m_s = clamp01((lum(S_s) - lum_prev_s) / (pass_spp / 4)) (S_s = the sub-pixel's rgb sums, lum = Rec. 709 weights on
+ * linear rgb), the batch value m = 0.25 * sum_s m_s, and a Welford (mean, M2) over the tile's B passes.  Error in 8-bit
+ * output levels, after gamma_correct: mu = clamp01(mean), sigma = sqrt(M2 / (B - 1) / B) (standard error of the mean),
+ * err = 255 * (min(mu + sigma, 1)^(1/2.2) - mu^(1/2.2)).
+ * A tile stays active while it has fewer than spp samples per pixel AND (fewer than min_spp OR the max of err over its
+ * in-frame pixels > target_levels).  target_levels = 0 never stops a tile early: the result is the uniform frame.
+ * Decisions are not bit-reproducible: the fp32 sums depend on the order of atomics, so a tile right at the threshold may
+ * get one pass more or fewer from run to run.  Whole frames only (world = 1).  Invalid options give RTB_EINVAL with a
+ * message naming the field. */
+typedef struct rtb_adaptive {
+    float target_levels; /* stop a 32x32 tile once every pixel's estimated standard error is <= this many 8-bit output levels; 0 = never */
+    int32_t pass_spp;    /* samples per pixel per pass (multiple of 4); params.spp (the budget) must be a multiple of it */
+    int32_t min_spp;     /* no tile stops before this many samples per pixel (multiple of pass_spp, >= 2 passes) */
+    int32_t reserved;    /* 0 */
+} rtb_adaptive;
+/* tile_spp / tile_error (optional): tiles_y*tiles_x entries, tile (tx, ty) at ty*tiles_x + tx — the samples per pixel the
+ * tile received and its err after its last pass.  rgb8_out and `cancel` as for rtb_render. */
+int rtb_render_adaptive(rtb_scene* scene, const rtb_params* params, const rtb_adaptive* opts, uint8_t* rgb8_out,
+                        int32_t* tile_spp, float* tile_error, volatile int* cancel);
+
 /* device-resident variants (bench `value`, multi-GPU gather): the result stays in device memory
  * owned by the caller.  d_rgb8_tiles receives this rank's pixels in tile order
  * (rtb_local_pixels() * 3 bytes); d_subpixel_sums (optional) receives the fp32 sums of the four
@@ -239,6 +266,10 @@ int rtb_get_stats(const rtb_scene* scene, rtb_stats* stats);
  * per pass with the running estimate; pass n + 1 renders while pass n is copied and consumed.
  * One consumer thread per job. */
 int rtb_job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, rtb_job** out);
+/* adaptive form (see rtb_adaptive): a progressive job whose tiles stop once converged.  Every pass re-sends the whole frame
+ * like progressive mode; at most spp / pass_spp passes, and the job is complete (not cancelled) as soon as no tile is left
+ * active, which may be earlier. */
+int rtb_job_begin_adaptive(rtb_scene* scene, const rtb_params* params, const rtb_adaptive* opts, rtb_job** out);
 int rtb_job_next(rtb_job* job, uint16_t* x, uint16_t* y, uint8_t* n, uint8_t* rgb /* >= 180 bytes */);
 /* bulk form: up to max_records records packed exactly like the reference's binary messages,
  * [0]=0 type, [1]=n, [2..4]=x u16le, [4..6]=y u16le, then n*(r,g,b) (src/server.rs:173-190);

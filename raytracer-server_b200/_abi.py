@@ -35,6 +35,10 @@ class Params(C.Structure):
                 ("accel", C.c_int32), ("tuning", C.c_int32 * 4)]
 
 
+class Adaptive(C.Structure):
+    _fields_ = [("target_levels", C.c_float), ("pass_spp", C.c_int32), ("min_spp", C.c_int32), ("reserved", C.c_int32)]
+
+
 class SceneInfo(C.Structure):
     _fields_ = [("n_objects", C.c_int32), ("n_planes", C.c_int32), ("n_spheres", C.c_int32), ("n_meshes", C.c_int32),
                 ("n_triangles", C.c_int32), ("light_object", C.c_int32), ("bvh_nodes", C.c_int32),
@@ -79,6 +83,7 @@ EXPORTS = [
     "rtb_untile_device", "rtb_get_stats", "rtb_job_begin", "rtb_job_next", "rtb_job_next_messages", "rtb_job_next_frame", "rtb_job_cancel",
     "rtb_job_end", "rtb_trace_primary", "rtb_trace_rays", "rtb_sample_radiance", "rtb_fp32_peak",
     "rtb_untile_device_async", "rtb_job_stats", "rtb_sample_pixels", "rtb_trace_rays_accel", "rtb_scene_octree_stats", "rtb_scene_export", "rtb_scene_import",
+    "rtb_render_adaptive", "rtb_job_begin_adaptive",
 ]
 
 _lib = None
@@ -113,6 +118,8 @@ def lib():
     L.rtb_untile_device.argtypes = [C.POINTER(Params), vp, C.c_int64, vp, C.c_int]
     L.rtb_get_stats.argtypes = [vp, C.POINTER(Stats)]
     L.rtb_job_begin.argtypes = [vp, C.POINTER(Params), C.c_int32, C.POINTER(vp)]
+    L.rtb_render_adaptive.argtypes = [vp, C.POINTER(Params), C.POINTER(Adaptive), C.POINTER(C.c_uint8), ip, fp, ip]
+    L.rtb_job_begin_adaptive.argtypes = [vp, C.POINTER(Params), C.POINTER(Adaptive), C.POINTER(vp)]
     L.rtb_job_next.argtypes = [vp, C.POINTER(C.c_uint16), C.POINTER(C.c_uint16), C.POINTER(C.c_uint8),
                                C.POINTER(C.c_uint8)]
     L.rtb_job_next_messages.argtypes = [vp, C.POINTER(C.c_uint8), C.c_int64, C.c_int32, C.POINTER(C.c_int64)]

@@ -8,10 +8,12 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <condition_variable>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -85,12 +87,23 @@ struct RenderContext {
                          // SAH tree (51 registers, a few spills, 40 warps per SM): bench frame 540.4 -> 537.0 ms; on the PLOC tree 4 was ahead
     int grid_oct = 0;    // k_traverse_octree's own persistent grid
     int grid_ext = 0, grid_ext_count = 0, grid_sh = 0, grid_sh_count = 0, grid_gen = 0, grid_shade = 0, grid_bin = 0;
+    // adaptive sampling (ensure_adaptive): allocated by the first adaptive request only
+    float2* ad_mom = nullptr;          // [pixel] (mean, M2)
+    size_t ad_mom_cap = 0;
+    int32_t* ad_list = nullptr;        // [tile] the active tiles, ascending
+    uint32_t* ad_tile_ks = nullptr;    // [tile] samples per pixel so far
+    float* ad_tile_err = nullptr;      // [tile] error estimate after the tile's latest pass
+    int ad_tiles_cap = 0;
+    volatile int* h_ad_count = nullptr;   // mapped pinned: active tiles after k_compact_tiles
+    int* d_ad_count = nullptr;
 
     ~RenderContext() {
         cudaSetDevice(device);
         if (stream) cudaStreamSynchronize(stream);
         cudaFree(qbuf); cudaFree(sbuf); cudaFree(accum); cudaFree(ctrl); cudaFree(d_rgb); cudaFree(d_probe);
         cudaFree(bin_buf); cudaFree(bin_hist);
+        cudaFree(ad_mom); cudaFree(ad_list); cudaFree(ad_tile_ks); cudaFree(ad_tile_err);
+        if (h_ad_count) cudaFreeHost((void*)h_ad_count);
         if (h_active) cudaFreeHost(h_active);
         if (h_state) cudaFreeHost((void*)h_state);
         for (auto& e : graph_exec) if (e) cudaGraphExecDestroy(e);
@@ -1037,6 +1050,90 @@ int ensure_rgb(RenderContext* c, size_t bytes, bool host) {
     return RTB_OK;
 }
 
+// ---------------------------------------------------------------- adaptive sampling
+// host-side checks only (a host-only scene reaches them): the error names the offending field
+int check_adaptive(const rtb_params* p, const rtb_adaptive* o) {
+    if (!o) return fail(RTB_EINVAL, "rtb_adaptive options are NULL");
+    if (!std::isfinite(o->target_levels) || o->target_levels < 0.f) return fail(RTB_EINVAL, "rtb_adaptive.target_levels must be finite and >= 0");
+    if (o->pass_spp <= 0 || o->pass_spp % 4 != 0) return fail(RTB_EINVAL, "rtb_adaptive.pass_spp must be a positive multiple of 4");
+    if (p->spp % o->pass_spp != 0) return fail(RTB_EINVAL, "params.spp (the budget) must be a multiple of rtb_adaptive.pass_spp");
+    if (o->min_spp % o->pass_spp != 0 || o->min_spp < 2 * o->pass_spp || o->min_spp > p->spp)
+        return fail(RTB_EINVAL, "rtb_adaptive.min_spp must be a multiple of pass_spp in [2 * pass_spp, spp]");
+    if (o->reserved != 0) return fail(RTB_EINVAL, "rtb_adaptive.reserved must be 0");
+    if (p->world != 1) return fail(RTB_EINVAL, "adaptive rendering renders whole frames (params.world must be 1)");
+    return RTB_OK;
+}
+
+// path slots of one pass over the whole frame (later passes hold fewer tiles)
+uint32_t adaptive_pool(const rtb_params* p, const rtb_adaptive* o) {
+    return pool_for((uint64_t)local_tiles(p) * 1024ull * (uint64_t)o->pass_spp, p->pool_paths);
+}
+
+int ensure_adaptive(RenderContext* c, int n_tiles, size_t pixels) {
+    if (!c->h_ad_count) {
+        CU_TRY(cudaHostAlloc((void**)&c->h_ad_count, sizeof(int), cudaHostAllocMapped));
+        CU_TRY(cudaHostGetDevicePointer((void**)&c->d_ad_count, (void*)c->h_ad_count, 0));
+    }
+    if (c->ad_mom_cap < pixels) {
+        cudaFree(c->ad_mom);
+        c->ad_mom = nullptr;
+        c->ad_mom_cap = 0;
+        CU_TRY(cudaMalloc((void**)&c->ad_mom, pixels * sizeof(float2)));
+        c->ad_mom_cap = pixels;
+    }
+    if (c->ad_tiles_cap < n_tiles) {
+        cudaFree(c->ad_list); cudaFree(c->ad_tile_ks); cudaFree(c->ad_tile_err);
+        c->ad_list = nullptr; c->ad_tile_ks = nullptr; c->ad_tile_err = nullptr;
+        c->ad_tiles_cap = 0;
+        CU_TRY(cudaMalloc((void**)&c->ad_list, (size_t)n_tiles * sizeof(int32_t)));
+        CU_TRY(cudaMalloc((void**)&c->ad_tile_ks, (size_t)n_tiles * sizeof(uint32_t)));
+        CU_TRY(cudaMalloc((void**)&c->ad_tile_err, (size_t)n_tiles * sizeof(float)));
+        c->ad_tiles_cap = n_tiles;
+    }
+    return RTB_OK;
+}
+
+void add_stats(rtb_stats& d, const rtb_stats& s);
+
+// The adaptive pass loop (world = 1): clears the accumulators, then renders pass after pass — samples
+// [pass * pass_spp, (pass + 1) * pass_spp) of the budget frame's numbering, so a tile's samples are a prefix of the budget
+// frame's — over the tiles still in the list, until none is left.  `after_pass` (may be empty) runs once per pass with that
+// pass's counters, once k_adapt has advanced tile_ks.  On return a.tile_ks holds the per-tile sample counts for k_resolve.
+int run_adaptive(rtb_scene* sc, RenderContext* c, RenderArgs& a, const rtb_adaptive& o, volatile int* cancel, rtb_stats& st,
+                 bool& cancelled, const std::function<int(int, const rtb_stats&)>& after_pass) {
+    const int n_tiles = a.tiles_x * a.tiles_y;
+    const size_t pixels = (size_t)a.width * a.height;
+    int rc = ensure_adaptive(c, n_tiles, pixels);
+    if (rc != RTB_OK) return rc;
+    AdaptArgs ad{c->accum, c->ad_mom, c->ad_list, c->ad_tile_ks, c->ad_tile_err, a.width, a.height, a.tiles_x,
+                 o.pass_spp, a.spp, o.min_spp, o.target_levels};
+    CU_TRY(cudaMemsetAsync(c->accum, 0, pixels * 4 * sizeof(float4), c->stream));
+    CU_TRY(cudaMemsetAsync(c->ad_mom, 0, pixels * sizeof(float2), c->stream));
+    k_adapt_init<<<(n_tiles + 255) / 256, 256, 0, c->stream>>>(ad, n_tiles);
+    st.kernel_launches += 1;
+    RenderArgs r = a;   // the list pointer stays the same from pass to pass: run_wavefront's captured graphs are re-used
+    r.tile_base = 0;
+    r.tile_list = c->ad_list;
+    cancelled = false;
+    for (int pass = 0, count = n_tiles; count > 0; ++pass) {
+        const uint32_t k0 = (uint32_t)pass * (uint32_t)o.pass_spp;
+        r.n_local_tiles = count;
+        rtb_stats ps{};
+        rc = run_wavefront(sc, c, r, k0, k0 + (uint32_t)o.pass_spp, false, cancel, ps, cancelled);
+        if (rc != RTB_OK || cancelled) return rc;
+        k_adapt<<<count, ADAPT_THREADS, 0, c->stream>>>(ad);
+        k_compact_tiles<<<1, COMPACT_THREADS, 0, c->stream>>>(c->ad_list, count, c->d_ad_count);
+        CU_TRY(cudaStreamSynchronize(c->stream));
+        CU_TRY(cudaGetLastError());
+        count = *c->h_ad_count;
+        ps.kernel_launches += 2;
+        add_stats(st, ps);
+        if (after_pass && (rc = after_pass(pass, ps)) != RTB_OK) return rc;
+    }
+    a.tile_ks = c->ad_tile_ks;
+    return RTB_OK;
+}
+
 }  // namespace
 
 // ======================================================================================= C ABI
@@ -1377,6 +1474,43 @@ int rtb_render(rtb_scene* scene, const rtb_params* params, uint8_t* rgb8_out, vo
     return cancelled ? RTB_ECANCELLED : RTB_OK;
 }
 
+int rtb_render_adaptive(rtb_scene* scene, const rtb_params* params, const rtb_adaptive* opts, uint8_t* rgb8_out, int32_t* tile_spp,
+                        float* tile_error, volatile int* cancel) {
+    if (!scene || !rgb8_out) return fail(RTB_EINVAL, "NULL argument");
+    int rc = check_params(params);
+    if (rc == RTB_OK) rc = check_adaptive(params, opts);
+    if (rc != RTB_OK) return rc;
+    if ((rc = need_device(scene)) != RTB_OK) return rc;
+    if ((rc = need_accel(scene, params)) != RTB_OK) return rc;
+    const uint32_t P = adaptive_pool(params, opts);
+    const uint32_t SP = params->estimator == RTB_EST_NEE ? P : 2 * P;
+    const size_t frame = (size_t)params->width * params->height * 3;
+    const int n_tiles = local_tiles(params);
+    RenderContext* c = acquire_context(scene, P);
+    RenderArgs a;
+    rtb_stats st{};
+    bool cancelled = false;
+    rc = ensure_context(scene, c, P, SP, (size_t)params->width * params->height * 4, requested_bin_bits(scene, params) > 0);
+    if (rc == RTB_OK) {
+        fill_args(scene, params, c, a);
+        rc = run_adaptive(scene, c, a, *opts, cancel, st, cancelled, {});
+    }
+    if (rc == RTB_OK && !cancelled) rc = ensure_rgb(c, frame, true);
+    if (rc == RTB_OK && !cancelled) rc = resolve_to(c, a, c->d_rgb, nullptr, 1, st);
+    if (rc == RTB_OK && !cancelled) {
+        cudaError_t e = cudaMemcpyAsync(c->h_rgb, c->d_rgb, frame, cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess && tile_spp) e = cudaMemcpyAsync(tile_spp, c->ad_tile_ks, (size_t)n_tiles * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess && tile_error) e = cudaMemcpyAsync(tile_error, c->ad_tile_err, (size_t)n_tiles * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+        if (e != cudaSuccess) rc = fail(RTB_ECUDA, std::string("frame read-back: ") + cudaGetErrorString(e));
+        else std::memcpy(rgb8_out, c->h_rgb, frame);
+    }
+    publish_stats(scene, st);
+    release_context(scene, c);
+    if (rc != RTB_OK) return rc;
+    return cancelled ? RTB_ECANCELLED : RTB_OK;
+}
+
 int rtb_untile_device_async(const rtb_params* params, const void* d_shards, int64_t shard_stride, void* d_rgb8_frame, int device,
                             void* cuda_stream) {
     int rc = check_params(params);
@@ -1642,6 +1776,8 @@ struct rtb_job {
     rtb_scene* scene = nullptr;
     rtb_params params{};
     int passes = 1;
+    rtb_adaptive adaptive{};   // pass_spp > 0: adaptive job (passes = the most the budget allows; the device decides how many run)
+    bool converged = false;    // adaptive job: no tile was left active, the frame is final (guarded by mu)
     std::vector<std::thread> workers;
     std::mutex mu;
     std::condition_variable cv;
@@ -1790,6 +1926,41 @@ void job_worker(rtb_job* j, int worker) {
     // progressive: one band = the frame; pass n + 1 renders while pass n is copied and consumed
     a.tile_base = 0;
     a.n_local_tiles = tiles_x * tiles_y;
+    // resolves pass `pass` (sample counts as `r` gives them) into the pinned frame of its parity and publishes it
+    auto publish = [&](int pass, const rtb_stats& ps, const RenderArgs& r) -> int {
+        const int b = pass & 1;
+        {   // the pinned frame of this parity must have been consumed (passes stay in order, memory stays bounded)
+            std::unique_lock<std::mutex> lk(j->mu);
+            j->cv.wait(lk, [&] { return j->buf_pass[b] < 0 || j->cancel; });
+            if (j->cancel) return RTB_ECANCELLED;
+            add_stats(j->stats, ps);
+        }
+        const int n = a.n_local_tiles * 1024;
+        k_resolve<<<(n + 255) / 256, 256, 0, c->stream>>>(r, c->d_rgb + (size_t)b * frame, nullptr, 1);   // in stream order: before the next pass adds samples
+        cudaError_t e = cudaEventRecord(j->ev_resolved[b], c->stream);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(c->copy_stream, j->ev_resolved[b], 0);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(j->h_frame[b], c->d_rgb + (size_t)b * frame, frame, cudaMemcpyDeviceToHost, c->copy_stream);
+        if (e == cudaSuccess) e = cudaEventRecord(j->pass_copied[b], c->copy_stream);
+        if (e != cudaSuccess) return fail(RTB_ECUDA, std::string("streaming job: ") + cudaGetErrorString(e));
+        publish_pass(j, pass, b);
+        return RTB_OK;
+    };
+    if (j->adaptive.pass_spp > 0) {
+        rtb_stats total{};
+        bool cancelled = false;
+        rc = run_adaptive(sc, c, a, j->adaptive, &j->cancel, total, cancelled, [&](int pass, const rtb_stats& ps) {
+            RenderArgs r = a;
+            r.tile_ks = c->ad_tile_ks;   // every tile resolved with its own sample count
+            return publish(pass, ps, r);
+        });
+        if (rc != RTB_OK) return finish(rc);
+        if (cancelled || j->cancel) return finish(RTB_ECANCELLED);
+        {
+            std::lock_guard<std::mutex> lk(j->mu);
+            j->converged = true;
+        }
+        return finish(RTB_OK);
+    }
     if (cudaError_t e = cudaMemsetAsync(c->accum, 0, accum_elems * sizeof(float4), c->stream); e != cudaSuccess) return cuda_fail(e);
     const int passes = j->passes;
     for (int pass = 0; pass < passes; ++pass) {
@@ -1801,23 +1972,9 @@ void job_worker(rtb_job* j, int worker) {
             if (rc != RTB_OK) return finish(rc);
         }
         if (cancelled || j->cancel) return finish(RTB_ECANCELLED);
-        const int b = pass & 1;
-        {   // the pinned frame of this parity must have been consumed (passes stay in order, memory stays bounded)
-            std::unique_lock<std::mutex> lk(j->mu);
-            j->cv.wait(lk, [&] { return j->buf_pass[b] < 0 || j->cancel; });
-            if (j->cancel) { lk.unlock(); return finish(RTB_ECANCELLED); }
-            add_stats(j->stats, ps);
-        }
         RenderArgs r = a;
         r.ks_done = k1;   // resolve with the per-sub-pixel sample counts reached so far
-        const int n = a.n_local_tiles * 1024;
-        k_resolve<<<(n + 255) / 256, 256, 0, c->stream>>>(r, c->d_rgb + (size_t)b * frame, nullptr, 1);   // in stream order: before the next pass adds samples
-        cudaError_t e = cudaEventRecord(j->ev_resolved[b], c->stream);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(c->copy_stream, j->ev_resolved[b], 0);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(j->h_frame[b], c->d_rgb + (size_t)b * frame, frame, cudaMemcpyDeviceToHost, c->copy_stream);
-        if (e == cudaSuccess) e = cudaEventRecord(j->pass_copied[b], c->copy_stream);
-        if (e != cudaSuccess) return cuda_fail(e);
-        publish_pass(j, pass, b);
+        if ((rc = publish(pass, ps, r)) != RTB_OK) return finish(rc);
     }
     finish(RTB_OK);
 }
@@ -1894,11 +2051,8 @@ int job_next_record(rtb_job* job, bool block, uint16_t* x, uint16_t* y, uint8_t*
     return 1;
 }
 
-}  // namespace
-
-extern "C" {
-
-int rtb_job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, rtb_job** out) {
+// adaptive: nullptr for a uniform job; otherwise checked options (check_adaptive) and passes = spp / pass_spp
+int job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, const rtb_adaptive* adaptive, rtb_job** out) {
     if (!scene || !out) return fail(RTB_EINVAL, "NULL argument");
     if (int rc0 = need_device(scene)) return rc0;
     int rc = check_params(params);
@@ -1910,6 +2064,7 @@ int rtb_job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, rt
     j->scene = scene;
     j->params = *params;
     j->passes = std::max(1, passes);
+    if (adaptive) j->adaptive = *adaptive;
     j->frame_bytes = (size_t)params->width * params->height * 3;
     j->stats.first_record_ms = -1.0;
     const bool progressive = j->passes > 1;
@@ -1957,6 +2112,22 @@ int rtb_job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, rt
     for (int w = 0; w < n_workers; ++w) j->workers.emplace_back(job_worker, j, w);
     *out = j;
     return RTB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rtb_job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, rtb_job** out) {
+    return job_begin(scene, params, passes, nullptr, out);
+}
+
+int rtb_job_begin_adaptive(rtb_scene* scene, const rtb_params* params, const rtb_adaptive* opts, rtb_job** out) {
+    if (!scene || !out) return fail(RTB_EINVAL, "NULL argument");
+    int rc = check_params(params);
+    if (rc == RTB_OK) rc = check_adaptive(params, opts);
+    if (rc != RTB_OK) return rc;
+    return job_begin(scene, params, params->spp / opts->pass_spp, opts, out);
 }
 
 // returns 1 = record produced, 0 = frame(s) complete, RTB_ESTOPPED after a cancel, or another negative error
@@ -2035,7 +2206,7 @@ int rtb_job_end(rtb_job* job) {
         job->cv.notify_all();
     }
     for (auto& t : job->workers) if (t.joinable()) t.join();
-    bool complete = job->passes > 1 ? job->passes_done >= job->passes : true;
+    bool complete = job->passes > 1 ? job->passes_done >= job->passes || job->converged : true;
     for (char d : job->band_done) complete = complete && (job->passes > 1 || d);
     const int was_cancelled = job->cancel && job->error == RTB_OK && !complete;
     cudaSetDevice(job->scene->device);

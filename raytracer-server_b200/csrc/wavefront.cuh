@@ -19,6 +19,7 @@
 // warp-aggregated atomics; k_extend only visits the front part.
 #pragma once
 
+#include "adaptive_rule.cuh"
 #include "intersect.cuh"
 #include "octree.cuh"
 #include "shade.cuh"
@@ -94,6 +95,8 @@ struct RenderArgs {
     int estimator;
     int rank, world, tiles_x, tiles_y, n_local_tiles;
     int tile_base;       // first LOCAL tile of this launch series (streaming jobs render a frame band by band; 0 = whole shard)
+    const int32_t* tile_list;   // adaptive passes (world = 1): k_generate's local tile lt is tile tile_list[lt]; nullptr = lt + tile_base
+    const uint32_t* tile_ks;    // adaptive resolve: ks_done per tile (indexed by tile); nullptr = ks_done for every tile
     uint32_t P, SP;          // most paths / shadow rays alive at once
     uint32_t Pcap, SPcap;    // physical slots per queue: P, SP + room for the unfilled tails of k_shade's per-warp segments
     PathQueue q[2];
@@ -254,7 +257,9 @@ __global__ void __launch_bounds__(WF_THREADS) k_generate(const __grid_constant__
                     y = a.probe_py[lp];
                     acc = (uint32_t)lp * 4u + (uint32_t)sub;
                 } else {
-                    valid = local_to_xy(lp + C->tile_base * 1024, a.rank, a.world, a.tiles_x, a.width, a.height, x, y);
+                    const int lt = lp >> 10;
+                    const int t = a.tile_list ? a.tile_list[lt] : lt + C->tile_base;
+                    valid = local_to_xy(t * 1024 + (lp & 1023), a.rank, a.world, a.tiles_x, a.width, a.height, x, y);
                     acc = (uint32_t)(y * a.width + x) * 4u + (uint32_t)sub;
                 }
                 sample = sub * a.num_samples + k;
@@ -1300,9 +1305,10 @@ __global__ void k_resolve(RenderArgs a, unsigned char* __restrict__ out_rgb8, fl
     float3 px = f3(0.f, 0.f, 0.f);
     if (in) {
         uint32_t p = (uint32_t)(y * a.width + x);
+        const uint32_t ks_done = a.tile_ks ? a.tile_ks[(lp >> 10) + a.tile_base] : a.ks_done;
         for (int s = 0; s < 4; ++s) {
             // sub-pixel s has received the samples ks < ks_done with ks % 4 == s
-            uint32_t cnt = a.ks_done > (uint32_t)s ? (a.ks_done - (uint32_t)s + 3u) / 4u : 0u;
+            uint32_t cnt = ks_done > (uint32_t)s ? (ks_done - (uint32_t)s + 3u) / 4u : 0u;
             float inv = cnt ? 1.0f / (float)cnt : 0.0f;
             float4 v = a.accum[p * 4u + s];
             if (out_sub) out_sub[(size_t)lp * 4 + s] = make_float4(v.x * inv, v.y * inv, v.z * inv, 0.f);
@@ -1342,6 +1348,92 @@ __global__ void k_resolve_list(const float4* __restrict__ accum, int n, int num_
     out3[3 * i] = powf(clamp01_keep_nan(px.x), 1.0f / 2.2f) * 255.0f + 0.5f;
     out3[3 * i + 1] = powf(clamp01_keep_nan(px.y), 1.0f / 2.2f) * 255.0f + 0.5f;
     out3[3 * i + 2] = powf(clamp01_keep_nan(px.z), 1.0f / 2.2f) * 255.0f + 0.5f;
+}
+
+// ---------------------------------------------------------------- adaptive sampling (world = 1)
+// A pass renders the tiles of `list` (ascending tile order); k_adapt then updates every pixel's statistic (adapt_pixel),
+// decides per tile whether it goes on, and k_compact_tiles squeezes the tiles that stopped out of the list.
+struct AdaptArgs {
+    float4* accum;       // [pixel*4 + sub]: .w holds lum709 of the sums after the previous pass
+    float2* mom;         // [pixel]: (mean, M2) of the batch values
+    int32_t* list;       // the pass's tiles; k_adapt marks a tile that stops with -1
+    uint32_t* tile_ks;   // [tile]: samples per pixel so far (= ks_done of k_resolve)
+    float* tile_err;     // [tile]: max over the tile's pixels of adapt_pixel's error after its latest pass
+    int width, height, tiles_x;
+    int pass_spp, spp, min_spp;
+    float target;        // 8-bit output levels; 0 = never stop before the budget
+};
+
+constexpr int ADAPT_THREADS = 256;
+constexpr int COMPACT_THREADS = 1024;
+
+__global__ void k_adapt_init(AdaptArgs a, int n_tiles) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_tiles) return;
+    a.list[t] = t;
+    a.tile_ks[t] = 0u;
+    a.tile_err[t] = 0.0f;
+}
+
+// one CTA per tile of the pass's list
+__global__ void __launch_bounds__(ADAPT_THREADS) k_adapt(AdaptArgs a) {
+    __shared__ float warp_max[ADAPT_THREADS / 32];
+    const int t = a.list[blockIdx.x];
+    const uint32_t ks = a.tile_ks[t] + (uint32_t)a.pass_spp;
+    const int B = (int)(ks / (uint32_t)a.pass_spp);
+    const float inv_n = 4.0f / (float)a.pass_spp;
+    float err = 0.0f;
+    for (int slot = threadIdx.x; slot < 1024; slot += ADAPT_THREADS) {
+        int x, y;
+        if (!local_to_xy(t * 1024 + slot, 0, 1, a.tiles_x, a.width, a.height, x, y)) continue;
+        const uint32_t p = (uint32_t)(y * a.width + x);
+        float4 sub[4];
+        for (int s = 0; s < 4; ++s) sub[s] = a.accum[p * 4u + s];
+        float2 mom = a.mom[p];
+        err = fmaxf(err, adapt_pixel(sub, inv_n, mom, B));
+        for (int s = 0; s < 4; ++s) a.accum[p * 4u + s].w = sub[s].w;
+        a.mom[p] = mom;
+    }
+    for (int off = 16; off; off >>= 1) err = fmaxf(err, __shfl_xor_sync(0xffffffffu, err, off));
+    if ((threadIdx.x & 31) == 0) warp_max[threadIdx.x >> 5] = err;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < ADAPT_THREADS / 32; ++w) err = fmaxf(err, warp_max[w]);
+        a.tile_ks[t] = ks;
+        a.tile_err[t] = err;
+        const bool go_on = ks < (uint32_t)a.spp && (ks < (uint32_t)a.min_spp || a.target <= 0.0f || err > a.target);
+        if (!go_on) a.list[blockIdx.x] = -1;
+    }
+}
+
+// one CTA: drops the -1 entries of list[0, n) in place, order kept (an entry only ever moves towards the front, and a chunk
+// is read completely before any of it is written); the new count goes to mapped host memory
+__global__ void __launch_bounds__(COMPACT_THREADS) k_compact_tiles(int32_t* list, int n, volatile int* host_count) {
+    __shared__ int warp_sum[COMPACT_THREADS / 32];
+    __shared__ int base;
+    const unsigned lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    if (threadIdx.x == 0) base = 0;
+    __syncthreads();
+    for (int c0 = 0; c0 < n; c0 += COMPACT_THREADS) {
+        const int i = c0 + (int)threadIdx.x;
+        const int32_t v = i < n ? list[i] : -1;
+        const unsigned keep = __ballot_sync(0xffffffffu, v >= 0);
+        if (lane == 0) warp_sum[w] = __popc(keep);
+        __syncthreads();
+        int before = base, total = 0;
+        for (int k = 0; k < COMPACT_THREADS / 32; ++k) {
+            before += k < (int)w ? warp_sum[k] : 0;
+            total += warp_sum[k];
+        }
+        if (v >= 0) list[before + __popc(keep & ((1u << lane) - 1u))] = v;
+        __syncthreads();
+        if (threadIdx.x == 0) base += total;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        *host_count = base;
+        __threadfence_system();
+    }
 }
 
 // scatter `world` tile-ordered shards into a scan-line frame

@@ -13,7 +13,7 @@ import threading
 import numpy as np
 
 from . import _abi
-from ._abi import ACCEL_LBVH, ACCEL_OCTREE_REFERENCE, EST_MIS_BALANCE, EST_MIS_DEAD, EST_NEE, ObjectDesc, ObjectInfo, Params, SceneDesc, SceneInfo, Stats
+from ._abi import ACCEL_LBVH, ACCEL_OCTREE_REFERENCE, EST_MIS_BALANCE, EST_MIS_DEAD, EST_NEE, Adaptive, ObjectDesc, ObjectInfo, Params, SceneDesc, SceneInfo, Stats
 
 
 class RtbError(RuntimeError):
@@ -58,6 +58,16 @@ def make_params(width: int, height: int, spp: int, *, use_mis: bool = False, see
     p.tuning[2] = tune_steps
     p.tuning[3] = (0 if bin_bits is None else (1 if bin_bits <= 0 else max(2, bin_bits))) + (256 if bin_octant_major else 0)
     return p
+
+
+def make_adaptive(spp: int, *, target_levels: float, pass_spp: int = 16, min_spp: int | None = None) -> Adaptive:
+    """rtb_adaptive for a budget of `spp` samples per pixel; min_spp None = 4 passes, clipped to the budget."""
+    o = Adaptive()
+    o.target_levels = target_levels
+    o.pass_spp = pass_spp
+    o.min_spp = min(4 * pass_spp, spp) if min_spp is None else min_spp
+    o.reserved = 0
+    return o
 
 
 class Scene:
@@ -209,6 +219,22 @@ class Scene:
         _check(_abi.lib().rtb_render(self._h, C.byref(p), out.ctypes.data_as(C.POINTER(C.c_uint8)), None))
         return out
 
+    def render_adaptive(self, width: int, height: int, spp: int, *, target_levels: float, pass_spp: int = 16,
+                        min_spp: int | None = None, use_mis: bool = False, seed: int = 0, accel: int = 0):
+        """Adaptive sampling (rtb_render_adaptive): spp is the budget; each 32x32 tile stops once every pixel's estimated
+        standard error is <= target_levels 8-bit output levels.  Returns (frame uint8 [h, w, 3], tile_spp int32 [ty, tx],
+        tile_error float32 [ty, tx])."""
+        p = make_params(width, height, spp, use_mis=use_mis, seed=seed, accel=accel)
+        o = make_adaptive(spp, target_levels=target_levels, pass_spp=pass_spp, min_spp=min_spp)
+        ty, tx = (height + 31) // 32, (width + 31) // 32
+        out = np.zeros((height, width, 3), dtype=np.uint8)
+        tile_spp = np.zeros((ty, tx), dtype=np.int32)
+        tile_error = np.zeros((ty, tx), dtype=np.float32)
+        _check(_abi.lib().rtb_render_adaptive(self._h, C.byref(p), C.byref(o), out.ctypes.data_as(C.POINTER(C.c_uint8)),
+                                              tile_spp.ctypes.data_as(C.POINTER(C.c_int32)),
+                                              tile_error.ctypes.data_as(C.POINTER(C.c_float)), None))
+        return out, tile_spp, tile_error
+
     def render_device(self, params: Params, d_rgb8_tiles: int, d_subpixel_sums: int = 0) -> int:
         """Device-resident render: raw device pointers (e.g. torch tensor .data_ptr())."""
         return _check(_abi.lib().rtb_render_device(self._h, C.byref(params), C.c_void_p(d_rgb8_tiles),
@@ -286,13 +312,20 @@ class RenderJob:
     PIXELS_PER_MSG = 60
 
     def __init__(self, scene: Scene, width: int, height: int, samples_per_pixel: int, *, passes: int = 1, seed: int = 0,
-                 use_mis: bool = False, pool_paths: int = 0, accel: int = 0):
+                 use_mis: bool = False, pool_paths: int = 0, accel: int = 0, adaptive: dict | None = None):
+        """adaptive: dict(target_levels=..., pass_spp=16, min_spp=None) makes this an adaptive job (rtb_job_begin_adaptive):
+        samples_per_pixel is the budget, `passes` is ignored and the job re-sends the frame once per pass until every tile
+        has converged."""
         self.scene = scene
         self.params = make_params(width, height, samples_per_pixel, use_mis=use_mis, seed=seed, pool_paths=pool_paths, accel=accel)
         self._h = C.c_void_p()
         # guards the handle: stop() may come from another thread (the server's event loop) while close() frees the job
         self._lock = threading.Lock()
-        _check(_abi.lib().rtb_job_begin(scene._h, C.byref(self.params), passes, C.byref(self._h)))
+        if adaptive is not None:
+            self.adaptive = make_adaptive(samples_per_pixel, **adaptive)
+            _check(_abi.lib().rtb_job_begin_adaptive(scene._h, C.byref(self.params), C.byref(self.adaptive), C.byref(self._h)))
+        else:
+            _check(_abi.lib().rtb_job_begin(scene._h, C.byref(self.params), passes, C.byref(self._h)))
         self._buf = (C.c_uint8 * (256 * (6 + 3 * self.PIXELS_PER_MSG)))()
         self.cancelled = False
         self.final_stats = None

@@ -5,7 +5,10 @@ Protocol (reference `src/server.rs`):
         {"type": "render", "scene": "<name>", "spp": <int>}      accepted only while the connection is idle (:94-106)
         {"type": "stop_rendering"}                                accepted only while a job runs (:108-111)
     anything else is ignored (:112).  Extension (ignored by the reference's serde structs, so old clients are
-    unaffected): "passes": <int> renders progressively and re-sends every record once per pass.
+    unaffected): "passes": <int> renders progressively and re-sends every record once per pass; "noise": <number> asks
+    for adaptive sampling instead — every 32x32 tile stops once its estimated standard error is at most that many 8-bit
+    output levels, with "spp" as the budget (rounded down to a multiple of ADAPTIVE_PASS_SPP), and every record is
+    re-sent once per pass until all tiles have stopped.
   * server -> client, binary, one message per <= 60 pixels of one screen row (:173-190):
         [0] = 0 (message type)   [1] = n   [2..4] = x u16le   [4..6] = y u16le (row 0 = top)   then n x (r, g, b)
     There is no "done" message; the client counts pixels (test-client/app.tsx:69-70).
@@ -24,6 +27,7 @@ from __future__ import annotations
 
 import asyncio
 import json
+import math
 import os
 import random
 import string
@@ -33,6 +37,8 @@ from typing import Callable, Iterable
 SCENE_NAMES = ("cornell_box", "cubes", "flying_unicorn")  # src/main.rs:17
 WIDTH, HEIGHT = 600, 450                                   # Server::WIDTH / HEIGHT, src/server.rs:29-30
 DEFAULT_PORT = "8080"                                      # src/main.rs:16
+ADAPTIVE_PASS_SPP = 16                                     # "noise" requests: samples per pixel per pass ...
+ADAPTIVE_MIN_SPP = 64                                      # ... and the least any tile gets (clipped to the budget)
 
 
 def default_job_factory(scenes: dict, width: int, height: int, accel: int = 0):
@@ -40,13 +46,14 @@ def default_job_factory(scenes: dict, width: int, height: int, accel: int = 0):
     Rust binary sends, non-nearest triangles included; 2.4 x slower on flying_unicorn).  `main` reads it from $RTB_ACCEL."""
     from .host import RenderJob
 
-    def make(scene_name: str, spp: int, passes: int = 1):
+    def make(scene_name: str, spp: int, passes: int = 1, adaptive: dict | None = None):
         scene = scenes.get(scene_name)
         if scene is None:
             return None
         # spp is an i32 in the reference (`ClientMessage::Render`, :123); `num_samples = spp / 4` makes every spp < 4,
         # negative ones included, an empty sample loop: a black frame is streamed (src/server.rs:332-362)
-        return RenderJob(scene, width, height, max(0, spp), passes=passes, seed=random.getrandbits(63), accel=accel)
+        return RenderJob(scene, width, height, max(0, spp), passes=passes, seed=random.getrandbits(63), accel=accel,
+                         adaptive=adaptive)
 
     return make
 
@@ -91,11 +98,16 @@ class Server:
                         if not isinstance(scene_name, str) or type(spp) is not int or not -2 ** 31 <= spp < 2 ** 31 or type(passes) is not int:
                             raise TypeError
                         passes = max(1, passes)
-                    except (KeyError, TypeError):
+                        adaptive = self._adaptive_options(req["noise"], spp) if "noise" in req else None
+                    except (KeyError, TypeError, ValueError, OverflowError):
                         await websocket.close(code=1007, reason="failed to parse message")
                         break
                     try:
-                        job = self.job_factory(scene_name, spp, passes)
+                        if adaptive is not None:
+                            budget, opts = adaptive
+                            job = self.job_factory(scene_name, budget, 1, adaptive=opts)
+                        else:
+                            job = self.job_factory(scene_name, spp, passes)
                     except RuntimeError as e:                  # the library refused the request (RtbError): not a reason to drop the client
                         self.log(f"[{cid}] render request refused: {e}")
                         continue
@@ -118,6 +130,17 @@ class Server:
                     pass
             self.connections.discard(cid)
             self.log(f"[{cid}] Disconnected.")
+
+    @staticmethod
+    def _adaptive_options(noise, spp: int) -> tuple[int, dict] | None:
+        """(budget, adaptive options) of the job a "noise" request asks for, or None when the budget is too small for two
+        passes (a plain job then renders the frame).  Raises ValueError unless noise is a finite non-negative JSON number."""
+        if type(noise) not in (int, float) or not math.isfinite(noise) or noise < 0:
+            raise ValueError("noise")
+        budget = max(0, spp) // ADAPTIVE_PASS_SPP * ADAPTIVE_PASS_SPP
+        if budget < 2 * ADAPTIVE_PASS_SPP:
+            return None
+        return budget, {"target_levels": float(noise), "pass_spp": ADAPTIVE_PASS_SPP, "min_spp": min(ADAPTIVE_MIN_SPP, budget)}
 
     async def _run_job(self, cid: str, websocket, job):
         """RenderJob::run: forward the job's records as binary messages; the GPU call runs in a worker thread."""
