@@ -63,12 +63,8 @@ struct DevScene {          // passed to kernels by value
     const DevSceneHeader* hdr;
     const DevPrim* prims;
     const DevMaterial* mats;
-    const float4* nodes;   // 4 x float4 per node (fp32 boxes: build output, kept for inspection)
     const uint4* qnodes;   // 2 x uint4 per node: the 16-bit quantised table the traversal reads (lbvh.cu)
     float3 qmin, qstep;    // quantisation grid of qnodes
-    const uint4* qnodes4;  // 4 x uint4 per node: the 4-wide table collapsed from the binary tree (lbvh.cu collapse_to_bvh4)
-    int32_t root4;         // root reference into qnodes4
-    int32_t wide;          // 1: traverse qnodes4 (default), 0: the binary table (RTB_BVH_WIDE=0)
     const float4* tris;    // TRI_STRIDE x float4 per triangle (3 used), leaf order
     const float4* tri_nrm; // unit geometric normal | object id per triangle, leaf order (shading)
     const float* light_cdf;

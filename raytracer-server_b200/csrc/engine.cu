@@ -10,6 +10,7 @@
 #include <chrono>
 #include <cmath>
 #include <condition_variable>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -83,8 +84,6 @@ struct RenderContext {
     cudaGraphExec_t graph_exec[4] = {nullptr, nullptr, nullptr, nullptr};   // one iteration (4 kernels) for cur = 0 / 1; [2], [3]: the same with the inline-tail k_shade ...
     std::vector<unsigned char> graph_args;                 // ... captured for exactly these kernel arguments
     int grid_shade_nomesh = 0;   // grid of the mesh-less k_shade instantiation (160-thread CTAs)
-    int trav_minb = 5;   // CTAs per SM the launched k_traverse instantiation was compiled for (RTB_TRAV_MINB = 4 | 5 | 6).  5 since the
-                         // SAH tree (51 registers, a few spills, 40 warps per SM): bench frame 540.4 -> 537.0 ms; on the PLOC tree 4 was ahead
     int grid_oct = 0;    // k_traverse_octree's own persistent grid
     int grid_ext = 0, grid_ext_count = 0, grid_sh = 0, grid_sh_count = 0, grid_gen = 0, grid_shade = 0, grid_bin = 0;
     // adaptive sampling (ensure_adaptive): allocated by the first adaptive request only
@@ -186,7 +185,7 @@ struct LbvhImport {
     LbvhResult meta;   // scalars; the pointers are unused
     int n_tris;
     const float4 *nodes, *tris, *tri_nrm;
-    const uint4 *qnodes, *qnodes4;
+    const uint4* qnodes;
 };
 
 int build_device_scene(rtb_scene* sc, const LbvhImport* import = nullptr) {
@@ -229,7 +228,7 @@ int build_device_scene(rtb_scene* sc, const LbvhImport* import = nullptr) {
     if (import) {   // the tables another rank built: copy instead of building (the scene + BVH broadcast of a multi-GPU job)
         LbvhResult& B = sc->bvh;
         B = import->meta;
-        B.d_nodes = nullptr; B.d_qnodes = nullptr; B.d_qnodes4 = nullptr; B.d_tris = nullptr; B.d_tri_nrm = nullptr;
+        B.d_nodes = nullptr; B.d_qnodes = nullptr; B.d_tris = nullptr; B.d_tri_nrm = nullptr;
         if (import->n_tris != n_tris) return fail(RTB_EPARSE, "exported scene: triangle count does not match the LBVH tables");
         auto up = [&](void** dst, const void* src, size_t bytes) -> cudaError_t {
             cudaError_t e = cudaMalloc(dst, std::max<size_t>(bytes, 16));
@@ -239,7 +238,6 @@ int build_device_scene(rtb_scene* sc, const LbvhImport* import = nullptr) {
         if (n_tris) {
             CU_TRY(up((void**)&B.d_nodes, import->nodes, (size_t)B.n_nodes * 4 * sizeof(float4)));
             CU_TRY(up((void**)&B.d_qnodes, import->qnodes, (size_t)B.n_nodes * 2 * sizeof(uint4)));
-            CU_TRY(up((void**)&B.d_qnodes4, import->qnodes4, (size_t)std::max(B.n_nodes4, 1) * 4 * sizeof(uint4)));
             CU_TRY(up((void**)&B.d_tris, import->tris, (size_t)n_tris * TRI_STRIDE * sizeof(float4)));
             CU_TRY(up((void**)&B.d_tri_nrm, import->tri_nrm, (size_t)n_tris * sizeof(float4)));
         }
@@ -284,12 +282,7 @@ int build_device_scene(rtb_scene* sc, const LbvhImport* import = nullptr) {
     V.hdr = reinterpret_cast<const DevSceneHeader*>(sc->d_stage);
     V.prims = reinterpret_cast<const DevPrim*>(sc->d_stage + sc->off_prims);
     V.mats = reinterpret_cast<const DevMaterial*>(sc->d_stage + sc->off_mats);
-    V.nodes = sc->bvh.d_nodes;
     V.qnodes = sc->bvh.d_qnodes;
-    V.qnodes4 = sc->bvh.d_qnodes4;
-    V.root4 = sc->bvh.root4;
-    V.wide = 0;   // measured: the 4-wide table halves the memory stalls but costs 36 % more instructions — a wash (DESIGN.md §8)
-    if (const char* e = getenv("RTB_BVH_WIDE")) V.wide = atoi(e) != 0;
     V.qmin = make_float3(sc->bvh.qmin[0], sc->bvh.qmin[1], sc->bvh.qmin[2]);
     V.qstep = make_float3(sc->bvh.qstep[0], sc->bvh.qstep[1], sc->bvh.qstep[2]);
     V.tris = sc->bvh.d_tris;
@@ -519,15 +512,9 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
         CU_TRY(cudaFuncSetAttribute(k_shade<1, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         CU_TRY(cudaFuncSetAttribute(k_shade<2, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         int b = 0;
-        if (sc->view.wide) c->trav_minb = 4;   // the 4-wide experiment table has one instantiation only
-        if (const char* e = getenv("RTB_TRAV_MINB")) c->trav_minb = atoi(e) == 5 ? 5 : (atoi(e) == 6 ? 6 : 4);
-        if (c->trav_minb == 5) CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<false, 5>, WF_THREADS, smem_stack));
-        else if (c->trav_minb == 6) CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<false, 6>, WF_THREADS, smem_stack));
-        else if (sc->view.wide) CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<false, 4, true>, WF_THREADS, smem_stack));
-        else CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<false>, WF_THREADS, smem_stack));
+        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<false>, WF_THREADS, smem_stack));
         c->grid_ext = std::max(1, b) * prop.multiProcessorCount;
-        if (sc->view.wide) CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<true, 4, true>, WF_THREADS, smem_stack));
-        else CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<true>, WF_THREADS, smem_stack));
+        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<true>, WF_THREADS, smem_stack));
         c->grid_ext_count = std::max(1, b) * prop.multiProcessorCount;
         CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse_octree<false>, WF_THREADS, (size_t)OCT_MAX_DEPTH * WF_THREADS * sizeof(int2)));
         c->grid_oct = std::max(1, b) * prop.multiProcessorCount;
@@ -663,11 +650,7 @@ void launch_traverse(RenderContext* c, const RenderArgs& a, int cur, bool count_
         const size_t smem_oct = (size_t)OCT_MAX_DEPTH * WF_THREADS * sizeof(int2);
         if (count_work) k_traverse_octree<true><<<c->grid_oct, WF_THREADS, smem_oct, c->stream>>>(a, cur);
         else k_traverse_octree<false><<<c->grid_oct, WF_THREADS, smem_oct, c->stream>>>(a, cur);
-    } else if (count_work && a.S.wide) k_traverse<true, 4, true><<<c->grid_ext_count, WF_THREADS, smem_stack, c->stream>>>(a, cur);
-    else if (count_work) k_traverse<true><<<c->grid_ext_count, WF_THREADS, smem_stack, c->stream>>>(a, cur);
-    else if (a.S.wide && c->trav_minb == 4) k_traverse<false, 4, true><<<c->grid_ext, WF_THREADS, smem_stack, c->stream>>>(a, cur);
-    else if (c->trav_minb == 5) k_traverse<false, 5><<<c->grid_ext, WF_THREADS, smem_stack, c->stream>>>(a, cur);
-    else if (c->trav_minb == 6) k_traverse<false, 6><<<c->grid_ext, WF_THREADS, smem_stack, c->stream>>>(a, cur);
+    } else if (count_work) k_traverse<true><<<c->grid_ext_count, WF_THREADS, smem_stack, c->stream>>>(a, cur);
     else k_traverse<false><<<c->grid_ext, WF_THREADS, smem_stack, c->stream>>>(a, cur);
 }
 
@@ -1205,31 +1188,34 @@ int rtb_scene_create(const rtb_scene_desc* desc, int device, rtb_scene** out) {
 
 // ---- scene + BVH as one blob: what a multi-GPU job broadcasts once (BASELINE.json north_star) --------------------
 // Layout: ExportHeader | per object: ExportObject, vertices (3 f64 each), indices (u32), cumulative areas (f64) | LBVH tables
-// (fp32 nodes, quantised nodes, 4-wide nodes, triangles, normals) exactly as they sit in device memory.  A rank that imports
-// the blob neither parses TOML / OBJ nor builds a BVH; it gets bit-identical tables, hence bit-identical traversal.
+// (fp32 nodes, quantised nodes, triangles, normals) exactly as they sit in device memory.  A rank that imports the blob
+// neither parses TOML / OBJ nor builds a BVH; it gets bit-identical tables, hence bit-identical traversal.
 namespace {
 struct ExportHeader {
     char magic[8];
     uint64_t total_bytes;
     double cam_pos[3], cam_dir[3];
     int32_t n_objects, light;
-    int32_t n_tris, n_nodes, n_leaves, root, depth, n_nodes4, root4, pad;
+    int32_t n_tris, n_nodes, n_leaves, root, depth, pad[3];   // pad: zero; no implicit padding, build_ms stays at byte 152
     float qmin[3], qstep[3], bmin[3], bmax[3];
     double build_ms;
 };
+// build_ms is the one header field that differs between two builds of one scene: readers that compare blobs mask it
+// at this offset
+static_assert(offsetof(ExportHeader, build_ms) == 152, "ExportHeader layout changed: bump EXPORT_MAGIC");
 struct ExportObject {
     double emitted[3], k[3], color_d[3], color_s[3], pos[3], n[3], bb_min[3], bb_max[3];
     double phong_kd, phong_ks, r, surface_area;
     int32_t brdf, phong_power, geom, pad;
     uint64_t n_vertices, n_indices, n_cum;
 };
-constexpr char EXPORT_MAGIC[8] = {'R', 'T', 'B', 'S', 'C', 'N', '2', 0};
+constexpr char EXPORT_MAGIC[8] = {'R', 'T', 'B', 'S', 'C', 'N', '3', 0};
 void put3(double* d, const D3& v) { d[0] = v.x; d[1] = v.y; d[2] = v.z; }
 D3 get3(const double* d) { return D3{d[0], d[1], d[2]}; }
 size_t lbvh_bytes(const LbvhResult& B, int n_tris) {
     if (n_tris == 0) return 0;
-    return (size_t)B.n_nodes * 4 * sizeof(float4) + (size_t)B.n_nodes * 2 * sizeof(uint4) + (size_t)std::max(B.n_nodes4, 1) * 4 * sizeof(uint4) +
-           (size_t)n_tris * TRI_STRIDE * sizeof(float4) + (size_t)n_tris * sizeof(float4);
+    return (size_t)B.n_nodes * 4 * sizeof(float4) + (size_t)B.n_nodes * 2 * sizeof(uint4) + (size_t)n_tris * TRI_STRIDE * sizeof(float4) +
+           (size_t)n_tris * sizeof(float4);
 }
 }  // namespace
 
@@ -1254,7 +1240,7 @@ int64_t rtb_scene_export(rtb_scene* scene, void* buf, int64_t cap) {
     H.n_objects = (int32_t)scene->hs.objects.size();
     H.light = scene->hs.light;
     const LbvhResult& B = scene->bvh;
-    H.n_tris = tables ? n_tris : -1; H.n_nodes = B.n_nodes; H.n_leaves = B.n_leaves; H.root = B.root; H.depth = B.depth; H.n_nodes4 = B.n_nodes4; H.root4 = B.root4;
+    H.n_tris = tables ? n_tris : -1; H.n_nodes = B.n_nodes; H.n_leaves = B.n_leaves; H.root = B.root; H.depth = B.depth;
     for (int k = 0; k < 3; ++k) { H.qmin[k] = B.qmin[k]; H.qstep[k] = B.qstep[k]; H.bmin[k] = B.bmin[k]; H.bmax[k] = B.bmax[k]; }
     H.build_ms = scene->info.build_ms;
     std::memcpy(p, &H, sizeof(H));
@@ -1278,7 +1264,6 @@ int64_t rtb_scene_export(rtb_scene* scene, void* buf, int64_t cap) {
         auto down = [&](const void* src, size_t bytes) { cudaError_t e = cudaMemcpy(p + off, src, bytes, cudaMemcpyDeviceToHost); off += bytes; return e; };
         CU_TRY(down(B.d_nodes, (size_t)B.n_nodes * 4 * sizeof(float4)));
         CU_TRY(down(B.d_qnodes, (size_t)B.n_nodes * 2 * sizeof(uint4)));
-        CU_TRY(down(B.d_qnodes4, (size_t)std::max(B.n_nodes4, 1) * 4 * sizeof(uint4)));
         CU_TRY(down(B.d_tris, (size_t)n_tris * TRI_STRIDE * sizeof(float4)));
         CU_TRY(down(B.d_tri_nrm, (size_t)n_tris * sizeof(float4)));
     }
@@ -1324,13 +1309,12 @@ int rtb_scene_import(const void* buf, int64_t bytes, int device, rtb_scene** out
     LbvhImport imp{};
     imp.n_tris = H.n_tris;
     LbvhResult& M = imp.meta;
-    M.n_nodes = H.n_nodes; M.n_leaves = H.n_leaves; M.root = H.root; M.depth = H.depth; M.n_nodes4 = H.n_nodes4; M.root4 = H.root4;
+    M.n_nodes = H.n_nodes; M.n_leaves = H.n_leaves; M.root = H.root; M.depth = H.depth;
     for (int k = 0; k < 3; ++k) { M.qmin[k] = H.qmin[k]; M.qstep[k] = H.qstep[k]; M.bmin[k] = H.bmin[k]; M.bmax[k] = H.bmax[k]; }
     if (H.n_tris > 0) {
-        if (H.n_nodes < 0 || H.n_nodes4 < 0 || !need(lbvh_bytes(M, H.n_tris))) { delete sc; return fail(RTB_EPARSE, "exported scene: truncated LBVH tables"); }
+        if (H.n_nodes < 0 || !need(lbvh_bytes(M, H.n_tris))) { delete sc; return fail(RTB_EPARSE, "exported scene: truncated LBVH tables"); }
         imp.nodes = reinterpret_cast<const float4*>(p + off); off += (size_t)M.n_nodes * 4 * sizeof(float4);
         imp.qnodes = reinterpret_cast<const uint4*>(p + off); off += (size_t)M.n_nodes * 2 * sizeof(uint4);
-        imp.qnodes4 = reinterpret_cast<const uint4*>(p + off); off += (size_t)std::max(M.n_nodes4, 1) * 4 * sizeof(uint4);
         imp.tris = reinterpret_cast<const float4*>(p + off); off += (size_t)H.n_tris * TRI_STRIDE * sizeof(float4);
         imp.tri_nrm = reinterpret_cast<const float4*>(p + off);
     }

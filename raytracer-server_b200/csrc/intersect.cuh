@@ -21,7 +21,7 @@
 
 namespace rtb {
 
-constexpr int STACK_SMEM = 24;   // stack levels kept in shared memory (per thread); a 4-wide step pushes up to three
+constexpr int STACK_SMEM = 24;   // stack levels kept in shared memory (per thread); an inner node pushes at most one
 constexpr int STACK_LOCAL = 72;  // overflow levels in local memory.  The loader measures the depth of the tree it built and
                                  // refuses (RTB_EUNSUPPORTED) what does not fit BVH_MAX_DEPTH = STACK_SMEM + STACK_LOCAL levels
                                  // (lbvh.hpp; PLOC trees have no a-priori depth bound, a too deep one is rebuilt as a Karras
@@ -337,7 +337,7 @@ struct Trav {
     int sp;
 };
 
-__device__ __forceinline__ void trav_begin(const DevScene& S, Trav& T, float3 o, float3 d, uint32_t origin, float tlimit, int root) {
+__device__ __forceinline__ void trav_begin(const DevScene& S, Trav& T, float3 o, float3 d, uint32_t origin, float tlimit) {
     T.o = o;
     T.d = d;
     // MUFU.RCP reciprocals (1-2 ulp).  The node boxes are quantised with QPAD = 2 grid steps of slack (lbvh.cu): the
@@ -360,7 +360,7 @@ __device__ __forceinline__ void trav_begin(const DevScene& S, Trav& T, float3 o,
     T.origin = origin;
     T.tlimit = tlimit;
     T.best_id = PC_NONE;
-    T.node = root;
+    T.node = S.root;
     T.sp = 0;
 }
 
@@ -435,68 +435,6 @@ __device__ __forceinline__ void trav_inner(const DevScene& S, Trav& T, uint32_t 
     }
 }
 
-// ---- 4-wide step ----------------------------------------------------------------------------------
-__device__ __forceinline__ void trav_push(Trav& T, uint32_t sbase, uint32_t sstride, int* lstack, int v) {
-    if (T.sp < STACK_SMEM) sts_i32(sbase + (uint32_t)T.sp * sstride, v);
-    else if (T.sp - STACK_SMEM < STACK_LOCAL) lstack[T.sp - STACK_SMEM] = v;
-    else return;   // deeper than any accepted tree (see STACK_LOCAL)
-    ++T.sp;
-}
-// one node of the 4-wide table: four slab tests, then the hit children sorted by entry distance — the nearest is
-// visited next, the others are pushed farthest first.  Half as many dependent node fetches per ray as the binary
-// table, for slightly fewer instructions (one 5-comparator network instead of two near/far decisions).
-template <bool COUNT>
-__device__ __forceinline__ void trav_inner4(const DevScene& S, Trav& T, uint32_t sbase, uint32_t sstride, int* lstack, uint32_t* work) {
-    uint4 q0, q1, q2, q3;
-    const uint4* np = S.qnodes4 + (size_t)T.node * 4;
-    ldg256u(np, q0, q1);
-    ldg256u(np + 2, q2, q3);
-    if (COUNT) work[0] += 2;   // four slab tests = two binary node visits in the flop model
-    auto pl = [](uint32_t w, uint32_t sel) { return __uint_as_float(__byte_perm(w, 0x4B000000u, sel)); };
-    const float2 sxy = make_float2(T.sx, T.sy), bxy = make_float2(T.bx, T.by);
-    const float2 szz = make_float2(T.sz, T.sz), bzz = make_float2(T.bz, T.bz);
-    // words: q0 = c0.x c0.y c0.z c1.x | q1 = c1.y c1.z c2.x c2.y | q2 = c2.z c3.x c3.y c3.z | q3 = refs
-    const float2 n0 = __ffma2_rn(make_float2(pl(q0.x, T.nsx), pl(q0.y, T.nsy)), sxy, bxy);
-    const float2 f0 = __ffma2_rn(make_float2(pl(q0.x, T.fsx), pl(q0.y, T.fsy)), sxy, bxy);
-    const float2 n1 = __ffma2_rn(make_float2(pl(q0.w, T.nsx), pl(q1.x, T.nsy)), sxy, bxy);
-    const float2 f1 = __ffma2_rn(make_float2(pl(q0.w, T.fsx), pl(q1.x, T.fsy)), sxy, bxy);
-    const float2 n2 = __ffma2_rn(make_float2(pl(q1.z, T.nsx), pl(q1.w, T.nsy)), sxy, bxy);
-    const float2 f2_ = __ffma2_rn(make_float2(pl(q1.z, T.fsx), pl(q1.w, T.fsy)), sxy, bxy);
-    const float2 n3 = __ffma2_rn(make_float2(pl(q2.y, T.nsx), pl(q2.z, T.nsy)), sxy, bxy);
-    const float2 f3_ = __ffma2_rn(make_float2(pl(q2.y, T.fsx), pl(q2.z, T.fsy)), sxy, bxy);
-    const float2 nz01 = __ffma2_rn(make_float2(pl(q0.z, T.nsz), pl(q1.y, T.nsz)), szz, bzz);
-    const float2 fz01 = __ffma2_rn(make_float2(pl(q0.z, T.fsz), pl(q1.y, T.fsz)), szz, bzz);
-    const float2 nz23 = __ffma2_rn(make_float2(pl(q2.x, T.nsz), pl(q2.w, T.nsz)), szz, bzz);
-    const float2 fz23 = __ffma2_rn(make_float2(pl(q2.x, T.fsz), pl(q2.w, T.fsz)), szz, bzz);
-    const float tmin0 = fmaxf(fmaxf(n0.x, n0.y), fmaxf(nz01.x, 0.0f)), tmax0 = fminf(fminf(f0.x, f0.y), fminf(fz01.x, T.tlimit));
-    const float tmin1 = fmaxf(fmaxf(n1.x, n1.y), fmaxf(nz01.y, 0.0f)), tmax1 = fminf(fminf(f1.x, f1.y), fminf(fz01.y, T.tlimit));
-    const float tmin2 = fmaxf(fmaxf(n2.x, n2.y), fmaxf(nz23.x, 0.0f)), tmax2 = fminf(fminf(f2_.x, f2_.y), fminf(fz23.x, T.tlimit));
-    const float tmin3 = fmaxf(fmaxf(n3.x, n3.y), fmaxf(nz23.y, 0.0f)), tmax3 = fminf(fminf(f3_.x, f3_.y), fminf(fz23.y, T.tlimit));
-    // sort keys: entry distance (>= 0, so its bit pattern orders like an unsigned integer); misses sort last
-    constexpr uint32_t MISS = 0xffffffffu;
-    uint32_t k0 = tmin0 <= tmax0 ? __float_as_uint(tmin0) : MISS, k1 = tmin1 <= tmax1 ? __float_as_uint(tmin1) : MISS;
-    uint32_t k2 = tmin2 <= tmax2 ? __float_as_uint(tmin2) : MISS, k3 = tmin3 <= tmax3 ? __float_as_uint(tmin3) : MISS;
-    int r0 = (int)q3.x, r1 = (int)q3.y, r2 = (int)q3.z, r3 = (int)q3.w;
-#define RTB_CSWAP(ka, ra, kb, rb)                 \
-    {                                             \
-        const bool sw = kb < ka;                  \
-        const uint32_t lo_ = min(ka, kb), hi_ = max(ka, kb); \
-        const int rl_ = sw ? rb : ra, rh_ = sw ? ra : rb;    \
-        ka = lo_; kb = hi_; ra = rl_; rb = rh_;   \
-    }
-    RTB_CSWAP(k0, r0, k1, r1)
-    RTB_CSWAP(k2, r2, k3, r3)
-    RTB_CSWAP(k0, r0, k2, r2)
-    RTB_CSWAP(k1, r1, k3, r3)
-    RTB_CSWAP(k1, r1, k2, r2)
-#undef RTB_CSWAP
-    if (k3 != MISS) trav_push(T, sbase, sstride, lstack, r3);
-    if (k2 != MISS) trav_push(T, sbase, sstride, lstack, r2);
-    if (k1 != MISS) trav_push(T, sbase, sstride, lstack, r1);
-    if (k0 != MISS) T.node = r0;
-    else trav_pop(T, sbase, sstride, lstack);
-}
-
 // one leaf (T.node < 0, not the sentinel): Triangle::intersect on its 1..8 triangles.
 // ANY_HIT: returns true at the first triangle with t < tlimit.  Closest: shrinks tlimit / records best_id.
 template <bool ANY_HIT, bool COUNT>
@@ -537,7 +475,7 @@ __device__ __forceinline__ bool trav_leaf(const DevScene& S, Trav& T, uint32_t* 
 
 // whole traversal for one ray ("while-while": a lane leaves the inner-node loop when it holds a leaf,
 // so the triangle code runs with as many lanes as possible)
-template <bool ANY_HIT, bool COUNT, bool WIDE = false>
+template <bool ANY_HIT, bool COUNT>
 __device__ __forceinline__ bool bvh_traverse(const DevScene& S, const SharedScene& sh, float3 o, float3 d, uint32_t origin,
                                              float& best_t, uint32_t& best_id, float dist, uint32_t* work) {
     // ANY_HIT: returns true as soon as some triangle has t + SHADOW_MARGIN < dist.
@@ -545,12 +483,9 @@ __device__ __forceinline__ bool bvh_traverse(const DevScene& S, const SharedScen
     const uint32_t sbase = (uint32_t)__cvta_generic_to_shared(sh.stack + threadIdx.x), sstride = blockDim.x * 4u;
     int lstack[STACK_LOCAL];
     Trav T;
-    trav_begin(S, T, o, d, origin, ANY_HIT ? dist - SHADOW_MARGIN : best_t, WIDE ? S.root4 : S.root);
+    trav_begin(S, T, o, d, origin, ANY_HIT ? dist - SHADOW_MARGIN : best_t);
     while (T.node != NODE_SENTINEL) {
-        while (T.node >= 0) {
-            if (WIDE) trav_inner4<COUNT>(S, T, sbase, sstride, lstack, work);
-            else trav_inner<COUNT>(S, T, sbase, sstride, lstack, work);
-        }
+        while (T.node >= 0) trav_inner<COUNT>(S, T, sbase, sstride, lstack, work);
         if (T.node != NODE_SENTINEL) {
             if (trav_leaf<ANY_HIT, COUNT>(S, T, work)) return true;
             trav_pop(T, sbase, sstride, lstack);

@@ -692,96 +692,25 @@ __global__ void k_quantise_nodes(int n_nodes, const float4* __restrict__ nodes, 
 static bool build_lbvh_f32(const float* d_verts, const int32_t* d_tri_obj, int n, cudaStream_t stream, LbvhResult& out, std::string& err,
                            bool force_karras = false);
 
-// The 4-wide table: every binary node kept becomes a node with up to four children — its two children, the larger
-// (by box area) inner child replaced by its own two children until four are there.  A ray then waits for half as many
-// dependent node fetches.  This pass runs on the host over the finished binary table (a few 10 k nodes, < 1 ms): it is a
-// re-indexing of a tree the GPU built, done once per scene.
-// Layout of one node (16 words): words 3c .. 3c+2 = child c (lo.x | hi.x << 16), (lo.y | hi.y << 16), (lo.z | hi.z << 16)
-// quantised exactly like the binary table; words 12..15 = the four references.  An empty slot holds an inverted box.
-static bool collapse_to_bvh4(cudaStream_t stream, LbvhResult& out, const float* qinv, std::string& err) {
-    out.root4 = out.root;
-    out.n_nodes4 = 0;
-    if (out.n_nodes == 0 || out.root < 0) {
-        LBVH_CHECK(cudaMalloc((void**)&out.d_qnodes4, 4 * sizeof(uint4)));
-        return true;
-    }
+// Depth of the binary tree: 0 when the root is a leaf, otherwise the root is level 1 and every inner child one more.  The
+// traversal stack is finite: build_lbvh checks it against BVH_MAX_DEPTH.  Walked on the host over the finished fp32 table.
+static bool measure_depth(cudaStream_t stream, LbvhResult& out, std::string& err) {
+    out.depth = 0;
+    if (out.n_nodes == 0 || out.root < 0) return true;
     std::vector<float4> nodes((size_t)out.n_nodes * 4);
     LBVH_CHECK(cudaMemcpyAsync(nodes.data(), out.d_nodes, nodes.size() * sizeof(float4), cudaMemcpyDeviceToHost, stream));
     LBVH_CHECK(cudaStreamSynchronize(stream));
-    struct Child { float lo[3], hi[3]; int ref; };
-    auto children_of = [&](int node, Child* c) {
-        const float4* o = &nodes[(size_t)node * 4];
-        c[0] = Child{{o[0].x, o[0].z, o[2].x}, {o[0].y, o[0].w, o[2].y}, 0};
-        c[1] = Child{{o[1].x, o[1].z, o[2].z}, {o[1].y, o[1].w, o[2].w}, 0};
-        memcpy(&c[0].ref, &o[3].x, 4);
-        memcpy(&c[1].ref, &o[3].y, 4);
-    };
-    auto area = [](const Child& c) {
-        const float dx = c.hi[0] - c.lo[0], dy = c.hi[1] - c.lo[1], dz = c.hi[2] - c.lo[2];
-        return dx * dy + dy * dz + dz * dx;
-    };
-    {   // depth of the binary tree (the traversal stack is finite: build_lbvh checks it against BVH_MAX_DEPTH)
-        std::vector<std::pair<int, int>> st;
-        st.push_back({out.root, 1});
-        out.depth = 0;
-        while (!st.empty()) {
-            const auto [node, d] = st.back();
-            st.pop_back();
-            out.depth = std::max(out.depth, d);
-            Child c[2];
-            children_of(node, c);
-            for (int k = 0; k < 2; ++k)
-                if (c[k].ref >= 0) st.push_back({c[k].ref, d + 1});
-        }
+    std::vector<std::pair<int, int>> st;
+    st.push_back({out.root, 1});
+    while (!st.empty()) {
+        const auto [node, d] = st.back();
+        st.pop_back();
+        out.depth = std::max(out.depth, d);
+        int ref[2];
+        memcpy(ref, &nodes[(size_t)node * 4 + 3].x, sizeof(ref));   // float4 3 of the node: (ref 0, ref 1, -, -)
+        for (int k = 0; k < 2; ++k)
+            if (ref[k] >= 0) st.push_back({ref[k], d + 1});
     }
-    std::vector<uint32_t> words;      // 16 per wide node
-    std::vector<int> todo;            // binary nodes that become wide nodes, in emission order
-    std::vector<int> wide_of(out.n_nodes, -1);
-    todo.push_back(out.root);
-    wide_of[out.root] = 0;
-    for (size_t head = 0; head < todo.size(); ++head) {
-        Child c[4];
-        int n = 2;
-        children_of(todo[head], c);
-        while (n < 4) {   // open the largest inner child
-            int best = -1;
-            float ba = -1.f;
-            for (int k = 0; k < n; ++k)
-                if (c[k].ref >= 0 && area(c[k]) > ba) { ba = area(c[k]); best = k; }
-            if (best < 0) break;
-            Child g[2];
-            children_of(c[best].ref, g);
-            c[best] = g[0];
-            c[n++] = g[1];
-        }
-        uint32_t w[16];
-        for (int k = 0; k < 4; ++k) {
-            if (k < n) {
-                for (int ax = 0; ax < 3; ++ax) {
-                    int lo = (int)floorf((c[k].lo[ax] - out.qmin[ax]) * qinv[ax]) - QPAD;
-                    int hi = (int)ceilf((c[k].hi[ax] - out.qmin[ax]) * qinv[ax]) + QPAD;
-                    lo = std::min(std::max(lo, 0), 65535);
-                    hi = std::min(std::max(hi, 0), 65535);
-                    w[3 * k + ax] = (uint32_t)lo | ((uint32_t)hi << 16);
-                }
-                int ref = c[k].ref;
-                if (ref >= 0) {
-                    if (wide_of[ref] < 0) { wide_of[ref] = (int)todo.size(); todo.push_back(ref); }
-                    ref = wide_of[ref];
-                }
-                w[12 + k] = (uint32_t)ref;
-            } else {
-                for (int ax = 0; ax < 3; ++ax) w[3 * k + ax] = 65535u;   // lo = 65535, hi = 0: never hit
-                w[12 + k] = 0x7fffffffu;
-            }
-        }
-        words.insert(words.end(), w, w + 16);
-    }
-    out.n_nodes4 = (int)todo.size();
-    out.root4 = 0;
-    LBVH_CHECK(cudaMalloc((void**)&out.d_qnodes4, words.size() * sizeof(uint32_t)));
-    LBVH_CHECK(cudaMemcpyAsync(out.d_qnodes4, words.data(), words.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
-    LBVH_CHECK(cudaStreamSynchronize(stream));
     return true;
 }
 
@@ -804,7 +733,7 @@ static bool build_lbvh_tables(const float* d_verts, const int32_t* d_tri_obj, in
         LBVH_CHECK(cudaStreamSynchronize(stream));
         LBVH_CHECK(cudaGetLastError());
     }
-    return collapse_to_bvh4(stream, out, qi, err);
+    return measure_depth(stream, out, err);
 }
 
 // The traversal stack holds BVH_MAX_DEPTH levels.  A Karras tree over 63-bit keys + a 32-bit tie-break cannot be deeper
@@ -1025,7 +954,6 @@ static bool build_lbvh_f32(const float* d_verts, const int32_t* d_tri_obj, int n
 void free_lbvh(LbvhResult& r) {
     if (r.d_nodes) cudaFree(r.d_nodes);
     if (r.d_qnodes) cudaFree(r.d_qnodes);
-    if (r.d_qnodes4) cudaFree(r.d_qnodes4);
     if (r.d_tris) cudaFree(r.d_tris);
     if (r.d_tri_nrm) cudaFree(r.d_tri_nrm);
     r = LbvhResult();

@@ -15,9 +15,6 @@ struct LbvhResult {
     uint4* d_qnodes = nullptr;  // the node table the traversal reads: 2 x uint4 (32 B) per node, child boxes quantised to 16 bits
                                 // on the grid qmin + k * qstep (conservative), see quantise_nodes in lbvh.cu
     float qmin[3] = {0, 0, 0}, qstep[3] = {1, 1, 1};
-    uint4* d_qnodes4 = nullptr; // 4-wide table collapsed from the binary tree: 4 x uint4 (64 B) per node = 4 quantised child boxes + 4 references
-    int root4 = 0;              // root reference into d_qnodes4 (>= 0 node, < 0 leaf)
-    int n_nodes4 = 0;
     float4* d_tris = nullptr;   // TRI_STRIDE (4) x float4 per triangle in leaf order: (a | 1/|N|), (b-a | global tri id), (c-a | object id), pad
     float4* d_tri_nrm = nullptr; // 1 x float4 per triangle in leaf order: Triangle::normal (unit) | object id
     int root = 0;               // encoded reference: >= 0 node index, < 0 leaf ~((first << 3) | (count - 1))

@@ -418,8 +418,11 @@ __device__ __forceinline__ bool warp_reserve(uint32_t* cursor, uint32_t count, u
 //   * any hit for the NEE candidates in shadow queue c                  (mutually_visible; accumulates if unoccluded)
 //   * closest hit for dead-MIS probes against a mesh light              (hit.id == light_source test)
 // Lanes refill individually from one work cursor, so the two ray kinds share warps and the tail is paid once.
-template <bool COUNT, int MINB = 4, bool WIDE = false>
-__global__ void __launch_bounds__(WF_THREADS, MINB) k_traverse(const __grid_constant__ RenderArgs a, int c) {
+// CTAs per SM the product build is compiled for.  5 since the SAH tree (51 registers, a few spills, 40 warps per SM): bench
+// frame 540.4 -> 537.0 ms; on the PLOC tree 4 was ahead.  The counting build keeps 4.
+constexpr int TRAV_MINB = 5;
+template <bool COUNT>
+__global__ void __launch_bounds__(WF_THREADS, COUNT ? 4 : TRAV_MINB) k_traverse(const __grid_constant__ RenderArgs a, int c) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const uint32_t sbase = (uint32_t)__cvta_generic_to_shared(reinterpret_cast<int*>(smem_raw) + threadIdx.x), sstride = blockDim.x * 4u;
     int lstack[STACK_LOCAL];
@@ -432,7 +435,7 @@ __global__ void __launch_bounds__(WF_THREADS, MINB) k_traverse(const __grid_cons
     const int light_obj = a.S.hdr->light_obj;
     const uint32_t* const perm = a.bin_bits > 0 ? a.bin_perm : nullptr;   // bin order (see k_bin_*), or queue order
     const int refill_below = a.tune_refill > 0 ? a.tune_refill : REFILL_BELOW;
-    const int steps = a.tune_steps > 0 ? a.tune_steps : (WIDE ? INNER_STEPS / 2 : INNER_STEPS);
+    const int steps = a.tune_steps > 0 ? a.tune_steps : INNER_STEPS;
     uint32_t work[2] = {0, 0};
     unsigned long long dbg[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     // first chunk: static (warp w owns [w*32, w*32+32)), later chunks from the atomic cursor, which k_prepare
@@ -482,7 +485,7 @@ __global__ void __launch_bounds__(WF_THREADS, MINB) k_traverse(const __grid_cons
                             slot = my;
                             kind = 0;
                             const float4 o4 = Q.o[my], d4 = Q.d[my];
-                            trav_begin(a.S, T, f3(o4), f3(d4), __float_as_uint(o4.w), h2.x, WIDE ? a.S.root4 : a.S.root);
+                            trav_begin(a.S, T, f3(o4), f3(d4), __float_as_uint(o4.w), h2.x);
                         }
                     } else {
                         const float4 d4 = SQ.d[my - n_ext];
@@ -491,7 +494,7 @@ __global__ void __launch_bounds__(WF_THREADS, MINB) k_traverse(const __grid_cons
                             const float4 o4 = SQ.o[slot];
                             kind = (__float_as_uint(SQ.c[slot].w) & SHADOW_PROBE) ? 2 : 1;
                             occluded = false;
-                            trav_begin(a.S, T, f3(o4), f3(d4), __float_as_uint(o4.w), d4.w, WIDE ? a.S.root4 : a.S.root);
+                            trav_begin(a.S, T, f3(o4), f3(d4), __float_as_uint(o4.w), d4.w);
                         }
                     }
                 }
@@ -508,7 +511,7 @@ __global__ void __launch_bounds__(WF_THREADS, MINB) k_traverse(const __grid_cons
         // `steps` inner nodes per round, so lanes whose ray ended are not left idle behind one long descent.
         for (;;) {
             int trips = 0;
-            if (!COUNT && !WIDE && steps == INNER_STEPS) {   // default knob: unrolled, no loop counter
+            if (!COUNT && steps == INNER_STEPS) {   // default knob: unrolled, no loop counter
 #pragma unroll
                 for (int k = 0; k < INNER_STEPS; ++k) {
                     if (T.node < 0) break;
@@ -516,8 +519,7 @@ __global__ void __launch_bounds__(WF_THREADS, MINB) k_traverse(const __grid_cons
                 }
             } else {
                 for (int k = 0; k < steps && T.node >= 0; ++k) {
-                    if (WIDE) trav_inner4<COUNT>(a.S, T, sbase, sstride, lstack, work);
-                    else trav_inner<COUNT>(a.S, T, sbase, sstride, lstack, work);
+                    trav_inner<COUNT>(a.S, T, sbase, sstride, lstack, work);
                     ++trips;
                 }
             }
@@ -1476,8 +1478,7 @@ __global__ void __launch_bounds__(WF_THREADS) k_trace_rays(DevScene S, long long
         if (accel == 1) {   // RTB_ACCEL_OCTREE_REFERENCE
             oct_trace_meshes(S, o, d, PC_NONE, t, id, COUNT ? work : nullptr);
         } else if (ray_hits_bvh_box(S, o, d, t)) {
-            if (S.wide) bvh_traverse<false, COUNT, true>(S, sh, o, d, PC_NONE, t, id, 0.0f, work);
-            else bvh_traverse<false, COUNT, false>(S, sh, o, d, PC_NONE, t, id, 0.0f, work);
+            bvh_traverse<false, COUNT>(S, sh, o, d, PC_NONE, t, id, 0.0f, work);
         }
         if (id == PC_NONE) {
             obj[i] = -1; tri[i] = -1; tout[i] = INFINITY;

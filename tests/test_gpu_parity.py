@@ -451,27 +451,6 @@ geometry = { type = "sphere", pos = [0.0, 30.0, 0.0], r = 2.0 }
     assert np.quantile(rel, 0.999) < T_REL_TOL
 
 
-def test_wide_table_gives_the_same_hits(rtb, gpu_scene, monkeypatch):
-    # RTB_BVH_WIDE=1 traverses the 4-wide table collapsed from the binary tree (kept as an experiment knob, DESIGN.md §8):
-    # same triangles, same order of tests within a leaf -> identical ids and distances, and an identical frame
-    g2 = gpu_scene("flying_unicorn")
-    monkeypatch.setenv("RTB_BVH_WIDE", "1")
-    g4 = rtb.Scene.from_toml(scene_path("flying_unicorn"), device=0)
-    monkeypatch.delenv("RTB_BVH_WIDE")
-    rng = np.random.default_rng(5)
-    n = 100_000
-    lo, hi = np.array(g2.info.bvh_min), np.array(g2.info.bvh_max)
-    org = (lo + (hi - lo) * rng.random((n, 3)) * 1.6 - 0.3 * (hi - lo)).astype(np.float32)
-    d = rng.normal(size=(n, 3))
-    d = (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(np.float32)
-    a, b = g2.trace_rays(org, d), g4.trace_rays(org, d)
-    assert np.array_equal(a["obj"], b["obj"]) and np.array_equal(a["t"], b["t"])
-    assert (a["tri"] != b["tri"]).mean() < 1e-4          # only exact distance ties (shared edges) may pick the other triangle
-    assert (a["tri"] >= 0).mean() > 0.05
-    f2, f4 = g2.render(160, 120, 16, seed=2).astype(int), g4.render(160, 120, 16, seed=2).astype(int)
-    assert np.abs(f2 - f4).max() <= 1
-
-
 @pytest.mark.gpu
 def test_every_hierarchy_builder_gives_the_same_hits(rtb, gpu_scene, monkeypatch):
     # RTB_BVH picks the hierarchy over the same triangles: binned SAH (default, top-down on the device), PLOC, Karras, and the
