@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <climits>
 #include <atomic>
 #include <chrono>
 #include <cmath>
@@ -84,6 +85,7 @@ struct RenderContext {
     cudaGraphExec_t graph_exec[4] = {nullptr, nullptr, nullptr, nullptr};   // one iteration (4 kernels) for cur = 0 / 1; [2], [3]: the same with the inline-tail k_shade ...
     std::vector<unsigned char> graph_args;                 // ... captured for exactly these kernel arguments
     int grid_shade_nomesh = 0;   // grid of the mesh-less k_shade instantiation (160-thread CTAs)
+    int grid_shade_nee = 0;      // grid of the live-NEE mesh instantiations (SHADE_THREADS_NEE); grid_shade: the others
     int grid_oct = 0;    // k_traverse_octree's own persistent grid
     int grid_ext = 0, grid_ext_count = 0, grid_sh = 0, grid_sh_count = 0, grid_gen = 0, grid_shade = 0, grid_bin = 0;
     // adaptive sampling (ensure_adaptive): allocated by the first adaptive request only
@@ -504,12 +506,13 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
         // (MAX_OBJECTS primitives + materials), never to this scene's own (smaller) size.
         const int smem_max = (int)shared_tables_bytes(MAX_OBJECTS, MAX_OBJECTS);
         CU_TRY(cudaFuncSetAttribute(k_shade<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
-        CU_TRY(cudaFuncSetAttribute(k_shade<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        CU_TRY(cudaFuncSetAttribute(k_shade<1, 0, 0, true, SHADE_THREADS_NEE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_shade<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_generate<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         const int smem_tail = (int)shared_scene_bytes(MAX_OBJECTS, MAX_OBJECTS, SHADE_THREADS);
+        const int smem_tail_nee = (int)shared_scene_bytes(MAX_OBJECTS, MAX_OBJECTS, SHADE_THREADS_NEE);
         CU_TRY(cudaFuncSetAttribute(k_shade<0, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
-        CU_TRY(cudaFuncSetAttribute(k_shade<1, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
+        CU_TRY(cudaFuncSetAttribute(k_shade<1, 0, 0, true, SHADE_THREADS_NEE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail_nee));
         CU_TRY(cudaFuncSetAttribute(k_shade<2, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         int b = 0;
         CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<false>, WF_THREADS, smem_stack));
@@ -518,20 +521,35 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
         c->grid_ext_count = std::max(1, b) * prop.multiProcessorCount;
         CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse_octree<false>, WF_THREADS, (size_t)OCT_MAX_DEPTH * WF_THREADS * sizeof(int2)));
         c->grid_oct = std::max(1, b) * prop.multiProcessorCount;
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_shade<0>, SHADE_THREADS, smem_tab));
-        c->grid_shade = std::max(1, b) * prop.multiProcessorCount;
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_shade<1, 5, 3, false, SHADE_THREADS_NOMESH>, SHADE_THREADS_NOMESH, smem_tab));
-        c->grid_shade_nomesh = std::max(1, b) * prop.multiProcessorCount;
+        // the queued k_shade instantiations of one CTA shape share a grid: it is sized for the one with the fewest CTAs per SM
+        // (their register counts differ; the inline-tail instantiations, limited by their stacks, may run in more than one wave)
+        auto shade_grid = [&](std::initializer_list<const void*> kernels, int threads, int& grid) -> int {
+            int fewest = INT_MAX;
+            for (const void* k : kernels) {
+                CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k, threads, smem_tab));
+                fewest = std::min(fewest, b);
+            }
+            grid = std::max(1, fewest) * prop.multiProcessorCount;
+            return RTB_OK;
+        };
+        if (int e = shade_grid({(const void*)k_shade<0>, (const void*)k_shade<2>, (const void*)k_shade<2, 8, 0>, (const void*)k_shade<2, 5, 1>,
+                                (const void*)k_shade<2, 5, 2>, (const void*)k_shade<2, 5, 3>}, SHADE_THREADS, c->grid_shade)) return e;
+        if (int e = shade_grid({(const void*)k_shade<1, 0, 0, true, SHADE_THREADS_NEE>, (const void*)k_shade<1, 8, 0, true, SHADE_THREADS_NEE>,
+                                (const void*)k_shade<1, 5, 1, true, SHADE_THREADS_NEE>, (const void*)k_shade<1, 5, 2, true, SHADE_THREADS_NEE>,
+                                (const void*)k_shade<1, 5, 3, true, SHADE_THREADS_NEE>}, SHADE_THREADS_NEE, c->grid_shade_nee)) return e;
+        if (int e = shade_grid({(const void*)k_shade<1, 5, 3, false, SHADE_THREADS_NOMESH>, (const void*)k_shade<2, 5, 3, false, SHADE_THREADS_NOMESH>},
+                               SHADE_THREADS_NOMESH, c->grid_shade_nomesh)) return e;
         CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_generate<0, 0>, WF_THREADS, smem_tab));
         c->grid_gen = std::max(1, b) * prop.multiProcessorCount;
         c->grid_bin = 8 * prop.multiProcessorCount;
         // experiment knobs: CTAs per SM of the two persistent kernels (two concurrent renders can then share every SM)
         if (const char* e = getenv("RTB_TRAV_CTAS")) c->grid_ext = c->grid_ext_count = std::max(1, atoi(e)) * prop.multiProcessorCount;
-        if (const char* e = getenv("RTB_SHADE_CTAS")) c->grid_shade = std::max(1, atoi(e)) * prop.multiProcessorCount;
+        if (const char* e = getenv("RTB_SHADE_CTAS")) c->grid_shade = c->grid_shade_nee = std::max(1, atoi(e)) * prop.multiProcessorCount;
         c->initialised = true;
     }
     // every k_shade warp may leave up to two unfilled SHADE_SEG segments per queue class behind in each iteration
-    const uint32_t seg_room = (uint32_t)std::max(c->grid_shade * (SHADE_THREADS / 32), c->grid_shade_nomesh * (SHADE_THREADS_NOMESH / 32)) * 2u * SHADE_SEG;
+    const uint32_t seg_room = (uint32_t)std::max({c->grid_shade * (SHADE_THREADS / 32), c->grid_shade_nee * (SHADE_THREADS_NEE / 32),
+                                                  c->grid_shade_nomesh * (SHADE_THREADS_NOMESH / 32)}) * 2u * SHADE_SEG;
     {
         const uint32_t cap = P + 2u * seg_room;   // front + back class
         if (c->Palloc < cap) {   // (re)allocation of GBs of queue costs 100s of ms: never shrink, so a scene that serves
@@ -753,13 +771,14 @@ uint32_t inline_tail_below() {   // read per run: tests and A/B tools flip it in
     return e ? (uint32_t)std::max(0, atoi(e)) : (2u << 20);   // measured: gains saturate between 1 Mi and 4 Mi paths
 }
 
+// The CTA shape follows the mode (shade_cta): `grid` must be the grid of that shape, as a.shade_warps counts its warps.
 static void launch_shade(int mode, int n_planes, int n_spheres, int grid, size_t smem, cudaStream_t st, const RenderArgs& a, int cur, bool inline_tail = false) {
-#define RTB_SHADE(M, P, S) k_shade<M, P, S><<<grid, SHADE_THREADS, smem, st>>>(a, cur)
+#define RTB_SHADE(M, P, S) k_shade<M, P, S, true, shade_cta(M)><<<grid, shade_cta(M), smem, st>>>(a, cur)
     if (inline_tail) {   // the tail of a run: k_shade traverses the LBVH itself (generic analytic table; + the traversal stack in shared memory)
-        const size_t smem_t = shared_scene_bytes(a.S.n_prims, a.S.n_objects, SHADE_THREADS);
-        if (mode == 1) k_shade<1, 0, 0, true, SHADE_THREADS, true><<<grid, SHADE_THREADS, smem_t, st>>>(a, cur);
-        else if (mode == 2) k_shade<2, 0, 0, true, SHADE_THREADS, true><<<grid, SHADE_THREADS, smem_t, st>>>(a, cur);
-        else k_shade<0, 0, 0, true, SHADE_THREADS, true><<<grid, SHADE_THREADS, smem_t, st>>>(a, cur);
+        const size_t smem_t = shared_scene_bytes(a.S.n_prims, a.S.n_objects, shade_cta(mode));
+        if (mode == 1) k_shade<1, 0, 0, true, shade_cta(1), true><<<grid, shade_cta(1), smem_t, st>>>(a, cur);
+        else if (mode == 2) k_shade<2, 0, 0, true, shade_cta(2), true><<<grid, shade_cta(2), smem_t, st>>>(a, cur);
+        else k_shade<0, 0, 0, true, shade_cta(0), true><<<grid, shade_cta(0), smem_t, st>>>(a, cur);
         return;
     }
     if (shade_is_nomesh(mode, a)) {
@@ -813,10 +832,10 @@ int run_wavefront(rtb_scene* sc, RenderContext* c, RenderArgs& a, uint32_t ks_be
     bool fast_shade = !a.probe_px && a.estimator != RTB_EST_MIS_BALANCE && sc->fs.light_geom == GEOM_SPHERE && !getenv("RTB_NO_FAST_SHADE");
     for (const FlatMaterial& m : sc->fs.materials) fast_shade = fast_shade && m.brdf != BRDF_PHONG;
     const int shade_mode = !fast_shade ? 0 : (a.estimator == 0 ? 1 : 2);
-    // the mesh-less instantiation runs 160-thread CTAs: its grid and warp count (static first chunks, k_prepare) differ
+    // the CTA shape of k_shade depends on the instantiation: so do its grid and warp count (static first chunks, k_prepare)
     const bool nomesh = shade_is_nomesh(shade_mode, a);
-    const int grid_shade = nomesh ? c->grid_shade_nomesh : c->grid_shade;
-    a.shade_warps = (uint32_t)grid_shade * (uint32_t)((nomesh ? SHADE_THREADS_NOMESH : SHADE_THREADS) / 32);
+    const int grid_shade = nomesh ? c->grid_shade_nomesh : (shade_mode == 1 ? c->grid_shade_nee : c->grid_shade);
+    a.shade_warps = (uint32_t)grid_shade * (uint32_t)(shade_cta(shade_mode, !nomesh) / 32);
     // the inline tail: once at most `tail_below` paths are left, k_shade traverses the LBVH itself and the run ends in one launch
     // (the LBVH only: the reference's octree search and the counting build keep the queued form)
     // — and never more than a quarter of the pool: a run whose pool is that small would otherwise spend its WHOLE life in the

@@ -806,11 +806,19 @@ __global__ void __launch_bounds__(WF_THREADS, 4) k_traverse_octree(const __grid_
 // current one still has room for two trips, so the atomic's round trip is never waited for.  (Exact per-trip
 // reservations cost one global atomic per warp and trip, whose latency the warp ends up waiting for.)  The slots
 // left over when the kernel ends are marked as holes (HIT_HOLE / TLIM_HOLE), which the consumers skip.
-// All arguments but `lane` are warp-uniform; lane `cls` keeps the base of the reserved-ahead segment in `nb`.
+// The segment state is warp-uniform, so it lives in a per-warp shared-memory record (reads are broadcasts) instead of
+// nine registers of every lane; lane `cls` keeps the base of the reserved-ahead segment in `nb`.
 // DIR = +1: slots grow upward from the returned counter value; -1: downward (back class of the path queue).
+constexpr uint32_t SEG_NEXT = 0x80000000u;   // ShadeSegs::used: the next segment of the class is reserved
+struct ShadeSegs {
+    uint32_t base[3];   // element 0 of the current segment: front / back class of the other path queue, shadow queue
+    uint32_t used[3];   // slots of it handed out | SEG_NEXT
+};
 template <int DIR>
-__device__ __forceinline__ uint32_t seg_alloc(uint32_t& base, uint32_t& used, bool& has_next, uint32_t& nb, unsigned cls,
-                                              uint32_t* ctr, unsigned mask, unsigned lane) {
+__device__ __forceinline__ uint32_t seg_alloc(ShadeSegs& W, uint32_t& nb, unsigned cls, uint32_t* ctr, unsigned mask, unsigned lane) {
+    uint32_t base = W.base[cls], used = W.used[cls];
+    bool has_next = used & SEG_NEXT;
+    used &= ~SEG_NEXT;
     const uint32_t n = __popc(mask);
     const uint32_t r = used + __popc(mask & ((1u << lane) - 1u));
     const uint32_t step = (uint32_t)(DIR * (int)SHADE_SEG);
@@ -831,6 +839,9 @@ __device__ __forceinline__ uint32_t seg_alloc(uint32_t& base, uint32_t& used, bo
         if (lane == cls) nb = atomic_add_lane(ctr, step);
         has_next = true;
     }
+    __syncwarp();   // every lane has read the record before it changes (all lanes store the same values)
+    W.base[cls] = base;
+    W.used[cls] = used | (has_next ? SEG_NEXT : 0u);
     return slot;
 }
 // element k of the segment whose element 0 is `base`
@@ -856,6 +867,11 @@ __device__ __forceinline__ uint32_t seg_slot(uint32_t base, uint32_t k) { return
 // light, no probe items; 1 = live NEE estimator, 2 = the dead "MIS" branch.  MODE 0, the general instantiation, keeps
 // every branch at run time (both estimators, Phong, mesh lights, rtb_sample_radiance probes).
 constexpr int SHADE_THREADS_NOMESH = 160;   // the mesh-less instantiation needs 96 registers: 4 CTAs of 160 threads = 20 warps per SM
+// The live-NEE instantiations with a mesh (MODE 1, the bench frame's) fit 96 registers without spills too and run the same
+// shape.  The general and dead-MIS ones need 128 (at 96 they spill 140 bytes) and keep 2 CTAs of SHADE_THREADS.  (3 CTAs of
+// 192 threads are no middle way: ptxas caps them at 96 registers as well, since 18 warps put 5 on one SM sub-partition.)
+constexpr int SHADE_THREADS_NEE = 160;
+constexpr int shade_cta(int mode, bool mesh = true) { return !mesh ? SHADE_THREADS_NOMESH : (mode == 1 ? SHADE_THREADS_NEE : SHADE_THREADS); }
 // INLINE = true (the TAIL of a run, launched by the host once few paths are left): a ray that needs the LBVH is traversed right
 // here (bvh_traverse, intersect.cuh) instead of being queued for k_traverse, so every remaining path runs to its end inside ONE
 // launch — the ~100 iterations in which the last long paths used to die out a few hundred at a time (each four launches that
@@ -888,8 +904,8 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
     uint32_t* const ctr_front = &C->ext_head(1 - c);
     uint32_t* const ctr_back = &C->ext_tail(1 - c);
     uint32_t* const ctr_sh = &C->sh_head(1 - c);
-    uint32_t n_ext = 0, n_ext_bvh = 0, n_sh = 0, n_sh_bvh = 0, n_queued = 0;
-    uint32_t n_sh_inline = 0;   // INLINE: shadow / probe rays traversed here (counted as BVH shadow rays, never pending)
+    uint32_t n_ext = 0, n_ext_bvh = 0, n_sh = 0, n_sh_bvh = 0, n_queued = 0;   // rays of this warp: sums of its ballots
+    uint32_t n_sh_inline = 0;   // INLINE: shadow / probe rays this lane traversed here (counted as BVH shadow rays, never pending)
     auto slot_of = [&](uint32_t i) { return i < head ? i : tail + (i - head); };
 
     // ---- work fetch (warp-uniform): static first chunk, then chunks from the cursor, reserved one ahead
@@ -910,9 +926,14 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
     float4 o4 = make_float4(0, 0, 0, 0), d4 = o4, b4 = o4, tri_n = o4;   // cont: tri_n carries the stale `o` instead
     float4 ev_keep = o4;   // INLINE: a kept path may sit on a triangle, so the stale `o` / MIS pdf needs its own register
     uint32_t cur_slot = 0, sp_slot = 0;
-    // output segments (warp-uniform): front / back class of the other path queue, shadow queue
-    uint32_t f_base = 0, f_used = SHADE_SEG, b_base = 0, b_used = SHADE_SEG, s_base = 0, s_used = SHADE_SEG;
-    bool f_next = false, b_next = false, s_next = false;
+    // output segments of this warp (see seg_alloc); none is reserved yet
+    __shared__ ShadeSegs segs[THREADS / 32];
+    ShadeSegs& W = segs[threadIdx.x >> 5];
+    if (lane < 3) {
+        W.base[lane] = 0;
+        W.used[lane] = SHADE_SEG;
+    }
+    __syncwarp();
     uint32_t nb = 0;           // lane = class: base of the segment reserved ahead
     // A path that queued a shadow ray (or a dead-MIS probe) stays in registers like any other as long as the shadow queue has
     // room: its NEE candidate is resolved by k_traverse on its own (the entry carries contribution and accumulator index).  Once
@@ -972,25 +993,32 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
         // alive for the rest of their length; the next iteration packs them densely again.
         const bool park = drained && big_launch && __popc(have_work) < SHADE_PARK_BELOW;
 
-        bool ext_push = false, ext_front = false, sh_push = false, pr_push = false;
-        // outputs of this vertex; each is written before it is read under the same flag (no zero-fill: 40 registers)
-        float4 eo, ed, eb, ev = make_float4(0.f, 0.f, 0.f, 0.f);
-        float2 eh;
-        float4 so, sd, sc;
-        float4 pd, pc;  // probe entry shares `so`
-        eo.w = 0.f;     // flags word: tested (PC_STALE_O) whenever ext_push is set
+        // The trip runs in four phases, so that each output of the vertex dies right where it is stored: (A) divergent shading
+        // produces only raw quantities, (B) the analytic pair + box test, (C) the shadow push, (D) keep / park and the path push.
+        // A queue entry is put together at its store, from `pos`, the direction and the throughput; no packed copy of it stays live.
+        bool ext_push = false, want_sh = false, pr_push = false, pr_try = false;
+        // raw outputs of (A); each is written before it is read under the same flag
+        float3 pos, nbeta;
+        uint32_t pcode, eflags;   // hit's pcode; pcode + flags of the extension entry
+        float3 next_dir = f3(0.f, 0.f, 0.f), sh_dir = f3(0.f, 0.f, 0.f), sh_contrib;
+        float sh_tlim = 0.f;
+        float4 ev = make_float4(0.f, 0.f, 0.f, 0.f);   // stale `o` of a specular vertex | pdf of a balance-heuristic BRDF sample
+        float4 pd, pc;   // dead-MIS probe entry (its origin is `pos`)
+        const uint32_t acc = __float_as_uint(d4.w);
+        const uint32_t sdw = __float_as_uint(b4.w);
 
+        // ---- (A) divergent shading
         if (cur_valid) {
             const uint32_t id = __float_as_uint(h2.y);
             if (id != PC_NONE) {
                 const float t = h2.x;
                 const float3 o = f3(o4), d = f3(d4);
                 const uint32_t origin = __float_as_uint(o4.w);
-                const uint32_t acc = __float_as_uint(d4.w);
                 float3 beta = f3(b4);
-                const uint32_t sdw = __float_as_uint(b4.w);
                 const uint32_t sample = sdw >> 12, depth = sdw & 0xfffu;
                 const HitGeom hg = hit_geometry(sh, o, d, t, id, tri_n);
+                pos = hg.pos;
+                pcode = hg.pcode;
                 const DevMaterial& mat = sh.mats[hg.obj];
                 const float3 ovec = (origin & PC_STALE_O) ? (cont ? f3(INLINE ? ev_keep : tri_n) : f3(Q.ov[cur_slot])) : -d;
                 const float3 emitted = f3(mat.emitted);
@@ -1030,15 +1058,12 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                     }
                     const float4 r0 = make_float4(vr.light_u1, vr.light_u2, vr.rr, select_u);
                     const float4 rb = make_float4(vr.brdf_u1, vr.brdf_u2, lobe_u, 0.f);
-                    float3 next_dir = f3(0.f, 0.f, 0.f), sh_dir = f3(0.f, 0.f, 0.f), sh_contrib = f3(0.f, 0.f, 0.f);
-                    float sh_tlim = 0.f;
-                    bool want_sh = false;
                     if (mat.brdf == 1) {  // specular branch, src/scene.rs:170-185
                         if (r0.z < p) {
                             next_dir = flip_across(ovec, hg.n);
                             ext_push = true;
-                            eo = make_float4(hg.pos.x, hg.pos.y, hg.pos.z, __uint_as_float(hg.pcode | PC_SPEC_PENDING | PC_STALE_O));
-                            eb = make_float4(beta.x, beta.y, beta.z, __uint_as_float((sample << 12) | (depth + 1u)));
+                            eflags = hg.pcode | PC_SPEC_PENDING | PC_STALE_O;
+                            nbeta = beta;
                             ev = make_float4(ovec.x, ovec.y, ovec.z, 0.f);  // the recursion is handed `o`, not -i (src/scene.rs:178)
                         }
                     } else {
@@ -1070,11 +1095,10 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                             contrib = beta * Le * f * (dot(hg.n, inc) / (pdf_light + pdf_fresh));
                         }
                         if (contrib.x != 0.f || contrib.y != 0.f || contrib.z != 0.f) {
-                            want_sh = true;     // mutually_visible is resolved below, together with the extension ray
+                            want_sh = true;     // mutually_visible is resolved in (B), together with the extension ray
                             sh_dir = inc;
                             sh_tlim = dist - SHADOW_MARGIN;
                             sh_contrib = contrib;
-                            ++n_sh;
                         }
                         if (mis) {  // src/scene.rs:203-214: own BRDF sample; counts only if it reaches the light
                             float3 i2;
@@ -1090,7 +1114,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                                 float3 c2 = beta * Le * brdf_eval<FAST>(mat, hg.n, ovec, i2) * (dot(hg.n, i2) / (pdf2 + pdf_light2));
                                 if (c2.x != 0.f || c2.y != 0.f || c2.z != 0.f) {
                                     // trace_ray(x, i2) and test hit.id == light_source
-                                    ++n_sh;
+                                    pr_try = true;
                                     float ta;
                                     uint32_t ida;
                                     if (NP > 0 && NP < 8) analytic_closest_small<NP, NS>(a.ss, origin_group_of(sh, hg.pcode), hg.pos, i2, hg.pcode, ta, ida);
@@ -1123,10 +1147,6 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                                         pd = make_float4(i2.x, i2.y, i2.z, ta);
                                         pc = make_float4(c2.x, c2.y, c2.z, __uint_as_float(acc | SHADOW_PROBE));
                                     }
-                                    if (pr_push) {
-                                        ++n_sh_bvh;
-                                        so = make_float4(hg.pos.x, hg.pos.y, hg.pos.z, __uint_as_float(hg.pcode));
-                                    }
                                 }
                             }
                         }
@@ -1135,110 +1155,125 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                             float pdf1;
                             brdf_sample<FAST>(mat, hg.n, ovec, rb, next_dir, pdf1);
                             if (next_dir.x != 0.f || next_dir.y != 0.f || next_dir.z != 0.f) {
-                                float3 nb;
-                                if (FAST || mat.brdf == 0) nb = beta * f3(mat.k) * inv_p;  // f (n.i) / pdf == kd exactly
-                                else nb = beta * brdf_eval(mat, hg.n, ovec, next_dir) * (dot(hg.n, next_dir) / (pdf1 * p));
+                                if (FAST || mat.brdf == 0) nbeta = beta * f3(mat.k) * inv_p;  // f (n.i) / pdf == kd exactly
+                                else nbeta = beta * brdf_eval(mat, hg.n, ovec, next_dir) * (dot(hg.n, next_dir) / (pdf1 * p));
                                 ext_push = true;
-                                eo = make_float4(hg.pos.x, hg.pos.y, hg.pos.z, __uint_as_float(hg.pcode));
-                                eb = make_float4(nb.x, nb.y, nb.z, __uint_as_float((sample << 12) | (depth + 1u)));
+                                eflags = hg.pcode;
                                 if (mis2 && mat.brdf == 0) {   // the sample's pdf travels with the ray (see PC_MIS_PENDING)
-                                    eo.w = __uint_as_float(hg.pcode | PC_MIS_PENDING);
+                                    eflags = hg.pcode | PC_MIS_PENDING;
                                     ev = make_float4(0.f, 0.f, 0.f, pdf1);
                                 }
                             }
                         }
                     }
-                    if (ext_push || want_sh) {
-                        // Analytic half of BOTH trace_ray calls this vertex makes (extension: nearest hit; shadow:
-                        // mutually_visible, src/scene.rs:258-270), here where every lane does it together.  Rays that
-                        // can still reach the mesh box afterwards are queued for k_traverse.
-                        float ta;
-                        uint32_t ida;
-                        bool occ;
-                        if (NP == 8) analytic_pair_small8(a.ss, n_planes, n_prims, origin_group_of(sh, hg.pcode), hg.pos, hg.pcode, next_dir, ta, ida, sh_dir, sh_tlim, occ);
-                        else if (NP > 0) analytic_pair_small<NP, NS>(a.ss, origin_group_of(sh, hg.pcode), hg.pos, hg.pcode, next_dir, ta, ida, sh_dir, sh_tlim, occ);
-                        else analytic_pair(sh, n_planes, n_prims, hg.pos, hg.pcode, next_dir, ta, ida, sh_dir, sh_tlim, occ);
-                        bool ext_box, sh_box;   // can the two rays still reach the mesh box?  (both at once: shared terms, packed products)
-                        if (MESH) ray_pair_hits_bvh_box(a.S, hg.pos, next_dir, ta, sh_dir, sh_tlim, ext_box, sh_box);
-                        else ext_box = sh_box = false;   // no triangles in the scene: no ray ever leaves this kernel for k_traverse
-                        if (want_sh && !occ) {
-                            if (sh_box && INLINE) {   // mutually_visible's mesh half, right here
-                                ++n_sh_inline;
-                                uint32_t idt = PC_NONE;
-                                float tt = sh_tlim;
-                                if (!bvh_traverse<true, false>(a.S, sh, hg.pos, sh_dir, hg.pcode, tt, idt, sh_tlim + SHADOW_MARGIN, nullptr)) accum_add(a.accum, acc, sh_contrib);
-                            } else if (sh_box) {
-                                sh_push = true;
-                                ++n_sh_bvh;
-                                so = make_float4(hg.pos.x, hg.pos.y, hg.pos.z, __uint_as_float(hg.pcode));
-                                sd = make_float4(sh_dir.x, sh_dir.y, sh_dir.z, sh_tlim);
-                                sc = make_float4(sh_contrib.x, sh_contrib.y, sh_contrib.z, __uint_as_float(acc));
-                            } else {
-                                accum_add(a.accum, acc, sh_contrib);
-                            }
-                        }
-                        if (ext_push) {
-                            ext_front = ext_box;
-                            n_ext_bvh += ext_front ? 1u : 0u;
-                            if (INLINE && ext_front) {   // Mesh::intersect for the extension ray, right here: the hit is final afterwards
-                                bvh_traverse<false, false>(a.S, sh, hg.pos, next_dir, hg.pcode, ta, ida, 0.f, nullptr);
-                                ext_front = false;
-                            }
-                            ed = make_float4(next_dir.x, next_dir.y, next_dir.z, __uint_as_float(acc));
-                            eh = make_float2(ta, __uint_as_float(ida));
-                            ++n_ext;
-                        }
-                    }
                 }
             }
         }
-        // ---- where does the path go?  In registers if its next hit is final and it queued no shadow ray.
+        // shadow rays of this trip (NEE candidates, dead-MIS probes): counted from the warp's ballots
+        uint32_t trip_sh = __popc(__ballot_sync(0xffffffffu, want_sh));
+        unsigned mp = 0;
+        if (mis) {
+            // dead-MIS probes need no pair test: pushed here, so their entries are dead before (B)
+            trip_sh += __popc(__ballot_sync(0xffffffffu, pr_try));
+            mp = __ballot_sync(0xffffffffu, pr_push);
+            if (mp) {
+                const uint32_t slot = seg_alloc<1>(W, nb, 2u, ctr_sh, mp, lane);
+                if (pr_push) {
+                    if (slot < a.SPcap) { SQ.o[slot] = make_float4(pos.x, pos.y, pos.z, __uint_as_float(pcode)); SQ.d[slot] = pd; SQ.c[slot] = pc; }
+                    else atomicAdd(&C->overflow, 1u);
+                }
+                n_sh_bvh += __popc(mp);
+            }
+        }
+        n_sh += trip_sh;
+
+        // ---- (B) analytic half of BOTH trace_ray calls this vertex makes (extension: nearest hit; shadow: mutually_visible,
+        // src/scene.rs:258-270), here where every lane does it together.  Rays that can still reach the mesh box afterwards are
+        // queued for k_traverse.
+        float ta;
+        uint32_t ida;
+        bool ext_box = false;
+        if (ext_push || want_sh) {
+            bool occ, sh_box;   // can the two rays still reach the mesh box?  (both at once: shared terms, packed products)
+            if (NP == 8) analytic_pair_small8(a.ss, n_planes, n_prims, origin_group_of(sh, pcode), pos, pcode, next_dir, ta, ida, sh_dir, sh_tlim, occ);
+            else if (NP > 0) analytic_pair_small<NP, NS>(a.ss, origin_group_of(sh, pcode), pos, pcode, next_dir, ta, ida, sh_dir, sh_tlim, occ);
+            else analytic_pair(sh, n_planes, n_prims, pos, pcode, next_dir, ta, ida, sh_dir, sh_tlim, occ);
+            if (MESH) ray_pair_hits_bvh_box(a.S, pos, next_dir, ta, sh_dir, sh_tlim, ext_box, sh_box);
+            else ext_box = sh_box = false;   // no triangles in the scene: no ray ever leaves this kernel for k_traverse
+            if (want_sh) {   // from here on: the shadow ray goes to the queue
+                want_sh = false;
+                if (occ) {
+                } else if (sh_box && INLINE) {   // mutually_visible's mesh half, right here
+                    ++n_sh_inline;
+                    uint32_t idt = PC_NONE;
+                    float tt = sh_tlim;
+                    if (!bvh_traverse<true, false>(a.S, sh, pos, sh_dir, pcode, tt, idt, sh_tlim + SHADOW_MARGIN, nullptr)) accum_add(a.accum, acc, sh_contrib);
+                } else if (sh_box) {
+                    want_sh = true;
+                } else {
+                    accum_add(a.accum, acc, sh_contrib);
+                }
+            }
+        }
+        const bool sh_push = want_sh;
+
+        // ---- (C) shadow push; the shadow ray's values are dead afterwards
+        const unsigned ms = __ballot_sync(0xffffffffu, sh_push);
+        if (ms) {
+            const uint32_t slot = seg_alloc<1>(W, nb, 2u, ctr_sh, ms, lane);
+            if (sh_push) {
+                if (slot < a.SPcap) {
+                    SQ.o[slot] = make_float4(pos.x, pos.y, pos.z, __uint_as_float(pcode));
+                    SQ.d[slot] = make_float4(sh_dir.x, sh_dir.y, sh_dir.z, sh_tlim);
+                    SQ.c[slot] = make_float4(sh_contrib.x, sh_contrib.y, sh_contrib.z, __uint_as_float(acc));
+                } else {
+                    atomicAdd(&C->overflow, 1u);
+                }
+            }
+            n_sh_bvh += __popc(ms);
+        }
+
+        // ---- (D) extension: where does the path go?  In registers if its next hit is final and it queued no shadow ray.
+        n_ext += __popc(__ballot_sync(0xffffffffu, ext_push));
+        n_ext_bvh += __popc(__ballot_sync(0xffffffffu, ext_push && ext_box));
+        if (INLINE && ext_push && ext_box) bvh_traverse<false, false>(a.S, sh, pos, next_dir, pcode, ta, ida, 0.f, nullptr);   // the hit is final afterwards
+        const bool ext_front = !INLINE && ext_box;
         bool keep = ext_push && !ext_front && !park && (!(sh_push || pr_push) || !sh_tight);
-        if (ext_push && !ext_front && __float_as_uint(eh.y) == PC_NONE) {   // left the scene: nothing to shade
+        if (ext_push && !ext_front && ida == PC_NONE) {   // left the scene: nothing to shade
             keep = false;
             ext_push = false;
         }
         if (keep) ext_push = false;
-        // ---- queue pushes: slots from the warp's segments (see seg_alloc), written straight away
+        // slots from the warp's segments (see seg_alloc), written straight away
         const unsigned mf = __ballot_sync(0xffffffffu, ext_push && ext_front);
         const unsigned mb = __ballot_sync(0xffffffffu, ext_push && !ext_front);
-        const unsigned ms = __ballot_sync(0xffffffffu, sh_push);
-        const unsigned mp = __ballot_sync(0xffffffffu, pr_push);
         if (mf | mb) {
             uint32_t slot = 0;
-            if (mf) { const uint32_t v = seg_alloc<1>(f_base, f_used, f_next, nb, 0u, ctr_front, mf, lane); if (ext_front) slot = v; }
-            if (mb) { const uint32_t v = seg_alloc<-1>(b_base, b_used, b_next, nb, 1u, ctr_back, mb, lane); if (!ext_front) slot = v; }
+            if (mf) { const uint32_t v = seg_alloc<1>(W, nb, 0u, ctr_front, mf, lane); if (ext_front) slot = v; }
+            if (mb) { const uint32_t v = seg_alloc<-1>(W, nb, 1u, ctr_back, mb, lane); if (!ext_front) slot = v; }
             if (ext_push && slot >= a.Pcap) { atomicAdd(&C->overflow, 1u); ext_push = false; }
             if (ext_push) {
-                N.o[slot] = eo;
-                N.d[slot] = ed;
-                N.beta[slot] = eb;
-                N.hit[slot] = eh;
-                if (__float_as_uint(eo.w) & (PC_STALE_O | PC_MIS_PENDING)) N.ov[slot] = ev;
-                ++n_queued;
+                N.o[slot] = make_float4(pos.x, pos.y, pos.z, __uint_as_float(eflags));
+                N.d[slot] = make_float4(next_dir.x, next_dir.y, next_dir.z, __uint_as_float(acc));
+                N.beta[slot] = make_float4(nbeta.x, nbeta.y, nbeta.z, __uint_as_float(sdw + 1u));   // depth + 1 (< 4096: no carry)
+                N.hit[slot] = make_float2(ta, __uint_as_float(ida));
+                if (eflags & (PC_STALE_O | PC_MIS_PENDING)) N.ov[slot] = ev;
             }
+            n_queued += __popc(__ballot_sync(0xffffffffu, ext_push));
         }
-        if (ms) {
-            const uint32_t slot = seg_alloc<1>(s_base, s_used, s_next, nb, 2u, ctr_sh, ms, lane);
-            if (sh_push && slot >= a.SPcap) { atomicAdd(&C->overflow, 1u); sh_push = false; }
-            if (sh_push) { SQ.o[slot] = so; SQ.d[slot] = sd; SQ.c[slot] = sc; }
-        }
-        if (mp) {
-            const uint32_t slot = seg_alloc<1>(s_base, s_used, s_next, nb, 2u, ctr_sh, mp, lane);
-            if (pr_push && slot >= a.SPcap) { atomicAdd(&C->overflow, 1u); pr_push = false; }
-            if (pr_push) { SQ.o[slot] = so; SQ.d[slot] = pd; SQ.c[slot] = pc; }
-        }
-        if (ms | mp) sh_tight = s_base + SHADE_SEG > a.SP;   // warp-uniform: where this warp's current shadow segment ends
+        if (ms | mp) sh_tight = W.base[2] + SHADE_SEG > a.SP;   // warp-uniform: where this warp's current shadow segment ends
         // ---- next vertex of the same path, straight from registers
         cur_valid = keep;
         if (keep) {
-            o4 = eo; d4 = ed; b4 = eb; h2 = eh;
+            o4 = make_float4(pos.x, pos.y, pos.z, __uint_as_float(eflags));
+            d4 = make_float4(next_dir.x, next_dir.y, next_dir.z, __uint_as_float(acc));
+            b4 = make_float4(nbeta.x, nbeta.y, nbeta.z, __uint_as_float(sdw + 1u));
+            h2 = make_float2(ta, __uint_as_float(ida));
             if (INLINE) {    // the next hit may be a triangle (traversed above): its normal, and the stale `o` in its own register
                 ev_keep = ev;
-                const uint32_t idk = __float_as_uint(eh.y);
-                if (idk != PC_NONE && idk >= TRI_BASE) tri_n = __ldg(a.S.tri_nrm + (idk - TRI_BASE));
+                if (ida != PC_NONE && ida >= TRI_BASE) tri_n = __ldg(a.S.tri_nrm + (ida - TRI_BASE));
             } else {
-                tri_n = ev;  // stale `o` of a specular vertex (PC_STALE_O in eo.w); analytic hits need no triangle normal
+                tri_n = ev;  // stale `o` of a specular vertex (PC_STALE_O in eflags); analytic hits need no triangle normal
             }
             cont = true;
         }
@@ -1260,23 +1295,18 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
         const float4 hole4 = make_float4(0.f, 0.f, 0.f, __uint_as_float(TLIM_HOLE));
         auto mark_path = [&](uint32_t slot) { if (slot < a.Pcap) N.hit[slot] = hole; else atomicAdd(&C->overflow, 1u); };
         auto mark_sh = [&](uint32_t slot) { if (slot < a.SPcap) SQ.d[slot] = hole4; else atomicAdd(&C->overflow, 1u); };
-        for (uint32_t k = f_used + lane; k < SHADE_SEG; k += 32) mark_path(seg_slot<1>(f_base, k));
-        for (uint32_t k = b_used + lane; k < SHADE_SEG; k += 32) mark_path(seg_slot<-1>(b_base, k));
-        for (uint32_t k = s_used + lane; k < SHADE_SEG; k += 32) mark_sh(seg_slot<1>(s_base, k));
+        const uint32_t fu = W.used[0] & ~SEG_NEXT, bu = W.used[1] & ~SEG_NEXT, su = W.used[2] & ~SEG_NEXT;
+        for (uint32_t k = fu + lane; k < SHADE_SEG; k += 32) mark_path(seg_slot<1>(W.base[0], k));
+        for (uint32_t k = bu + lane; k < SHADE_SEG; k += 32) mark_path(seg_slot<-1>(W.base[1], k));
+        for (uint32_t k = su + lane; k < SHADE_SEG; k += 32) mark_sh(seg_slot<1>(W.base[2], k));
         const uint32_t nf = __shfl_sync(0xffffffffu, nb, 0), nbk = __shfl_sync(0xffffffffu, nb, 1) - 1u, ns = __shfl_sync(0xffffffffu, nb, 2);
-        if (f_next) for (uint32_t k = lane; k < SHADE_SEG; k += 32) mark_path(seg_slot<1>(nf, k));
-        if (b_next) for (uint32_t k = lane; k < SHADE_SEG; k += 32) mark_path(seg_slot<-1>(nbk, k));
-        if (s_next) for (uint32_t k = lane; k < SHADE_SEG; k += 32) mark_sh(seg_slot<1>(ns, k));
+        if (W.used[0] & SEG_NEXT) for (uint32_t k = lane; k < SHADE_SEG; k += 32) mark_path(seg_slot<1>(nf, k));
+        if (W.used[1] & SEG_NEXT) for (uint32_t k = lane; k < SHADE_SEG; k += 32) mark_path(seg_slot<-1>(nbk, k));
+        if (W.used[2] & SEG_NEXT) for (uint32_t k = lane; k < SHADE_SEG; k += 32) mark_sh(seg_slot<1>(ns, k));
     }
-    // counters
-    for (int off = 16; off; off >>= 1) {
-        n_ext += __shfl_down_sync(0xffffffffu, n_ext, off);
-        n_ext_bvh += __shfl_down_sync(0xffffffffu, n_ext_bvh, off);
-        n_sh += __shfl_down_sync(0xffffffffu, n_sh, off);
-        n_sh_bvh += __shfl_down_sync(0xffffffffu, n_sh_bvh, off);
-        if (INLINE) n_sh_inline += __shfl_down_sync(0xffffffffu, n_sh_inline, off);
-        n_queued += __shfl_down_sync(0xffffffffu, n_queued, off);
-    }
+    // counters (warp-uniform, but for the inline shadow rays)
+    if (INLINE)
+        for (int off = 16; off; off >>= 1) n_sh_inline += __shfl_down_sync(0xffffffffu, n_sh_inline, off);
     if (lane == 0) {
         if (n_queued) { atomicAdd(&C->live[1 - c], n_queued); atomicAdd(&C->paths_queued, (unsigned long long)n_queued); }
         if (n_sh_bvh) atomicAdd(&C->sh_live[1 - c], n_sh_bvh);

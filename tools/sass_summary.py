@@ -9,7 +9,7 @@ import collections, os, re, subprocess, sys, tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "raytracer-server_b200", "librtb200.so")
-KERNELS = sys.argv[1:] or ["k_shadeILi1ELi5ELi1ELb1ELi256", "k_traverseILb0E"]
+KERNELS = sys.argv[1:] or ["k_shadeILi1ELi5ELi1ELb1ELi160", "k_traverseILb0E"]
 
 
 def disassemble():
