@@ -234,6 +234,48 @@ typedef struct rtb_adaptive {
 int rtb_render_adaptive(rtb_scene* scene, const rtb_params* params, const rtb_adaptive* opts, uint8_t* rgb8_out,
                         int32_t* tile_spp, float* tile_error, volatile int* cancel);
 
+/* ---- denoising (not in the reference): an opt-in edge-aware filter of whole frames ------------------------------------
+ * Guides (rtb_scene_gbuffer), per pixel from the four sub-pixel centre rays of rtb_trace_primary(sx, sy, 0, 0), each
+ * followed through up to 8 specular (BRDF 1) vertices in the direction the renderer takes there (the stale-`o` quirk of
+ * src/scene.rs:178 included): albedo = mean over the rays of the first non-specular hit's albedo (diffuse k, Phong
+ * kd * color_d + ks * color_s) times ks of every mirror on the way, 1 for an emitter, a miss or an unfinished chain;
+ * normal = the renormalised mean of the hit normals facing the ray (0 for misses); depth = mean path length to the
+ * first non-specular hit over the rays that hit; obj = the object most of the four rays end on (ties: lowest sub-pixel,
+ * -1 = miss).  No RNG, independent of spp: a job computes them once.
+ * Filter: the pixel's linear value px exactly as the resolve forms it (per-sub-pixel clamp, mean of four) is demodulated,
+ * I = px / max(albedo, 1e-3); its luminance variance is the sample variance of the four clamped sub-pixel means' Rec. 709
+ * luminances / 4, divided by lum(max(albedo, 1e-3))^2.  Then `levels` a-trous levels (Dammertz et al. 2010; step 2^i at
+ * level i, 5x5 B3-spline taps 1/16 1/4 3/8 1/4 1/16), each tap q of pixel p weighted by
+ *     [obj_p == obj_q] * max(0, n_p . n_q)^sigma_normal * exp(-|z_p - z_q| / (sigma_depth * |grad z_p . (p - q)| + 1e-3))
+ *     * exp(-|l_p - l_q| / (sigma_color * sqrt(var_p) + 1e-4))
+ * (the centre tap with weight 1; l = Rec. 709 luminance of I; var_p = 3x3 Gaussian of the level's variance around p;
+ * grad z by central differences), the variance carried as sum w^2 var / (sum w)^2 (SVGF, Schied et al. 2017).  The
+ * result is multiplied by max(albedo, 1e-3) again and goes through the resolve's clamp, gamma and `as u8`.  No atomics:
+ * the filter is deterministic for given inputs.  Whole frames only (world = 1).  Invalid options give RTB_EINVAL with a
+ * message naming the field. */
+typedef struct rtb_denoise {
+    int32_t levels;       /* a-trous levels 1..8 (step 2^i); 0 = no filtering (the resolve through the denoise path) */
+    float sigma_color;    /* luminance edge-stop, in standard deviations */
+    float sigma_normal;   /* exponent of the normal edge-stop */
+    float sigma_depth;    /* depth edge-stop, in units of the local depth gradient */
+    int32_t reserved[4];  /* 0 */
+} rtb_denoise;
+/* rtb_render (adaptive = NULL) or rtb_render_adaptive with every frame denoised; tile_spp / tile_error as for
+ * rtb_render_adaptive (ignored without `adaptive`) */
+int rtb_render_denoised(rtb_scene* scene, const rtb_params* params, const rtb_adaptive* adaptive, const rtb_denoise* denoise,
+                        uint8_t* rgb8_out, int32_t* tile_spp, float* tile_error, volatile int* cancel);
+/* progressive (passes > 1) or adaptive job whose every published frame is denoised; passes = 1 renders one band */
+int rtb_job_begin_denoised(rtb_scene* scene, const rtb_params* params, int32_t passes, const rtb_adaptive* adaptive,
+                           const rtb_denoise* denoise, rtb_job** out);
+/* the guides above for a width x height frame under RTB_ACCEL_* `accel`; row 0 = top; any output may be NULL */
+int rtb_scene_gbuffer(rtb_scene* scene, int32_t width, int32_t height, int32_t accel, float* albedo3, float* normal3, float* depth,
+                      int32_t* obj);
+/* the filter alone on host buffers (scan-line order): linear colour, its luminance variance and the guides -> the denoised
+ * linear colour (before clamp and gamma).  For tests and for callers who denoise their own images. */
+int rtb_denoise_image(int device, int32_t width, int32_t height, const rtb_denoise* denoise, const float* color3,
+                      const float* variance, const float* albedo3, const float* normal3, const float* depth, const int32_t* obj,
+                      float* out3);
+
 /* device-resident variants (bench `value`, multi-GPU gather): the result stays in device memory
  * owned by the caller.  d_rgb8_tiles receives this rank's pixels in tile order
  * (rtb_local_pixels() * 3 bytes); d_subpixel_sums (optional) receives the fp32 sums of the four

@@ -39,6 +39,11 @@ class Adaptive(C.Structure):
     _fields_ = [("target_levels", C.c_float), ("pass_spp", C.c_int32), ("min_spp", C.c_int32), ("reserved", C.c_int32)]
 
 
+class Denoise(C.Structure):
+    _fields_ = [("levels", C.c_int32), ("sigma_color", C.c_float), ("sigma_normal", C.c_float), ("sigma_depth", C.c_float),
+                ("reserved", C.c_int32 * 4)]
+
+
 class SceneInfo(C.Structure):
     _fields_ = [("n_objects", C.c_int32), ("n_planes", C.c_int32), ("n_spheres", C.c_int32), ("n_meshes", C.c_int32),
                 ("n_triangles", C.c_int32), ("light_object", C.c_int32), ("bvh_nodes", C.c_int32),
@@ -84,6 +89,7 @@ EXPORTS = [
     "rtb_job_end", "rtb_trace_primary", "rtb_trace_rays", "rtb_sample_radiance", "rtb_fp32_peak",
     "rtb_untile_device_async", "rtb_job_stats", "rtb_sample_pixels", "rtb_trace_rays_accel", "rtb_scene_octree_stats", "rtb_scene_export", "rtb_scene_import",
     "rtb_render_adaptive", "rtb_job_begin_adaptive",
+    "rtb_render_denoised", "rtb_job_begin_denoised", "rtb_scene_gbuffer", "rtb_denoise_image",
 ]
 
 _lib = None
@@ -120,6 +126,10 @@ def lib():
     L.rtb_job_begin.argtypes = [vp, C.POINTER(Params), C.c_int32, C.POINTER(vp)]
     L.rtb_render_adaptive.argtypes = [vp, C.POINTER(Params), C.POINTER(Adaptive), C.POINTER(C.c_uint8), ip, fp, ip]
     L.rtb_job_begin_adaptive.argtypes = [vp, C.POINTER(Params), C.POINTER(Adaptive), C.POINTER(vp)]
+    L.rtb_render_denoised.argtypes = [vp, C.POINTER(Params), C.POINTER(Adaptive), C.POINTER(Denoise), C.POINTER(C.c_uint8), ip, fp, ip]
+    L.rtb_job_begin_denoised.argtypes = [vp, C.POINTER(Params), C.c_int32, C.POINTER(Adaptive), C.POINTER(Denoise), C.POINTER(vp)]
+    L.rtb_scene_gbuffer.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, fp, fp, fp, ip]
+    L.rtb_denoise_image.argtypes = [C.c_int, C.c_int32, C.c_int32, C.POINTER(Denoise), fp, fp, fp, fp, fp, ip, fp]
     L.rtb_job_next.argtypes = [vp, C.POINTER(C.c_uint16), C.POINTER(C.c_uint16), C.POINTER(C.c_uint8),
                                C.POINTER(C.c_uint8)]
     L.rtb_job_next_messages.argtypes = [vp, C.POINTER(C.c_uint8), C.c_int64, C.c_int32, C.POINTER(C.c_int64)]

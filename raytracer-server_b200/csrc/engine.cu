@@ -26,6 +26,7 @@
 #include "octree_host.hpp"
 #include "scene_host.hpp"
 #include "wavefront.cuh"
+#include "denoise.cuh"
 
 using namespace rtb;
 
@@ -97,6 +98,10 @@ struct RenderContext {
     int ad_tiles_cap = 0;
     volatile int* h_ad_count = nullptr;   // mapped pinned: active tiles after k_compact_tiles
     int* d_ad_count = nullptr;
+    // denoiser (ensure_denoise): allocated by the first denoised request only
+    float4* dn_guides = nullptr;       // [pixel] albedo | depth, then [pixel] normal | object id
+    float4* dn_buf = nullptr;          // two ping-pong [pixel] illumination | variance buffers
+    size_t dn_cap = 0;                 // pixels
 
     ~RenderContext() {
         cudaSetDevice(device);
@@ -104,6 +109,7 @@ struct RenderContext {
         cudaFree(qbuf); cudaFree(sbuf); cudaFree(accum); cudaFree(ctrl); cudaFree(d_rgb); cudaFree(d_probe);
         cudaFree(bin_buf); cudaFree(bin_hist);
         cudaFree(ad_mom); cudaFree(ad_list); cudaFree(ad_tile_ks); cudaFree(ad_tile_err);
+        cudaFree(dn_guides); cudaFree(dn_buf);
         if (h_ad_count) cudaFreeHost((void*)h_ad_count);
         if (h_active) cudaFreeHost(h_active);
         if (h_state) cudaFreeHost((void*)h_state);
@@ -1136,6 +1142,140 @@ int run_adaptive(rtb_scene* sc, RenderContext* c, RenderArgs& a, const rtb_adapt
     return RTB_OK;
 }
 
+// ---------------------------------------------------------------- denoiser
+// host-side checks only (a host-only scene reaches them): the error names the offending field; p = nullptr for
+// rtb_denoise_image (no frame request)
+int check_denoise(const rtb_params* p, const rtb_denoise* o) {
+    if (!o) return fail(RTB_EINVAL, "rtb_denoise options are NULL");
+    if (o->levels < 0 || o->levels > DENOISE_MAX_LEVELS) return fail(RTB_EINVAL, "rtb_denoise.levels must be in 0..8");
+    if (!std::isfinite(o->sigma_color) || o->sigma_color < 0.f) return fail(RTB_EINVAL, "rtb_denoise.sigma_color must be finite and >= 0");
+    if (!std::isfinite(o->sigma_normal) || o->sigma_normal < 0.f) return fail(RTB_EINVAL, "rtb_denoise.sigma_normal must be finite and >= 0");
+    if (!std::isfinite(o->sigma_depth) || o->sigma_depth < 0.f) return fail(RTB_EINVAL, "rtb_denoise.sigma_depth must be finite and >= 0");
+    for (int r : o->reserved)
+        if (r != 0) return fail(RTB_EINVAL, "rtb_denoise.reserved must be 0");
+    if (p && p->world != 1) return fail(RTB_EINVAL, "denoising filters whole frames (params.world must be 1)");
+    return RTB_OK;
+}
+
+int ensure_denoise(RenderContext* c, size_t pixels) {
+    if (c->dn_cap < pixels) {
+        cudaFree(c->dn_guides); cudaFree(c->dn_buf);
+        c->dn_guides = nullptr; c->dn_buf = nullptr;
+        c->dn_cap = 0;
+        CU_TRY(cudaMalloc((void**)&c->dn_guides, pixels * 2 * sizeof(float4)));
+        CU_TRY(cudaMalloc((void**)&c->dn_buf, pixels * 2 * sizeof(float4)));
+        c->dn_cap = pixels;
+    }
+    return RTB_OK;
+}
+
+// the guides of a width x height frame into c->dn_guides, enqueued on `st` (callers asking for RTB_ACCEL_OCTREE_REFERENCE have
+// run need_accel)
+int launch_gbuffer(rtb_scene* sc, RenderContext* c, int width, int height, int accel, cudaStream_t st) {
+    DevScene S;
+    {
+        std::lock_guard<std::mutex> lk(sc->mu);
+        S = sc->view;
+    }
+    const size_t pixels = (size_t)width * height;
+    CU_TRY(cudaFuncSetAttribute(k_gbuffer, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shared_scene_bytes(MAX_OBJECTS, MAX_OBJECTS, WF_THREADS)));
+    const Camera cam = make_camera(sc->fs.cam_pos, sc->fs.cam_dir, width, height);
+    const int grid = (int)std::min<size_t>((pixels + WF_THREADS - 1) / WF_THREADS, 148 * 8);
+    k_gbuffer<<<grid, WF_THREADS, shared_scene_bytes(S.n_prims, S.n_objects, WF_THREADS), st>>>(S, cam, width, height, accel, c->dn_guides,
+                                                                                              c->dn_guides + pixels);
+    CU_TRY(cudaGetLastError());
+    return RTB_OK;
+}
+
+DenoiseArgs denoise_args(RenderContext* c, int width, int height) {
+    DenoiseArgs d{};
+    const size_t pixels = (size_t)width * height;
+    d.width = width;
+    d.height = height;
+    d.tiles_x = (width + TILE - 1) / TILE;
+    d.ga = c->dn_guides;
+    d.gn = c->dn_guides + pixels;
+    d.buf[0] = c->dn_buf;
+    d.buf[1] = c->dn_buf + pixels;
+    return d;
+}
+
+// the filter over d's buffers, enqueued on `st`: prep, o.levels à-trous levels, output; returns the kernels launched
+int launch_filter(const DenoiseArgs& d, const rtb_denoise& o, unsigned char* rgb8, float* out3, cudaStream_t st) {
+    const int n = d.width * d.height, grid = (n + DENOISE_THREADS - 1) / DENOISE_THREADS;
+    const DenoiseSigmas s{o.sigma_color, o.sigma_normal, o.sigma_depth};
+    k_denoise_prep<<<grid, DENOISE_THREADS, 0, st>>>(d);
+    for (int level = 0; level < o.levels; ++level)
+        k_atrous<<<grid, DENOISE_THREADS, 0, st>>>(d, d.buf[level & 1], d.buf[(level + 1) & 1], 1 << level, s);
+    k_denoise_out<<<grid, DENOISE_THREADS, 0, st>>>(d, d.buf[o.levels & 1], rgb8, out3);
+    return o.levels + 2;
+}
+
+// the denoised frame of the accumulators r describes (sample counts as r.ks_done / r.tile_ks give them) into rgb8 (scan-line);
+// the guides must already be in c->dn_guides
+int launch_denoise(RenderContext* c, const RenderArgs& r, const rtb_denoise& o, unsigned char* rgb8, cudaStream_t st) {
+    DenoiseArgs d = denoise_args(c, r.width, r.height);
+    d.accum = r.accum;
+    d.ks_done = r.ks_done;
+    d.tile_ks = r.tile_ks;
+    return launch_filter(d, o, rgb8, nullptr, st);
+}
+
+// Whole-frame render (world = 1) of rtb_render_adaptive and rtb_render_denoised: the adaptive passes (opts) or one uniform
+// pass, then k_resolve (dn = nullptr) or the denoiser, read back into rgb8_out.  Options are checked by the caller.
+int render_whole_frame(rtb_scene* scene, const rtb_params* params, const rtb_adaptive* opts, const rtb_denoise* dn, uint8_t* rgb8_out,
+                       int32_t* tile_spp, float* tile_error, volatile int* cancel) {
+    int rc = need_device(scene);
+    if (rc != RTB_OK) return rc;
+    if ((rc = need_accel(scene, params)) != RTB_OK) return rc;
+    const uint32_t P = opts ? adaptive_pool(params, opts) : default_pool(params);
+    const uint32_t SP = params->estimator == RTB_EST_NEE ? P : 2 * P;
+    const size_t frame = (size_t)params->width * params->height * 3;
+    const int n_tiles = local_tiles(params);
+    RenderContext* c = acquire_context(scene, P);
+    RenderArgs a;
+    rtb_stats st{};
+    bool cancelled = false;
+    if (opts) {
+        rc = ensure_context(scene, c, P, SP, (size_t)params->width * params->height * 4, requested_bin_bits(scene, params) > 0);
+        if (rc == RTB_OK) {
+            fill_args(scene, params, c, a);
+            rc = run_adaptive(scene, c, a, *opts, cancel, st, cancelled, {});
+        }
+    } else {
+        rc = render_into_context(scene, params, c, a, cancel, st, cancelled);
+    }
+    if (rc == RTB_OK && !cancelled) rc = ensure_rgb(c, frame, true);
+    if (rc == RTB_OK && !cancelled) {
+        if (!dn) rc = resolve_to(c, a, c->d_rgb, nullptr, 1, st);
+        else if ((rc = ensure_denoise(c, (size_t)params->width * params->height)) == RTB_OK &&
+                 (rc = launch_gbuffer(scene, c, params->width, params->height, params->accel, c->stream)) == RTB_OK) {
+            cudaEvent_t e0 = c->ev_begin, e1 = c->ev_end;
+            cudaError_t e = cudaEventRecord(e0, c->stream);
+            if (e == cudaSuccess) st.kernel_launches += 1 + launch_denoise(c, a, *dn, c->d_rgb, c->stream);
+            if (e == cudaSuccess) e = cudaEventRecord(e1, c->stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+            if (e == cudaSuccess) e = cudaGetLastError();
+            float ms = 0;
+            if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, e0, e1);
+            if (e != cudaSuccess) rc = fail(RTB_ECUDA, std::string("denoiser: ") + cudaGetErrorString(e));
+            st.resolve_ms += ms;
+        }
+    }
+    if (rc == RTB_OK && !cancelled) {
+        cudaError_t e = cudaMemcpyAsync(c->h_rgb, c->d_rgb, frame, cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess && opts && tile_spp) e = cudaMemcpyAsync(tile_spp, c->ad_tile_ks, (size_t)n_tiles * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess && opts && tile_error) e = cudaMemcpyAsync(tile_error, c->ad_tile_err, (size_t)n_tiles * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+        if (e != cudaSuccess) rc = fail(RTB_ECUDA, std::string("frame read-back: ") + cudaGetErrorString(e));
+        else std::memcpy(rgb8_out, c->h_rgb, frame);
+    }
+    publish_stats(scene, st);
+    release_context(scene, c);
+    if (rc != RTB_OK) return rc;
+    return cancelled ? RTB_ECANCELLED : RTB_OK;
+}
+
 }  // namespace
 
 // ======================================================================================= C ABI
@@ -1483,35 +1623,95 @@ int rtb_render_adaptive(rtb_scene* scene, const rtb_params* params, const rtb_ad
     int rc = check_params(params);
     if (rc == RTB_OK) rc = check_adaptive(params, opts);
     if (rc != RTB_OK) return rc;
-    if ((rc = need_device(scene)) != RTB_OK) return rc;
-    if ((rc = need_accel(scene, params)) != RTB_OK) return rc;
-    const uint32_t P = adaptive_pool(params, opts);
-    const uint32_t SP = params->estimator == RTB_EST_NEE ? P : 2 * P;
-    const size_t frame = (size_t)params->width * params->height * 3;
-    const int n_tiles = local_tiles(params);
-    RenderContext* c = acquire_context(scene, P);
-    RenderArgs a;
-    rtb_stats st{};
-    bool cancelled = false;
-    rc = ensure_context(scene, c, P, SP, (size_t)params->width * params->height * 4, requested_bin_bits(scene, params) > 0);
+    return render_whole_frame(scene, params, opts, nullptr, rgb8_out, tile_spp, tile_error, cancel);
+}
+
+int rtb_render_denoised(rtb_scene* scene, const rtb_params* params, const rtb_adaptive* adaptive, const rtb_denoise* denoise,
+                        uint8_t* rgb8_out, int32_t* tile_spp, float* tile_error, volatile int* cancel) {
+    if (!scene || !rgb8_out) return fail(RTB_EINVAL, "NULL argument");
+    int rc = check_params(params);
+    if (rc == RTB_OK && adaptive) rc = check_adaptive(params, adaptive);
+    if (rc == RTB_OK) rc = check_denoise(params, denoise);
+    if (rc != RTB_OK) return rc;
+    return render_whole_frame(scene, params, adaptive, denoise, rgb8_out, tile_spp, tile_error, cancel);
+}
+
+int rtb_scene_gbuffer(rtb_scene* scene, int32_t width, int32_t height, int32_t accel, float* albedo3, float* normal3, float* depth,
+                      int32_t* obj) {
+    if (!scene) return fail(RTB_EINVAL, "NULL scene");
+    if (width <= 0 || height <= 0 || width > 65535 || height > 65535 || (long long)width * height >= (1ll << 31))
+        return fail(RTB_EINVAL, "width/height must be in 1..65535");
+    if (accel != RTB_ACCEL_LBVH && accel != RTB_ACCEL_OCTREE_REFERENCE) return fail(RTB_EINVAL, "unknown accel mode");
+    if (int rc0 = need_device(scene)) return rc0;
+    rtb_params p{};
+    p.accel = accel;
+    if (int rc1 = need_accel(scene, &p)) return rc1;
+    const size_t pixels = (size_t)width * height;
+    RenderContext* c = acquire_context(scene);
+    int rc = ensure_context(scene, c, 1024, 1024, 0);
+    if (rc == RTB_OK) rc = ensure_denoise(c, pixels);
+    if (rc == RTB_OK) rc = launch_gbuffer(scene, c, width, height, accel, c->stream);
+    std::vector<float4> host(pixels * 2);
     if (rc == RTB_OK) {
-        fill_args(scene, params, c, a);
-        rc = run_adaptive(scene, c, a, *opts, cancel, st, cancelled, {});
-    }
-    if (rc == RTB_OK && !cancelled) rc = ensure_rgb(c, frame, true);
-    if (rc == RTB_OK && !cancelled) rc = resolve_to(c, a, c->d_rgb, nullptr, 1, st);
-    if (rc == RTB_OK && !cancelled) {
-        cudaError_t e = cudaMemcpyAsync(c->h_rgb, c->d_rgb, frame, cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess && tile_spp) e = cudaMemcpyAsync(tile_spp, c->ad_tile_ks, (size_t)n_tiles * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess && tile_error) e = cudaMemcpyAsync(tile_error, c->ad_tile_err, (size_t)n_tiles * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
+        cudaError_t e = cudaMemcpyAsync(host.data(), c->dn_guides, pixels * 2 * sizeof(float4), cudaMemcpyDeviceToHost, c->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-        if (e != cudaSuccess) rc = fail(RTB_ECUDA, std::string("frame read-back: ") + cudaGetErrorString(e));
-        else std::memcpy(rgb8_out, c->h_rgb, frame);
+        if (e != cudaSuccess) rc = fail(RTB_ECUDA, std::string("rtb_scene_gbuffer: ") + cudaGetErrorString(e));
     }
-    publish_stats(scene, st);
     release_context(scene, c);
     if (rc != RTB_OK) return rc;
-    return cancelled ? RTB_ECANCELLED : RTB_OK;
+    for (size_t i = 0; i < pixels; ++i) {
+        const float4 ga = host[i], gn = host[pixels + i];
+        if (albedo3) { albedo3[3 * i] = ga.x; albedo3[3 * i + 1] = ga.y; albedo3[3 * i + 2] = ga.z; }
+        if (normal3) { normal3[3 * i] = gn.x; normal3[3 * i + 1] = gn.y; normal3[3 * i + 2] = gn.z; }
+        if (depth) depth[i] = ga.w;
+        if (obj) std::memcpy(&obj[i], &gn.w, 4);
+    }
+    return RTB_OK;
+}
+
+int rtb_denoise_image(int device, int32_t width, int32_t height, const rtb_denoise* denoise, const float* color3, const float* variance,
+                      const float* albedo3, const float* normal3, const float* depth, const int32_t* obj, float* out3) {
+    int rc = check_denoise(nullptr, denoise);
+    if (rc != RTB_OK) return rc;
+    if (!color3 || !variance || !albedo3 || !normal3 || !depth || !obj || !out3) return fail(RTB_EINVAL, "NULL argument");
+    if (width <= 0 || height <= 0 || (long long)width * height >= (1ll << 31)) return fail(RTB_EINVAL, "bad image size");
+    const size_t pixels = (size_t)width * height;
+    std::vector<float4> host(pixels * 3);   // guides (albedo | depth, normal | object), then colour | variance
+    for (size_t i = 0; i < pixels; ++i) {
+        float o;
+        std::memcpy(&o, &obj[i], 4);
+        host[i] = make_float4(albedo3[3 * i], albedo3[3 * i + 1], albedo3[3 * i + 2], depth[i]);
+        host[pixels + i] = make_float4(normal3[3 * i], normal3[3 * i + 1], normal3[3 * i + 2], o);
+        host[2 * pixels + i] = make_float4(color3[3 * i], color3[3 * i + 1], color3[3 * i + 2], variance[i]);
+    }
+    CU_TRY(cudaSetDevice(device));
+    float4 *d_guides = nullptr, *d_buf = nullptr;
+    float* d_out = nullptr;
+    cudaStream_t st = nullptr;
+    cudaError_t e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
+    auto T = [&](cudaError_t x) { if (e == cudaSuccess) e = x; };
+    T(cudaMalloc((void**)&d_guides, pixels * 2 * sizeof(float4)));
+    T(cudaMalloc((void**)&d_buf, pixels * 2 * sizeof(float4)));
+    T(cudaMalloc((void**)&d_out, pixels * 3 * sizeof(float)));
+    T(cudaMemcpyAsync(d_guides, host.data(), pixels * 2 * sizeof(float4), cudaMemcpyHostToDevice, st));
+    T(cudaMemcpyAsync(d_buf + pixels, host.data() + 2 * pixels, pixels * sizeof(float4), cudaMemcpyHostToDevice, st));
+    if (e == cudaSuccess) {
+        DenoiseArgs d{};
+        d.width = width;
+        d.height = height;
+        d.ga = d_guides;
+        d.gn = d_guides + pixels;
+        d.buf[0] = d_buf;
+        d.buf[1] = d_buf + pixels;   // d.accum = nullptr: k_denoise_prep reads the colour and variance from here
+        launch_filter(d, *denoise, nullptr, d_out, st);
+        T(cudaGetLastError());
+    }
+    T(cudaMemcpyAsync(out3, d_out, pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+    T(cudaStreamSynchronize(st));
+    cudaFree(d_guides); cudaFree(d_buf); cudaFree(d_out);
+    if (st) cudaStreamDestroy(st);
+    if (e != cudaSuccess) return fail(RTB_ECUDA, std::string("rtb_denoise_image: ") + cudaGetErrorString(e));
+    return RTB_OK;
 }
 
 int rtb_untile_device_async(const rtb_params* params, const void* d_shards, int64_t shard_stride, void* d_rgb8_frame, int device,
@@ -1781,6 +1981,8 @@ struct rtb_job {
     int passes = 1;
     rtb_adaptive adaptive{};   // pass_spp > 0: adaptive job (passes = the most the budget allows; the device decides how many run)
     bool converged = false;    // adaptive job: no tile was left active, the frame is final (guarded by mu)
+    bool denoise = false;      // every published frame goes through the denoiser (`dn`) instead of k_resolve; one band
+    rtb_denoise dn{};
     std::vector<std::thread> workers;
     std::mutex mu;
     std::condition_variable cv;
@@ -1885,6 +2087,11 @@ void job_worker(rtb_job* j, int worker) {
     const size_t accum_elems = (size_t)p.width * p.height * 4;
     int rc = ensure_context(sc, c, P, SP, accum_elems, requested_bin_bits(sc, &p) > 0);
     if (rc == RTB_OK) rc = ensure_rgb(c, frame * (progressive ? 2 : 1), false);
+    if (rc == RTB_OK && j->denoise) rc = ensure_denoise(c, (size_t)p.width * p.height);
+    if (rc == RTB_OK && j->denoise) {   // once: the guides need no RNG.  Complete before any resolve, which may run on copy_stream
+        rc = launch_gbuffer(sc, c, p.width, p.height, p.accel, c->stream);
+        if (rc == RTB_OK && cudaStreamSynchronize(c->stream) != cudaSuccess) rc = fail(RTB_ECUDA, "streaming job: guides");
+    }
     if (rc != RTB_OK) return finish(rc);
     RenderArgs a;
     fill_args(sc, &p, c, a);
@@ -1911,7 +2118,8 @@ void job_worker(rtb_job* j, int worker) {
             if (cancelled || j->cancel) return finish(RTB_ECANCELLED);
             // resolve + copy + publish on the side stream; this thread goes straight on to its next band
             const int n = a.n_local_tiles * 1024;
-            k_resolve<<<(n + 255) / 256, 256, 0, c->copy_stream>>>(a, c->d_rgb, nullptr, 1);
+            if (j->denoise) bs.kernel_launches += launch_denoise(c, a, j->dn, c->d_rgb, c->copy_stream) - 1;
+            else k_resolve<<<(n + 255) / 256, 256, 0, c->copy_stream>>>(a, c->d_rgb, nullptr, 1);
             const size_t off = (size_t)row0 * p.width * 3, bytes = (size_t)(row1 - row0) * p.width * 3;
             e = cudaMemcpyAsync(j->h_frame[0] + off, c->d_rgb + off, bytes, cudaMemcpyDeviceToHost, c->copy_stream);
             if (e == cudaSuccess) e = cudaEventRecord(j->band_copied[b], c->copy_stream);
@@ -1939,7 +2147,9 @@ void job_worker(rtb_job* j, int worker) {
             add_stats(j->stats, ps);
         }
         const int n = a.n_local_tiles * 1024;
-        k_resolve<<<(n + 255) / 256, 256, 0, c->stream>>>(r, c->d_rgb + (size_t)b * frame, nullptr, 1);   // in stream order: before the next pass adds samples
+        // in stream order: before the next pass adds samples
+        if (j->denoise) launch_denoise(c, r, j->dn, c->d_rgb + (size_t)b * frame, c->stream);
+        else k_resolve<<<(n + 255) / 256, 256, 0, c->stream>>>(r, c->d_rgb + (size_t)b * frame, nullptr, 1);
         cudaError_t e = cudaEventRecord(j->ev_resolved[b], c->stream);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(c->copy_stream, j->ev_resolved[b], 0);
         if (e == cudaSuccess) e = cudaMemcpyAsync(j->h_frame[b], c->d_rgb + (size_t)b * frame, frame, cudaMemcpyDeviceToHost, c->copy_stream);
@@ -2054,8 +2264,10 @@ int job_next_record(rtb_job* job, bool block, uint16_t* x, uint16_t* y, uint8_t*
     return 1;
 }
 
-// adaptive: nullptr for a uniform job; otherwise checked options (check_adaptive) and passes = spp / pass_spp
-int job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, const rtb_adaptive* adaptive, rtb_job** out) {
+// adaptive: nullptr for a uniform job; otherwise checked options (check_adaptive) and passes = spp / pass_spp.
+// dn: nullptr, or checked options (check_denoise) for a denoised job
+int job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, const rtb_adaptive* adaptive, const rtb_denoise* dn,
+              rtb_job** out) {
     if (!scene || !out) return fail(RTB_EINVAL, "NULL argument");
     if (int rc0 = need_device(scene)) return rc0;
     int rc = check_params(params);
@@ -2068,6 +2280,10 @@ int job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, const 
     j->params = *params;
     j->passes = std::max(1, passes);
     if (adaptive) j->adaptive = *adaptive;
+    if (dn) {
+        j->denoise = true;
+        j->dn = *dn;
+    }
     j->frame_bytes = (size_t)params->width * params->height * 3;
     j->stats.first_record_ms = -1.0;
     const bool progressive = j->passes > 1;
@@ -2084,7 +2300,7 @@ int job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, const 
     if (const char* e = getenv("RTB_BAND_TILE_ROWS")) { rows = std::max(1, atoi(e)); growth_cap = 1; }   // test / experiment knobs
     if (const char* e = getenv("RTB_BAND_GROWTH_CAP")) growth_cap = std::max(1, atoi(e));
     j->band_ty.assign(1, 0);
-    if (progressive || 2 * rows > tiles_y) j->band_ty.push_back(tiles_y);   // one band
+    if (progressive || j->denoise || 2 * rows > tiles_y) j->band_ty.push_back(tiles_y);   // one band (the denoiser filters whole frames)
     else
         for (int ty = 0, k = 0, mult = 1; ty < tiles_y; ++k) {
             if (k >= 2) mult = std::min(mult * 2, growth_cap);
@@ -2122,7 +2338,7 @@ int job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, const 
 extern "C" {
 
 int rtb_job_begin(rtb_scene* scene, const rtb_params* params, int32_t passes, rtb_job** out) {
-    return job_begin(scene, params, passes, nullptr, out);
+    return job_begin(scene, params, passes, nullptr, nullptr, out);
 }
 
 int rtb_job_begin_adaptive(rtb_scene* scene, const rtb_params* params, const rtb_adaptive* opts, rtb_job** out) {
@@ -2130,7 +2346,17 @@ int rtb_job_begin_adaptive(rtb_scene* scene, const rtb_params* params, const rtb
     int rc = check_params(params);
     if (rc == RTB_OK) rc = check_adaptive(params, opts);
     if (rc != RTB_OK) return rc;
-    return job_begin(scene, params, params->spp / opts->pass_spp, opts, out);
+    return job_begin(scene, params, params->spp / opts->pass_spp, opts, nullptr, out);
+}
+
+int rtb_job_begin_denoised(rtb_scene* scene, const rtb_params* params, int32_t passes, const rtb_adaptive* adaptive,
+                           const rtb_denoise* denoise, rtb_job** out) {
+    if (!scene || !out) return fail(RTB_EINVAL, "NULL argument");
+    int rc = check_params(params);
+    if (rc == RTB_OK && adaptive) rc = check_adaptive(params, adaptive);
+    if (rc == RTB_OK) rc = check_denoise(params, denoise);
+    if (rc != RTB_OK) return rc;
+    return job_begin(scene, params, adaptive ? params->spp / adaptive->pass_spp : passes, adaptive, denoise, out);
 }
 
 // returns 1 = record produced, 0 = frame(s) complete, RTB_ESTOPPED after a cancel, or another negative error

@@ -13,7 +13,7 @@ import threading
 import numpy as np
 
 from . import _abi
-from ._abi import ACCEL_LBVH, ACCEL_OCTREE_REFERENCE, EST_MIS_BALANCE, EST_MIS_DEAD, EST_NEE, Adaptive, ObjectDesc, ObjectInfo, Params, SceneDesc, SceneInfo, Stats
+from ._abi import ACCEL_LBVH, ACCEL_OCTREE_REFERENCE, EST_MIS_BALANCE, EST_MIS_DEAD, EST_NEE, Adaptive, Denoise, ObjectDesc, ObjectInfo, Params, SceneDesc, SceneInfo, Stats
 
 
 class RtbError(RuntimeError):
@@ -68,6 +68,25 @@ def make_adaptive(spp: int, *, target_levels: float, pass_spp: int = 16, min_spp
     o.min_spp = min(4 * pass_spp, spp) if min_spp is None else min_spp
     o.reserved = 0
     return o
+
+
+def make_denoise(levels: int = 5, *, sigma_color: float = 4.0, sigma_normal: float = 128.0, sigma_depth: float = 1.0) -> Denoise:
+    """rtb_denoise: `levels` à-trous levels (0 = the resolve through the denoise path, no filtering) and the three edge-stops."""
+    o = Denoise()
+    o.levels = levels
+    o.sigma_color, o.sigma_normal, o.sigma_depth = sigma_color, sigma_normal, sigma_depth
+    return o
+
+
+def _denoise_opts(denoise) -> Denoise | None:
+    """None (no denoising) | True (the defaults) | dict of make_denoise keywords | a Denoise"""
+    if denoise is None or denoise is False:
+        return None
+    if denoise is True:
+        return make_denoise()
+    if isinstance(denoise, dict):
+        return make_denoise(**denoise)
+    return denoise
 
 
 class Scene:
@@ -208,32 +227,54 @@ class Scene:
     def render(self, width: int, height: int, spp: int, *, use_mis: bool = False, seed: int = 0, rank: int = 0,
                world: int = 1, pool_paths: int = 0, out: np.ndarray | None = None, count_work: bool = False,
                tune_refill: int = 0, tune_steps: int = 0, bin_bits: int | None = None, bin_octant_major: bool = False,
-               estimator: int | None = None, accel: int = 0) -> np.ndarray:
-        """Returns the frame as uint8 [height, width, 3], row 0 = top (the bytes of src/server.rs:187-189)."""
+               estimator: int | None = None, accel: int = 0, denoise=None) -> np.ndarray:
+        """Returns the frame as uint8 [height, width, 3], row 0 = top (the bytes of src/server.rs:187-189).
+        denoise: None = rtb_render; True / dict of make_denoise keywords / Denoise = rtb_render_denoised (whole frames)."""
         p = make_params(width, height, spp, use_mis=use_mis, seed=seed, rank=rank, world=world, pool_paths=pool_paths,
                         count_work=count_work, tune_refill=tune_refill, tune_steps=tune_steps, bin_bits=bin_bits,
                         bin_octant_major=bin_octant_major, estimator=estimator, accel=accel)
         if out is None:
             out = np.zeros((height, width, 3), dtype=np.uint8)
         assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"] and out.size == width * height * 3
-        _check(_abi.lib().rtb_render(self._h, C.byref(p), out.ctypes.data_as(C.POINTER(C.c_uint8)), None))
+        dn = _denoise_opts(denoise)
+        if dn is not None:
+            _check(_abi.lib().rtb_render_denoised(self._h, C.byref(p), None, C.byref(dn), out.ctypes.data_as(C.POINTER(C.c_uint8)),
+                                                  None, None, None))
+        else:
+            _check(_abi.lib().rtb_render(self._h, C.byref(p), out.ctypes.data_as(C.POINTER(C.c_uint8)), None))
         return out
 
     def render_adaptive(self, width: int, height: int, spp: int, *, target_levels: float, pass_spp: int = 16,
-                        min_spp: int | None = None, use_mis: bool = False, seed: int = 0, accel: int = 0):
+                        min_spp: int | None = None, use_mis: bool = False, seed: int = 0, accel: int = 0, denoise=None):
         """Adaptive sampling (rtb_render_adaptive): spp is the budget; each 32x32 tile stops once every pixel's estimated
         standard error is <= target_levels 8-bit output levels.  Returns (frame uint8 [h, w, 3], tile_spp int32 [ty, tx],
-        tile_error float32 [ty, tx])."""
+        tile_error float32 [ty, tx]).  denoise as for render (rtb_render_denoised)."""
         p = make_params(width, height, spp, use_mis=use_mis, seed=seed, accel=accel)
         o = make_adaptive(spp, target_levels=target_levels, pass_spp=pass_spp, min_spp=min_spp)
         ty, tx = (height + 31) // 32, (width + 31) // 32
         out = np.zeros((height, width, 3), dtype=np.uint8)
         tile_spp = np.zeros((ty, tx), dtype=np.int32)
         tile_error = np.zeros((ty, tx), dtype=np.float32)
-        _check(_abi.lib().rtb_render_adaptive(self._h, C.byref(p), C.byref(o), out.ctypes.data_as(C.POINTER(C.c_uint8)),
-                                              tile_spp.ctypes.data_as(C.POINTER(C.c_int32)),
-                                              tile_error.ctypes.data_as(C.POINTER(C.c_float)), None))
+        args = (out.ctypes.data_as(C.POINTER(C.c_uint8)), tile_spp.ctypes.data_as(C.POINTER(C.c_int32)),
+                tile_error.ctypes.data_as(C.POINTER(C.c_float)), None)
+        dn = _denoise_opts(denoise)
+        if dn is not None:
+            _check(_abi.lib().rtb_render_denoised(self._h, C.byref(p), C.byref(o), C.byref(dn), *args))
+        else:
+            _check(_abi.lib().rtb_render_adaptive(self._h, C.byref(p), C.byref(o), *args))
         return out, tile_spp, tile_error
+
+    def gbuffer(self, width: int, height: int, accel: int = 0) -> dict:
+        """The denoiser's guides (rtb_scene_gbuffer): albedo float32 [h, w, 3], normal float32 [h, w, 3], depth float32
+        [h, w], obj int32 [h, w] (-1 = miss); row 0 = top."""
+        albedo = np.empty((height, width, 3), dtype=np.float32)
+        normal = np.empty((height, width, 3), dtype=np.float32)
+        depth = np.empty((height, width), dtype=np.float32)
+        obj = np.empty((height, width), dtype=np.int32)
+        fp = C.POINTER(C.c_float)
+        _check(_abi.lib().rtb_scene_gbuffer(self._h, width, height, accel, albedo.ctypes.data_as(fp), normal.ctypes.data_as(fp),
+                                            depth.ctypes.data_as(fp), obj.ctypes.data_as(C.POINTER(C.c_int32))))
+        return {"albedo": albedo, "normal": normal, "depth": depth, "obj": obj}
 
     def render_device(self, params: Params, d_rgb8_tiles: int, d_subpixel_sums: int = 0) -> int:
         """Device-resident render: raw device pointers (e.g. torch tensor .data_ptr())."""
@@ -312,16 +353,24 @@ class RenderJob:
     PIXELS_PER_MSG = 60
 
     def __init__(self, scene: Scene, width: int, height: int, samples_per_pixel: int, *, passes: int = 1, seed: int = 0,
-                 use_mis: bool = False, pool_paths: int = 0, accel: int = 0, adaptive: dict | None = None):
+                 use_mis: bool = False, pool_paths: int = 0, accel: int = 0, adaptive: dict | None = None, denoise=None):
         """adaptive: dict(target_levels=..., pass_spp=16, min_spp=None) makes this an adaptive job (rtb_job_begin_adaptive):
         samples_per_pixel is the budget, `passes` is ignored and the job re-sends the frame once per pass until every tile
-        has converged."""
+        has converged.  denoise (True / dict of make_denoise keywords / Denoise): every frame the job sends is denoised
+        (rtb_job_begin_denoised); a single-pass job then renders the frame as one band."""
         self.scene = scene
         self.params = make_params(width, height, samples_per_pixel, use_mis=use_mis, seed=seed, pool_paths=pool_paths, accel=accel)
         self._h = C.c_void_p()
         # guards the handle: stop() may come from another thread (the server's event loop) while close() frees the job
         self._lock = threading.Lock()
-        if adaptive is not None:
+        dn = _denoise_opts(denoise)
+        if dn is not None:
+            self.adaptive = make_adaptive(samples_per_pixel, **adaptive) if adaptive is not None else None
+            self.denoise = dn
+            _check(_abi.lib().rtb_job_begin_denoised(scene._h, C.byref(self.params), passes,
+                                                     C.byref(self.adaptive) if self.adaptive is not None else None, C.byref(dn),
+                                                     C.byref(self._h)))
+        elif adaptive is not None:
             self.adaptive = make_adaptive(samples_per_pixel, **adaptive)
             _check(_abi.lib().rtb_job_begin_adaptive(scene._h, C.byref(self.params), C.byref(self.adaptive), C.byref(self._h)))
         else:
@@ -400,6 +449,24 @@ class RenderJob:
             self.close()
         except Exception:
             pass
+
+
+def denoise_image(color, variance, albedo, normal, depth, obj, *, levels: int = 5, sigma_color: float = 4.0,
+                  sigma_normal: float = 128.0, sigma_depth: float = 1.0, device: int = 0) -> np.ndarray:
+    """The filter alone (rtb_denoise_image) on host arrays: color / albedo / normal [h, w, 3], variance / depth [h, w] float,
+    obj [h, w] int.  Returns the denoised linear colour float32 [h, w, 3] (before clamp and gamma)."""
+    color = np.ascontiguousarray(color, dtype=np.float32)
+    h, w = color.shape[:2]
+    arrs = [np.ascontiguousarray(a, dtype=np.float32) for a in (variance, albedo, normal, depth)]
+    obj = np.ascontiguousarray(obj, dtype=np.int32)
+    assert color.shape == (h, w, 3) and arrs[1].shape == arrs[2].shape == (h, w, 3)
+    assert arrs[0].shape == arrs[3].shape == obj.shape == (h, w)
+    out = np.empty((h, w, 3), dtype=np.float32)
+    o = make_denoise(levels, sigma_color=sigma_color, sigma_normal=sigma_normal, sigma_depth=sigma_depth)
+    fp = C.POINTER(C.c_float)
+    _check(_abi.lib().rtb_denoise_image(device, w, h, C.byref(o), color.ctypes.data_as(fp), *[a.ctypes.data_as(fp) for a in arrs],
+                                        obj.ctypes.data_as(C.POINTER(C.c_int32)), out.ctypes.data_as(fp)))
+    return out
 
 
 def fp32_peak_tflops(device: int = 0) -> float:
