@@ -98,12 +98,13 @@ typedef struct rtb_scene_info {
 
 /* one object as the loader built it (f64, after transforms) — Object / Geometry, src/scene.rs:10-15 */
 typedef struct rtb_object_info {
-    int32_t brdf;          /* 0 diffuse, 1 specular, 2 phong */
+    int32_t brdf;          /* 0 diffuse, 1 specular, 2 phong, 3 dielectric */
     int32_t geometry;      /* 0 sphere, 1 plane, 2 mesh (cube / prism / OBJ) */
     int32_t n_triangles;
     int32_t first_triangle; /* global triangle index of the mesh's first triangle, or -1 */
     double emitted[3];
-    double k[3];           /* kd | ks | phong {kd, ks, power} */
+    double k[3];           /* kd | ks | phong {kd, ks, power} | dielectric {ior, orientation sign, 0}: the sign is +1 when the
+                              stored normals point out of the medium (sphere: radial, plane: n, mesh: see rtb_object_desc) */
     double color_d[3];
     double color_s[3];
     double pos[3];
@@ -154,7 +155,13 @@ void rtb_scene_destroy(rtb_scene* scene);
  * Mesh::triangle, src/geometry.rs:872-877).  Same light rule and error codes as the TOML path. */
 typedef struct rtb_object_desc {
     double emitted[3];
-    int32_t brdf;           /* 0 diffuse {k = kd}, 1 specular {k = ks}, 2 phong {k = kd, ks, power; color_d; color_s} */
+    int32_t brdf;           /* 0 diffuse {k = kd}, 1 specular {k = ks}, 2 phong {k = kd, ks, power; color_d; color_s},
+                               3 dielectric {k = ior, 0, 0 (ior finite, > 0); color_d = transmission tint, each in [0, 1]}:
+                               smooth glass, air outside.  Outside is the side of a sphere's outward normal, the side a
+                               plane's n points to, and for a mesh the outside of the solid it bounds: the loader winds
+                               each connected piece consistently and orients it by its signed volume (f64), and keeps
+                               the stored normal norm((c-a) x (b-a)) of the first triangle, turning triangles wound
+                               against it around (b <-> c).  Meant for closed meshes; an open one gets an arbitrary side. */
     int32_t geometry;       /* 0 sphere, 1 plane, 2 mesh */
     double k[3];
     double color_d[3];

@@ -17,6 +17,8 @@ constexpr int DENOISE_THREADS = 256;
 // GBUFFER_MAX_BOUNCES specular vertices in the direction k_shade takes there (the stale-`o` quirk included: every vertex
 // of a chain reflects the camera ray's -d).  Per ray: the first non-specular hit's object, facing normal, path length and
 // albedo (times ks of every mirror on the way); an emitter, a miss or an unfinished chain has albedo 1.  Per pixel:
+// A dielectric counts as a specular vertex: the ray follows the refracted direction (the reflected one under total internal
+// reflection) and the albedo takes the tint on transmission.
 // ga = (mean albedo, mean depth over the rays that hit), gn = (renormalised sum of the normals, the object most rays hit,
 // ties to the lowest sub-pixel; -1 = miss).
 __global__ void __launch_bounds__(WF_THREADS) k_gbuffer(DevScene S, const Camera cam, int width, int height, int accel,
@@ -56,8 +58,24 @@ __global__ void __launch_bounds__(WF_THREADS) k_gbuffer(DevScene S, const Camera
                     origin = hg.pcode;
                     continue;
                 }
+                if (m.brdf == 3 && b < GBUFFER_MAX_BOUNCES) {   // dielectric: refract, or reflect under total internal reflection
+                    const bool flipped = (hg.pcode & PC_FLIPPED) != 0u;
+                    float cos_t;
+                    const float F = dielectric_fresnel(-dot(d, hg.n), dielectric_entering(flipped, m.k.y) ? 1.0f / m.k.x : m.k.x, cos_t);
+                    bool refracted;
+                    d = dielectric_scatter(d, hg.n, flipped, m.k.y, m.k.x, F < 1.0f ? 1.0f : 0.0f, refracted);
+                    ovec = -d;   // the stale-`o` quirk restarts from the true direction, as in k_shade
+                    o = hg.pos;
+                    origin = hg.pcode;
+                    if (refracted) {   // k_shade's rule: leave through the other side
+                        origin ^= PC_FLIPPED;
+                        if (m.geom != 0) o = hg.pos - (2.0f * SURF_OFFSET) * hg.n;
+                        thr = thr * f3(m.color_d);
+                    }
+                    continue;
+                }
                 const bool emits = m.emitted.x != 0.f || m.emitted.y != 0.f || m.emitted.z != 0.f;
-                if (m.brdf != 1 && !emits)
+                if (m.brdf != 1 && m.brdf != 3 && !emits)
                     a = thr * (m.brdf == 0 ? f3(m.k) : f3(m.color_d) * m.k.x + f3(m.color_s) * m.k.y);
                 nrm = nrm + hg.n;
                 depth += path;

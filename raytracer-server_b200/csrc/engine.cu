@@ -514,12 +514,14 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
         CU_TRY(cudaFuncSetAttribute(k_shade<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_shade<1, 0, 0, true, SHADE_THREADS_NEE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_shade<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        CU_TRY(cudaFuncSetAttribute(k_shade<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_generate<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         const int smem_tail = (int)shared_scene_bytes(MAX_OBJECTS, MAX_OBJECTS, SHADE_THREADS);
         const int smem_tail_nee = (int)shared_scene_bytes(MAX_OBJECTS, MAX_OBJECTS, SHADE_THREADS_NEE);
         CU_TRY(cudaFuncSetAttribute(k_shade<0, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         CU_TRY(cudaFuncSetAttribute(k_shade<1, 0, 0, true, SHADE_THREADS_NEE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail_nee));
         CU_TRY(cudaFuncSetAttribute(k_shade<2, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
+        CU_TRY(cudaFuncSetAttribute(k_shade<3, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         int b = 0;
         CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<false>, WF_THREADS, smem_stack));
         c->grid_ext = std::max(1, b) * prop.multiProcessorCount;
@@ -539,7 +541,7 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
             return RTB_OK;
         };
         if (int e = shade_grid({(const void*)k_shade<0>, (const void*)k_shade<2>, (const void*)k_shade<2, 8, 0>, (const void*)k_shade<2, 5, 1>,
-                                (const void*)k_shade<2, 5, 2>, (const void*)k_shade<2, 5, 3>}, SHADE_THREADS, c->grid_shade)) return e;
+                                (const void*)k_shade<2, 5, 2>, (const void*)k_shade<2, 5, 3>, (const void*)k_shade<3>}, SHADE_THREADS, c->grid_shade)) return e;
         if (int e = shade_grid({(const void*)k_shade<1, 0, 0, true, SHADE_THREADS_NEE>, (const void*)k_shade<1, 8, 0, true, SHADE_THREADS_NEE>,
                                 (const void*)k_shade<1, 5, 1, true, SHADE_THREADS_NEE>, (const void*)k_shade<1, 5, 2, true, SHADE_THREADS_NEE>,
                                 (const void*)k_shade<1, 5, 3, true, SHADE_THREADS_NEE>}, SHADE_THREADS_NEE, c->grid_shade_nee)) return e;
@@ -768,7 +770,7 @@ static void launch_generate(int n_planes, int n_spheres, int grid, size_t smem, 
 // k_shade instantiations: general | reference-scene fast paths | fast paths with the analytic table in the kernel
 // parameters, unrolled for 5 planes + 1..3 spheres (cubes, flying_unicorn, cornell_box)
 static bool shade_is_nomesh(int mode, const RenderArgs& a) {
-    return a.S.n_tris == 0 && mode != 0 && a.S.n_planes == 5 && a.S.n_prims - a.S.n_planes == 3 && !getenv("RTB_NO_SMALL_TABLE") &&
+    return a.S.n_tris == 0 && (mode == 1 || mode == 2) && a.S.n_planes == 5 && a.S.n_prims - a.S.n_planes == 3 && !getenv("RTB_NO_SMALL_TABLE") &&
            !getenv("RTB_GENERIC_TABLE");
 }
 // paths left below which a run switches to the inline-tail k_shade (0 = never); RTB_INLINE_TAIL overrides
@@ -784,6 +786,7 @@ static void launch_shade(int mode, int n_planes, int n_spheres, int grid, size_t
         const size_t smem_t = shared_scene_bytes(a.S.n_prims, a.S.n_objects, shade_cta(mode));
         if (mode == 1) k_shade<1, 0, 0, true, shade_cta(1), true><<<grid, shade_cta(1), smem_t, st>>>(a, cur);
         else if (mode == 2) k_shade<2, 0, 0, true, shade_cta(2), true><<<grid, shade_cta(2), smem_t, st>>>(a, cur);
+        else if (mode == 3) k_shade<3, 0, 0, true, shade_cta(3), true><<<grid, shade_cta(3), smem_t, st>>>(a, cur);
         else k_shade<0, 0, 0, true, shade_cta(0), true><<<grid, shade_cta(0), smem_t, st>>>(a, cur);
         return;
     }
@@ -800,6 +803,7 @@ static void launch_shade(int mode, int n_planes, int n_spheres, int grid, size_t
     else if (mode == 2 && n_planes + n_spheres <= 8 && !getenv("RTB_NO_SMALL_TABLE")) RTB_SHADE(2, 8, 0);
     else if (mode == 1) RTB_SHADE(1, 0, 0);
     else if (mode == 2) RTB_SHADE(2, 0, 0);
+    else if (mode == 3) RTB_SHADE(3, 0, 0);
     else RTB_SHADE(0, 0, 0);
 #undef RTB_SHADE
 }
@@ -835,9 +839,12 @@ int run_wavefront(rtb_scene* sc, RenderContext* c, RenderArgs& a, uint32_t ks_be
     // compile-time specialisation of k_shade for the common case (see its definition)
     if (a.estimator == RTB_EST_MIS_BALANCE && sc->fs.light_geom != GEOM_SPHERE)
         return fail(RTB_EUNSUPPORTED, "RTB_EST_MIS_BALANCE needs a sphere light (the reference's mesh-light sampler does not return points of the mesh, src/geometry.rs:622-628)");
+    // a scene with a dielectric always runs the general kernel with the dielectric branch (MODE 3), probes included
+    bool dielectric = false;
+    for (const FlatMaterial& m : sc->fs.materials) dielectric = dielectric || m.brdf == BRDF_DIELECTRIC;
     bool fast_shade = !a.probe_px && a.estimator != RTB_EST_MIS_BALANCE && sc->fs.light_geom == GEOM_SPHERE && !getenv("RTB_NO_FAST_SHADE");
     for (const FlatMaterial& m : sc->fs.materials) fast_shade = fast_shade && m.brdf != BRDF_PHONG;
-    const int shade_mode = !fast_shade ? 0 : (a.estimator == 0 ? 1 : 2);
+    const int shade_mode = dielectric ? 3 : (!fast_shade ? 0 : (a.estimator == 0 ? 1 : 2));
     // the CTA shape of k_shade depends on the instantiation: so do its grid and warp count (static first chunks, k_prepare)
     const bool nomesh = shade_is_nomesh(shade_mode, a);
     const int grid_shade = nomesh ? c->grid_shade_nomesh : (shade_mode == 1 ? c->grid_shade_nee : c->grid_shade);
@@ -1316,13 +1323,20 @@ int rtb_scene_create(const rtb_scene_desc* desc, int device, rtb_scene** out) {
         const rtb_object_desc& d = desc->objects[i];
         HostObject o;
         o.emitted = {d.emitted[0], d.emitted[1], d.emitted[2]};
-        if (d.brdf < 0 || d.brdf > 2 || d.geometry < 0 || d.geometry > 2) { rc = RTB_EPARSE; err = "object " + std::to_string(i) + ": unknown brdf / geometry kind"; break; }
+        if (d.brdf < 0 || d.brdf > 3 || d.geometry < 0 || d.geometry > 2) { rc = RTB_EPARSE; err = "object " + std::to_string(i) + ": unknown brdf / geometry kind"; break; }
         o.brdf = d.brdf;
         if (d.brdf == BRDF_PHONG) {
             if (d.k[2] < 0) { rc = RTB_EPARSE; err = "phong power must be >= 0"; break; }
             o.phong_kd = d.k[0]; o.phong_ks = d.k[1]; o.phong_power = (int)d.k[2];
             o.color_d = {d.color_d[0], d.color_d[1], d.color_d[2]};
             o.color_s = {d.color_s[0], d.color_s[1], d.color_s[2]};
+        } else if (d.brdf == BRDF_DIELECTRIC) {
+            if (!std::isfinite(d.k[0]) || !(d.k[0] > 0)) { rc = RTB_EPARSE; err = "object " + std::to_string(i) + ": dielectric ior (k[0]) must be a finite number > 0"; break; }
+            bool tint_ok = true;
+            for (int c = 0; c < 3; ++c) tint_ok = tint_ok && d.color_d[c] >= 0 && d.color_d[c] <= 1;
+            if (!tint_ok) { rc = RTB_EPARSE; err = "object " + std::to_string(i) + ": dielectric tint (color_d) components must lie in [0, 1]"; break; }
+            o.k = {d.k[0], 0, 0};
+            o.color_d = {d.color_d[0], d.color_d[1], d.color_d[2]};
         } else {
             o.k = {d.k[0], d.k[1], d.k[2]};
         }
@@ -1514,6 +1528,9 @@ int rtb_scene_object(const rtb_scene* scene, int32_t index, rtb_object_info* out
         out->k[0] = o.phong_kd; out->k[1] = o.phong_ks; out->k[2] = o.phong_power;
         out->color_d[0] = o.color_d.x; out->color_d[1] = o.color_d.y; out->color_d[2] = o.color_d.z;
         out->color_s[0] = o.color_s.x; out->color_s[1] = o.color_s.y; out->color_s[2] = o.color_s.z;
+    } else if (o.brdf == BRDF_DIELECTRIC) {
+        out->k[0] = o.k.x; out->k[1] = scene->fs.materials[index].k[1];   // ior, orientation sign
+        out->color_d[0] = o.color_d.x; out->color_d[1] = o.color_d.y; out->color_d[2] = o.color_d.z;
     } else {
         out->k[0] = o.k.x; out->k[1] = o.k.y; out->k[2] = o.k.z;
     }

@@ -1,10 +1,12 @@
 // scene_host.cpp — see scene_host.hpp.  Reference citations are relative to /root/reference.
 #include "scene_host.hpp"
 
+#include <array>
 #include <cmath>
 #include <cstring>
 #include <fstream>
 #include <limits>
+#include <map>
 #include <sstream>
 
 #include "../../include/rtb200.h"
@@ -195,8 +197,19 @@ void build_object(const Value& spec, const std::string& assets_dir, HostObject& 
         const Value& pw = need(b, "power", "brdf");
         if (pw.kind != Value::Integer || pw.integer < 0) bad("phong power must be a non-negative integer (usize)");
         o.phong_power = (int)pw.integer;
+    } else if (bt == "dielectric") {
+        o.brdf = BRDF_DIELECTRIC;
+        const double ior = num(need(b, "ior", "brdf"), "ior");
+        if (!std::isfinite(ior) || !(ior > 0)) bad("dielectric ior must be a finite number > 0");
+        o.k = {ior, 0, 0};
+        o.color_d = {1, 1, 1};
+        if (const Value* t = b.find("tint")) {
+            o.color_d = vec3(*t, "tint");
+            for (double c : {o.color_d.x, o.color_d.y, o.color_d.z})
+                if (!(c >= 0 && c <= 1)) bad("dielectric tint components must lie in [0, 1]");
+        }
     } else {
-        bad("unknown variant `" + bt + "`, expected one of `diffuse`, `specular`, `phong`");
+        bad("unknown variant `" + bt + "`, expected one of `diffuse`, `specular`, `phong`, `dielectric`");
     }
     const Value& g = need(spec, "geometry", "object");
     if (g.kind != Value::Table) bad("geometry must be a table");
@@ -318,14 +331,27 @@ int flatten_scene(const HostScene& hs, FlatScene& fs, std::string& err) {
             m.k[0] = (float)o.phong_kd; m.k[1] = (float)o.phong_ks; m.k[2] = (float)o.phong_power;
             m.color_d[0] = (float)o.color_d.x; m.color_d[1] = (float)o.color_d.y; m.color_d[2] = (float)o.color_d.z;
             m.color_s[0] = (float)o.color_s.x; m.color_s[1] = (float)o.color_s.y; m.color_s[2] = (float)o.color_s.z;
+        } else if (o.brdf == BRDF_DIELECTRIC) {
+            m.k[0] = (float)o.k.x;
+            m.k[1] = 1.0f;   // spheres and planes; meshes below
+            m.color_d[0] = (float)o.color_d.x; m.color_d[1] = (float)o.color_d.y; m.color_d[2] = (float)o.color_d.z;
         } else {
             m.k[0] = (float)o.k.x; m.k[1] = (float)o.k.y; m.k[2] = (float)o.k.z;
         }
         if (o.geom == GEOM_MESH) {
             m.first_tri = (int)(fs.tri_verts.size() / 9);
             m.n_tri = (int)(o.indices.size() / 3);
+            // a dielectric mesh gets ONE orientation sign: the side of its first triangle.  Triangles wound the other way
+            // (the built-in cube / prism alternate within each face) are stored with b and c swapped.
+            std::vector<int> out;
+            if (o.brdf == BRDF_DIELECTRIC) {
+                out = triangle_outward(o);
+                m.k[1] = (float)out[0];
+            }
             for (size_t k = 0; k < o.indices.size(); ++k) {
-                const D3& p = o.vertices[o.indices[k]];
+                const size_t t = k / 3, c = k % 3;
+                const bool swap = !out.empty() && out[t] != out[0] && c != 0;
+                const D3& p = o.vertices[o.indices[swap ? 3 * t + 3 - c : k]];
                 fs.tri_verts.push_back((float)p.x);
                 fs.tri_verts.push_back((float)p.y);
                 fs.tri_verts.push_back((float)p.z);
@@ -394,6 +420,52 @@ int flatten_scene(const HostScene& hs, FlatScene& fs, std::string& err) {
     }
     (void)err;
     return RTB_OK;
+}
+
+std::vector<int> triangle_outward(const HostObject& o) {
+    const size_t n = o.indices.size() / 3;
+    // vertex ids by position (rtb_scene_create hands every triangle its own three vertices)
+    std::map<std::array<double, 3>, int> vid;
+    std::vector<int> v(3 * n);
+    for (size_t k = 0; k < 3 * n; ++k) {
+        const D3& p = o.vertices[o.indices[k]];
+        v[k] = vid.emplace(std::array<double, 3>{p.x, p.y, p.z}, (int)vid.size()).first->second;
+    }
+    // undirected edge -> (triangle, traversed low -> high id)
+    std::map<std::pair<int, int>, std::vector<std::pair<int, bool>>> edges;
+    for (size_t t = 0; t < n; ++t)
+        for (int e = 0; e < 3; ++e) {
+            const int a = v[3 * t + e], b = v[3 * t + (e + 1) % 3];
+            if (a != b) edges[{std::min(a, b), std::max(a, b)}].push_back({(int)t, a < b});
+        }
+    // rel[t] = +1 / -1: wound like / against the seed of its piece (consistent neighbours traverse a shared edge in opposite
+    // directions); pieces are flood-filled one after another
+    std::vector<int> rel(n, 0), out(n, 1), piece;
+    for (size_t seed = 0; seed < n; ++seed) {
+        if (rel[seed]) continue;
+        rel[seed] = 1;
+        piece.assign(1, (int)seed);
+        double vol = 0;
+        for (size_t q = 0; q < piece.size(); ++q) {
+            const int t = piece[q];
+            const D3 &a = o.vertices[o.indices[3 * t]], &b = o.vertices[o.indices[3 * t + 1]], &c = o.vertices[o.indices[3 * t + 2]];
+            vol += rel[t] * (a.x * (b.y * c.z - b.z * c.y) + a.y * (b.z * c.x - b.x * c.z) + a.z * (b.x * c.y - b.y * c.x));
+            for (int e = 0; e < 3; ++e) {
+                const int a0 = v[3 * t + e], b0 = v[3 * t + (e + 1) % 3];
+                if (a0 == b0) continue;
+                const bool up = a0 < b0;
+                for (const auto& nb : edges[{std::min(a0, b0), std::max(a0, b0)}]) {
+                    if (rel[nb.first]) continue;
+                    rel[nb.first] = nb.second == up ? -rel[t] : rel[t];
+                    piece.push_back(nb.first);
+                }
+            }
+        }
+        // vol > 0: the winding rel = +1 runs counter-clockwise seen from outside, so (b-a) x (c-a) points out and the stored
+        // normal (c-a) x (b-a) points in
+        for (int t : piece) out[t] = vol > 0 ? -rel[t] : rel[t];
+    }
+    return out;
 }
 
 }  // namespace rtb

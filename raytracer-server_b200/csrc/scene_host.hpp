@@ -17,15 +17,15 @@ struct D3 {
 };
 
 enum GeomKind : int { GEOM_SPHERE = 0, GEOM_PLANE = 1, GEOM_MESH = 2 };
-enum BrdfKind : int { BRDF_DIFFUSE = 0, BRDF_SPECULAR = 1, BRDF_PHONG = 2 };
+enum BrdfKind : int { BRDF_DIFFUSE = 0, BRDF_SPECULAR = 1, BRDF_PHONG = 2, BRDF_DIELECTRIC = 3 };
 
 struct HostObject {
     D3 emitted;
     int brdf = BRDF_DIFFUSE;
-    D3 k;                      // kd (diffuse) / ks (specular)
+    D3 k;                      // kd (diffuse) / ks (specular) / {ior, 0, 0} (dielectric)
     double phong_kd = 0, phong_ks = 0;
     int phong_power = 0;
-    D3 color_d, color_s;
+    D3 color_d, color_s;       // phong colours; dielectric: color_d = transmission tint
     int geom = GEOM_SPHERE;
     D3 pos;                    // sphere centre / plane point
     double r = 0;
@@ -64,8 +64,8 @@ struct FlatPrim {      // analytic primitive, in object order
 
 struct FlatMaterial {  // one per object
     float emitted[4];  // rgb, -
-    float k[4];        // diffuse kd / specular ks rgb; phong: kd, ks, power, -
-    float color_d[4];
+    float k[4];        // diffuse kd / specular ks rgb; phong: kd, ks, power, -; dielectric: ior, orientation sign, -
+    float color_d[4];  // phong colour_d; dielectric: tint
     float color_s[4];
     int32_t brdf;
     int32_t geom;
@@ -89,6 +89,11 @@ struct FlatScene {
 };
 
 int flatten_scene(const HostScene& hs, FlatScene& out, std::string& err);
+
+// Dielectric meshes: +1 / -1 per triangle = whether its stored normal norm((c-a) x (b-a)) points out of the solid.  The
+// winding is made consistent across shared edges (vertices matched by position) within each connected piece, and each
+// piece is oriented by the sign of its signed volume (f64).  An open piece gets an arbitrary side.
+std::vector<int> triangle_outward(const HostObject& o);
 
 // shared tail of every way to build a HostScene: Scene::new's light rule (src/scene.rs:126-141) + mesh tables
 int finish_host_scene(HostScene& hs, std::string& err);

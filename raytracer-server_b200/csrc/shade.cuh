@@ -13,6 +13,8 @@
 //           block 2 : {brdf u1, u2, lobe} = u24(x>>8, y>>8, z>>8)   dead-MIS "fresh" sample used only for its pdf (:195)
 //           block 3 : {light u1, u2, -, select}                      dead-MIS second light point (:206)
 //           block 4 : {brdf u1, u2, lobe}                            dead-MIS own BRDF sample (:203)
+//   dielectric vertex (DESIGN §3e): block 0 only — russian roulette as for a mirror, reflect iff brdf u1 < Fresnel F;
+//                     no light sample, no block 1
 #pragma once
 
 #include "device_types.cuh"

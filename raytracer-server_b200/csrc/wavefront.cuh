@@ -20,6 +20,7 @@
 #pragma once
 
 #include "adaptive_rule.cuh"
+#include "dielectric_rule.cuh"
 #include "intersect.cuh"
 #include "octree.cuh"
 #include "shade.cuh"
@@ -865,7 +866,9 @@ __device__ __forceinline__ uint32_t seg_slot(uint32_t base, uint32_t k) { return
 // NP = 8, NS = 0: any scene with <= 8 analytic primitives (generic 8-slot form, run-time counts).
 // MODE 1 / 2 (FAST) = the reference scenes' case, resolved at compile time: Diffuse / Specular materials only, sphere
 // light, no probe items; 1 = live NEE estimator, 2 = the dead "MIS" branch.  MODE 0, the general instantiation, keeps
-// every branch at run time (both estimators, Phong, mesh lights, rtb_sample_radiance probes).
+// every branch at run time (both estimators, Phong, mesh lights, rtb_sample_radiance probes).  MODE 3 is MODE 0 plus the
+// dielectric branch (brdf 3, DESIGN §3e): the host runs it for every scene with a dielectric, so that the other
+// instantiations compile exactly as they did before glass existed.
 constexpr int SHADE_THREADS_NOMESH = 160;   // the mesh-less instantiation needs 96 registers: 4 CTAs of 160 threads = 20 warps per SM
 // The live-NEE instantiations with a mesh (MODE 1, the bench frame's) fit 96 registers without spills too and run the same
 // shape.  The general and dead-MIS ones need 128 (at 96 they spill 140 bytes) and keep 2 CTAs of SHADE_THREADS.  (3 CTAs of
@@ -878,7 +881,8 @@ constexpr int shade_cta(int mode, bool mesh = true) { return !mesh ? SHADE_THREA
 // hardly fill an SM) collapse into one.  SIMD utilisation of the inline traversal is poor, but the tail holds < 0.1 % of the work.
 template <int MODE, int NP = 0, int NS = 0, bool MESH = true, int THREADS = SHADE_THREADS, bool INLINE = false>
 __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_MINB : 640 / THREADS) k_shade(const __grid_constant__ RenderArgs a, int c) {
-    constexpr bool FAST = MODE != 0;
+    constexpr bool FAST = MODE == 1 || MODE == 2;
+    constexpr bool DIEL = MODE == 3;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     DevCtrl* C = a.ctrl;
     const DevSceneHeader* hdr = a.S.hdr;
@@ -1039,7 +1043,11 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                     if (emits) accum_add(a.accum, acc, beta * emitted);
                     const DevMaterial& pm = sh.mats[object_of(a.S, sh, origin & PC_ID_MASK)];
                     const float inv_pp = (depth - 1u) <= 5u ? 1.0f : (1.0f / 0.9f);   // 1 / survival probability of the specular vertex
-                    beta = beta * f3(pm.k) * inv_pp;
+                    if constexpr (DIEL) {
+                        if (pm.brdf != 3) beta = beta * f3(pm.k) * inv_pp;   // a dielectric vertex has put its weight into beta already
+                    } else {
+                        beta = beta * f3(pm.k) * inv_pp;
+                    }
                 }
                 const float p = depth <= 5u ? 1.0f : 0.9f;  // MAX_BOUNCES / SURVIVAL_PROBABILITY (src/scene.rs:109-110,164-168)
                 const float inv_p = depth <= 5u ? 1.0f : (1.0f / 0.9f);
@@ -1051,14 +1059,31 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                     const VertexRng vr = rng_vertex(rng_pixel, sample, depth, a.keys);
                     // lobe / light-triangle selectors live in block 1 and are only drawn by Phong surfaces / mesh lights
                     float lobe_u = 0.f, select_u = 0.f;
-                    if (!FAST && (mat.brdf == 2 || light_is_mesh)) {
+                    if (!FAST && (mat.brdf == 2 || light_is_mesh) && !(DIEL && mat.brdf == 3)) {
                         const float4 r1 = rng_block(rng_pixel, sample, depth, 1u, a.keys);
                         lobe_u = r1.x;
                         select_u = r1.y;
                     }
                     const float4 r0 = make_float4(vr.light_u1, vr.light_u2, vr.rr, select_u);
                     const float4 rb = make_float4(vr.brdf_u1, vr.brdf_u2, lobe_u, 0.f);
-                    if (mat.brdf == 1) {  // specular branch, src/scene.rs:170-185
+                    if (DIEL && mat.brdf == 3) {
+                        // dielectric: reflect or refract with the Fresnel probability; the TRUE direction d, never the stale `o`.
+                        // No light sample: emission reached through glass is added at the next hit (PC_SPEC_PENDING).
+                        if (r0.z < p) {
+                            bool refracted;
+                            next_dir = dielectric_scatter(d, hg.n, (hg.pcode & PC_FLIPPED) != 0u, mat.k.y, mat.k.x, rb.x, refracted);
+                            nbeta = beta * inv_p;
+                            if (refracted) {
+                                // the ray leaves through the other side: with the flip bit toggled the self-intersection rule sees
+                                // its origin 1e-5 beyond the surface (spheres: on it, roots 0 and 2b), so the origin moves there
+                                pcode = hg.pcode ^ PC_FLIPPED;
+                                if (mat.geom != 0) pos = hg.pos - (2.0f * SURF_OFFSET) * hg.n;   // not a sphere
+                                nbeta = nbeta * f3(mat.color_d);   // no eta^2 factor: camera and light lie outside every medium
+                            }
+                            ext_push = true;
+                            eflags = pcode | PC_SPEC_PENDING;
+                        }
+                    } else if (mat.brdf == 1) {  // specular branch, src/scene.rs:170-185
                         if (r0.z < p) {
                             next_dir = flip_across(ovec, hg.n);
                             ext_push = true;

@@ -123,15 +123,18 @@ class Scene:
     @classmethod
     def from_objects(cls, camera_pos, camera_dir, objects: list, device: int = 0, name: str = "") -> "Scene":
         """Programmatic scene (rtb_scene_create).  Each object is a dict: emitted (opt), brdf = ("diffuse", kd) |
-        ("specular", ks) | ("phong", kd, ks, power, color_d, color_s), geometry = ("sphere", pos, r) |
-        ("plane", pos, n) | ("mesh", triangles[n, 3, 3])."""
+        ("specular", ks) | ("phong", kd, ks, power, color_d, color_s) | ("dielectric", ior, tint) (tint optional, default
+        (1, 1, 1)), geometry = ("sphere", pos, r) | ("plane", pos, n) | ("mesh", triangles[n, 3, 3])."""
         arr = (ObjectDesc * max(1, len(objects)))()
         keep = []
         for d, ob in zip(arr, objects):
             d.emitted[:] = list(map(float, ob.get("emitted", (0.0, 0.0, 0.0))))
             b = ob["brdf"]
-            d.brdf = {"diffuse": 0, "specular": 1, "phong": 2}[b[0]]
-            if b[0] == "phong":
+            d.brdf = {"diffuse": 0, "specular": 1, "phong": 2, "dielectric": 3}[b[0]]
+            if b[0] == "dielectric":
+                d.k[:] = [float(b[1]), 0.0, 0.0]
+                d.color_d[:] = list(map(float, b[2])) if len(b) > 2 else [1.0, 1.0, 1.0]
+            elif b[0] == "phong":
                 d.k[:] = [float(b[1]), float(b[2]), float(b[3])]
                 d.color_d[:] = list(map(float, b[4]))
                 d.color_s[:] = list(map(float, b[5]))
