@@ -50,6 +50,15 @@ typedef struct rtb_job rtb_job;
 #define RTB_EST_MIS_BALANCE 2 /* NOT in the reference: light sample + BRDF sample combined with the balance heuristic, i.e. the
                                  "TODO: Do multiple importance sampling properly" of src/scene.rs:187 done.  Same expectation as
                                  RTB_EST_NEE, less variance near the light; sphere lights only; never used for parity */
+#define RTB_EST_NEE_ALL_LIGHTS 3 /* NOT in the reference: next-event estimation over EVERY emitter, not just the first.  The light
+                                 table (rtb_scene_lights) holds each sphere or mesh with weight w = lum(max(emitted, 0)) * area > 0
+                                 (lum = Rec. 709 weights, area after the transforms: 4 pi r^2, or a mesh's true area), in object
+                                 order; a vertex picks entry i with p_i = w_i / sum w (block 1 z of the RNG contract), a triangle
+                                 of a mesh light by area (block 1 y) and a uniform point (block 0 light u1, u2), and adds
+                                 beta Le_i f max(n.w, 0) |n_y.w| / (r^2 p_i / area_i) if the point is visible.  Emission reached
+                                 from a diffuse or Phong vertex counts only for emitters outside the table (planes, zero weight);
+                                 at depth 1 and behind a mirror or glass it always counts.  With one sphere light this is
+                                 RTB_EST_NEE but for its unclamped cosines. */
 
 /* mesh acceleration (Mesh::intersect, src/geometry.rs:883-905) */
 #define RTB_ACCEL_LBVH 0             /* true nearest hit = the reference's brute-force branch (:887-903), through the device-built BVH (binned SAH, linear node table) */
@@ -200,6 +209,10 @@ int rtb_scene_upload(rtb_scene* scene, uint64_t* bytes);
 /* host-side view of the loader result, for cross-checks: triangles as 9 floats each (a,b,c) in
  * global triangle order; returns the count (call with cap = 0 to query) */
 int64_t rtb_scene_triangles(const rtb_scene* scene, float* out9, int64_t cap);
+/* the light table of RTB_EST_NEE_ALL_LIGHTS: per entry the object index, its selection probability and its area (f64);
+ * returns the entry count and fills at most cap entries of each non-NULL array (call with cap = 0 to query).  Works on
+ * host-only handles. */
+int64_t rtb_scene_lights(const rtb_scene* scene, int32_t* objects, double* prob, double* area, int64_t cap);
 
 /* Octree::build (src/geometry.rs:1149-1216) for one mesh object, on the host: counts4 = {nodes, parents, leaves, triangle
  * references}.  What RTB_ACCEL_OCTREE_REFERENCE traverses; needs no device. */

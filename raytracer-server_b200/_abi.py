@@ -25,6 +25,7 @@ RTB_ECANCELLED = 1
 EST_NEE = 0
 EST_MIS_DEAD = 1
 EST_MIS_BALANCE = 2
+EST_NEE_ALL_LIGHTS = 3
 ACCEL_LBVH = 0
 ACCEL_OCTREE_REFERENCE = 1
 
@@ -90,6 +91,7 @@ EXPORTS = [
     "rtb_untile_device_async", "rtb_job_stats", "rtb_sample_pixels", "rtb_trace_rays_accel", "rtb_scene_octree_stats", "rtb_scene_export", "rtb_scene_import",
     "rtb_render_adaptive", "rtb_job_begin_adaptive",
     "rtb_render_denoised", "rtb_job_begin_denoised", "rtb_scene_gbuffer", "rtb_denoise_image",
+    "rtb_scene_lights",
 ]
 
 _lib = None
@@ -115,6 +117,8 @@ def lib():
     L.rtb_scene_upload.argtypes = [vp, C.POINTER(C.c_uint64)]
     L.rtb_scene_triangles.argtypes = [vp, fp, C.c_int64]
     L.rtb_scene_triangles.restype = C.c_int64
+    L.rtb_scene_lights.argtypes = [vp, ip, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_int64]
+    L.rtb_scene_lights.restype = C.c_int64
     L.rtb_render.argtypes = [vp, C.POINTER(Params), C.POINTER(C.c_uint8), ip]
     L.rtb_local_pixels.argtypes = [C.POINTER(Params)]
     L.rtb_local_pixels.restype = C.c_int64

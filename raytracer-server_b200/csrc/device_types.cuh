@@ -57,6 +57,13 @@ struct DevSceneHeader {  // lives in global memory; one per scene
     int32_t root;          // encoded BVH root reference (inner >= 0, leaf < 0), valid if n_tris > 0
     float bvh_min[3];
     float bvh_max[3];
+    // the light table of RTB_EST_NEE_ALL_LIGHTS (light_rule.cuh, DESIGN §3f).  The offsets count 256-byte units from the header
+    // (every staged table starts on such a boundary), so they reach past 4 GB of scene while the header keeps 4-byte fields.
+    int32_t n_lights;
+    int32_t lights_select;   // 1: a vertex draws block 1 for the choice (more than one light, or a mesh light)
+    int32_t off_lights;      // DevLight[n_lights]
+    int32_t off_light_cdf;   // float[]: the lights' cdf (n_lights entries), then one triangle cdf per mesh light
+    int32_t off_light_of;    // int32_t[n_objects]: each object's table entry, -1 = not in the table
 };
 
 struct DevScene {          // passed to kernels by value

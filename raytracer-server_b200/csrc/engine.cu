@@ -212,10 +212,41 @@ int build_device_scene(rtb_scene* sc, const LbvhImport* import = nullptr) {
     sc->off_verts = align_up(sc->off_mats + fs.materials.size() * sizeof(DevMaterial), 256);
     sc->off_triobj = align_up(sc->off_verts + fs.tri_verts.size() * sizeof(float), 256);
     sc->off_cdf = align_up(sc->off_triobj + fs.tri_obj.size() * sizeof(int32_t), 256);
-    sc->stage_bytes = align_up(sc->off_cdf + fs.light_cdf.size() * sizeof(float), 256);
+    // the light table of RTB_EST_NEE_ALL_LIGHTS (light_rule.cuh) goes behind the other tables; only the header knows where
+    std::vector<DevLight> lights;
+    std::vector<float> light_cdf;
+    std::vector<int32_t> light_of((size_t)fs.n_objects, -1);
+    {
+        double cum = 0;
+        for (size_t k = 0; k < fs.lights.size(); ++k) {
+            cum += fs.lights[k].prob;
+            light_cdf.push_back(k + 1 == fs.lights.size() ? 1.0f : (float)cum);
+        }
+        for (size_t k = 0; k < fs.lights.size(); ++k) {
+            const FlatLight& l = fs.lights[k];
+            const HostObject& o = sc->hs.objects[(size_t)l.obj];
+            DevLight d{};
+            d.sphere = make_float4((float)o.pos.x, (float)o.pos.y, (float)o.pos.z, (float)o.r);
+            d.pdf_area = (float)(l.prob / l.area);
+            d.obj = l.obj;
+            d.tri_cdf = l.tri_cdf.empty() ? -1 : (int32_t)light_cdf.size();
+            for (double c : l.tri_cdf) light_cdf.push_back((float)c);
+            lights.push_back(d);
+            light_of[(size_t)l.obj] = (int32_t)k;
+        }
+    }
+    const size_t off_lights = align_up(sc->off_cdf + fs.light_cdf.size() * sizeof(float), 256);
+    const size_t off_light_cdf = align_up(off_lights + lights.size() * sizeof(DevLight), 256);
+    const size_t off_light_of = align_up(off_light_cdf + light_cdf.size() * sizeof(float), 256);
+    sc->stage_bytes = align_up(off_light_of + light_of.size() * sizeof(int32_t), 256);
     CU_TRY(cudaMallocHost((void**)&sc->h_stage, sc->stage_bytes));
     CU_TRY(cudaMalloc((void**)&sc->d_stage, sc->stage_bytes));
     std::memset(sc->h_stage, 0, sc->stage_bytes);
+    if (!lights.empty()) {
+        std::memcpy(sc->h_stage + off_lights, lights.data(), lights.size() * sizeof(DevLight));
+        std::memcpy(sc->h_stage + off_light_cdf, light_cdf.data(), light_cdf.size() * sizeof(float));
+    }
+    std::memcpy(sc->h_stage + off_light_of, light_of.data(), light_of.size() * sizeof(int32_t));
     if (!fs.prims.empty()) std::memcpy(sc->h_stage + sc->off_prims, fs.prims.data(), fs.prims.size() * sizeof(DevPrim));
     std::memcpy(sc->h_stage + sc->off_mats, fs.materials.data(), fs.materials.size() * sizeof(DevMaterial));
     if (n_tris) {
@@ -282,6 +313,11 @@ int build_device_scene(rtb_scene* sc, const LbvhImport* import = nullptr) {
     H.light_area = fs.light_area;
     H.n_tris = n_tris;
     H.root = sc->bvh.root;
+    H.n_lights = (int32_t)lights.size();
+    H.lights_select = lights.size() > 1 || (lights.size() == 1 && lights[0].tri_cdf >= 0);
+    H.off_lights = (int32_t)(off_lights / 256);
+    H.off_light_cdf = (int32_t)(off_light_cdf / 256);
+    H.off_light_of = (int32_t)(off_light_of / 256);
     std::memcpy(sc->h_stage, &H, sizeof(H));
     CU_TRY(cudaMemcpyAsync(sc->d_stage, sc->h_stage, sizeof(H), cudaMemcpyHostToDevice, sc->stream));
     CU_TRY(cudaStreamSynchronize(sc->stream));
@@ -515,6 +551,8 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
         CU_TRY(cudaFuncSetAttribute(k_shade<1, 0, 0, true, SHADE_THREADS_NEE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_shade<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_shade<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        CU_TRY(cudaFuncSetAttribute(k_shade<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        CU_TRY(cudaFuncSetAttribute(k_shade<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_generate<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         const int smem_tail = (int)shared_scene_bytes(MAX_OBJECTS, MAX_OBJECTS, SHADE_THREADS);
         const int smem_tail_nee = (int)shared_scene_bytes(MAX_OBJECTS, MAX_OBJECTS, SHADE_THREADS_NEE);
@@ -522,6 +560,8 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
         CU_TRY(cudaFuncSetAttribute(k_shade<1, 0, 0, true, SHADE_THREADS_NEE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail_nee));
         CU_TRY(cudaFuncSetAttribute(k_shade<2, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         CU_TRY(cudaFuncSetAttribute(k_shade<3, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
+        CU_TRY(cudaFuncSetAttribute(k_shade<4, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
+        CU_TRY(cudaFuncSetAttribute(k_shade<5, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         int b = 0;
         CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<false>, WF_THREADS, smem_stack));
         c->grid_ext = std::max(1, b) * prop.multiProcessorCount;
@@ -541,7 +581,8 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
             return RTB_OK;
         };
         if (int e = shade_grid({(const void*)k_shade<0>, (const void*)k_shade<2>, (const void*)k_shade<2, 8, 0>, (const void*)k_shade<2, 5, 1>,
-                                (const void*)k_shade<2, 5, 2>, (const void*)k_shade<2, 5, 3>, (const void*)k_shade<3>}, SHADE_THREADS, c->grid_shade)) return e;
+                                (const void*)k_shade<2, 5, 2>, (const void*)k_shade<2, 5, 3>, (const void*)k_shade<3>, (const void*)k_shade<4>,
+                                (const void*)k_shade<5>}, SHADE_THREADS, c->grid_shade)) return e;
         if (int e = shade_grid({(const void*)k_shade<1, 0, 0, true, SHADE_THREADS_NEE>, (const void*)k_shade<1, 8, 0, true, SHADE_THREADS_NEE>,
                                 (const void*)k_shade<1, 5, 1, true, SHADE_THREADS_NEE>, (const void*)k_shade<1, 5, 2, true, SHADE_THREADS_NEE>,
                                 (const void*)k_shade<1, 5, 3, true, SHADE_THREADS_NEE>}, SHADE_THREADS_NEE, c->grid_shade_nee)) return e;
@@ -628,11 +669,16 @@ int check_params(const rtb_params* p) {
     if (p->spp < 0) return fail(RTB_EINVAL, "spp must be >= 0");
     if ((long long)p->spp / 4 * 4 >= (1 << 20)) return fail(RTB_EINVAL, "spp too large (sample index field is 20 bits)");
     if (p->world < 1 || p->rank < 0 || p->rank >= p->world) return fail(RTB_EINVAL, "need 0 <= rank < world");
-    if (p->estimator != RTB_EST_NEE && p->estimator != RTB_EST_MIS_DEAD && p->estimator != RTB_EST_MIS_BALANCE)
+    if (p->estimator != RTB_EST_NEE && p->estimator != RTB_EST_MIS_DEAD && p->estimator != RTB_EST_MIS_BALANCE && p->estimator != RTB_EST_NEE_ALL_LIGHTS)
         return fail(RTB_EINVAL, "unknown estimator");
     if ((long long)p->width * p->height * 4 >= (1ll << 31)) return fail(RTB_EINVAL, "frame too large for 31-bit accumulator indices");
     if (p->accel != RTB_ACCEL_LBVH && p->accel != RTB_ACCEL_OCTREE_REFERENCE) return fail(RTB_EINVAL, "unknown accel mode");
     return RTB_OK;
+}
+
+// shadow-queue slots for P paths: the NEE estimators queue at most one shadow ray per vertex, the MIS ones two
+uint32_t shadow_slots(int estimator, uint32_t P) {
+    return estimator == RTB_EST_NEE || estimator == RTB_EST_NEE_ALL_LIGHTS ? P : 2 * P;
 }
 
 int local_tiles(const rtb_params* p) {
@@ -787,6 +833,8 @@ static void launch_shade(int mode, int n_planes, int n_spheres, int grid, size_t
         if (mode == 1) k_shade<1, 0, 0, true, shade_cta(1), true><<<grid, shade_cta(1), smem_t, st>>>(a, cur);
         else if (mode == 2) k_shade<2, 0, 0, true, shade_cta(2), true><<<grid, shade_cta(2), smem_t, st>>>(a, cur);
         else if (mode == 3) k_shade<3, 0, 0, true, shade_cta(3), true><<<grid, shade_cta(3), smem_t, st>>>(a, cur);
+        else if (mode == 4) k_shade<4, 0, 0, true, shade_cta(4), true><<<grid, shade_cta(4), smem_t, st>>>(a, cur);
+        else if (mode == 5) k_shade<5, 0, 0, true, shade_cta(5), true><<<grid, shade_cta(5), smem_t, st>>>(a, cur);
         else k_shade<0, 0, 0, true, shade_cta(0), true><<<grid, shade_cta(0), smem_t, st>>>(a, cur);
         return;
     }
@@ -804,6 +852,8 @@ static void launch_shade(int mode, int n_planes, int n_spheres, int grid, size_t
     else if (mode == 1) RTB_SHADE(1, 0, 0);
     else if (mode == 2) RTB_SHADE(2, 0, 0);
     else if (mode == 3) RTB_SHADE(3, 0, 0);
+    else if (mode == 4) RTB_SHADE(4, 0, 0);
+    else if (mode == 5) RTB_SHADE(5, 0, 0);
     else RTB_SHADE(0, 0, 0);
 #undef RTB_SHADE
 }
@@ -844,7 +894,10 @@ int run_wavefront(rtb_scene* sc, RenderContext* c, RenderArgs& a, uint32_t ks_be
     for (const FlatMaterial& m : sc->fs.materials) dielectric = dielectric || m.brdf == BRDF_DIELECTRIC;
     bool fast_shade = !a.probe_px && a.estimator != RTB_EST_MIS_BALANCE && sc->fs.light_geom == GEOM_SPHERE && !getenv("RTB_NO_FAST_SHADE");
     for (const FlatMaterial& m : sc->fs.materials) fast_shade = fast_shade && m.brdf != BRDF_PHONG;
-    const int shade_mode = dielectric ? 3 : (!fast_shade ? 0 : (a.estimator == 0 ? 1 : 2));
+    // RTB_EST_NEE_ALL_LIGHTS: the general kernel with next-event estimation over the whole light table (MODE 4), or MODE 3's
+    // dielectric kernel with it (MODE 5), probes included
+    const int shade_mode = a.estimator == RTB_EST_NEE_ALL_LIGHTS ? (dielectric ? 5 : 4)
+                                                                 : (dielectric ? 3 : (!fast_shade ? 0 : (a.estimator == 0 ? 1 : 2)));
     // the CTA shape of k_shade depends on the instantiation: so do its grid and warp count (static first chunks, k_prepare)
     const bool nomesh = shade_is_nomesh(shade_mode, a);
     const int grid_shade = nomesh ? c->grid_shade_nomesh : (shade_mode == 1 ? c->grid_shade_nee : c->grid_shade);
@@ -1008,7 +1061,7 @@ int run_wavefront(rtb_scene* sc, RenderContext* c, RenderArgs& a, uint32_t ks_be
 int render_into_context(rtb_scene* sc, const rtb_params* p, RenderContext* c, RenderArgs& a, volatile int* cancel, rtb_stats& st,
                         bool& cancelled) {
     uint32_t P = default_pool(p);
-    uint32_t SP = p->estimator == RTB_EST_NEE ? P : 2 * P;
+    uint32_t SP = shadow_slots(p->estimator, P);
     size_t accum_elems = (size_t)p->width * p->height * 4;
     int rc = ensure_context(sc, c, P, SP, accum_elems, requested_bin_bits(sc, p) > 0);
     if (rc != RTB_OK) return rc;
@@ -1236,7 +1289,7 @@ int render_whole_frame(rtb_scene* scene, const rtb_params* params, const rtb_ada
     if (rc != RTB_OK) return rc;
     if ((rc = need_accel(scene, params)) != RTB_OK) return rc;
     const uint32_t P = opts ? adaptive_pool(params, opts) : default_pool(params);
-    const uint32_t SP = params->estimator == RTB_EST_NEE ? P : 2 * P;
+    const uint32_t SP = shadow_slots(params->estimator, P);
     const size_t frame = (size_t)params->width * params->height * 3;
     const int n_tiles = local_tiles(params);
     RenderContext* c = acquire_context(scene, P);
@@ -1514,6 +1567,17 @@ int64_t rtb_scene_triangles(const rtb_scene* scene, float* out9, int64_t cap) {
     int64_t n = (int64_t)scene->fs.tri_obj.size();
     if (out9 && cap > 0) std::memcpy(out9, scene->fs.tri_verts.data(), (size_t)std::min(n, cap) * 9 * sizeof(float));
     return n;
+}
+
+int64_t rtb_scene_lights(const rtb_scene* scene, int32_t* objects, double* prob, double* area, int64_t cap) {
+    if (!scene) return fail(RTB_EINVAL, "NULL scene");
+    const std::vector<FlatLight>& L = scene->fs.lights;
+    for (int64_t k = 0; k < std::min<int64_t>((int64_t)L.size(), cap); ++k) {
+        if (objects) objects[k] = L[(size_t)k].obj;
+        if (prob) prob[k] = L[(size_t)k].prob;
+        if (area) area[k] = L[(size_t)k].area;
+    }
+    return (int64_t)L.size();
 }
 
 int rtb_scene_object(const rtb_scene* scene, int32_t index, rtb_object_info* out) {
@@ -1853,7 +1917,7 @@ int rtb_sample_radiance(rtb_scene* scene, const rtb_params* params, int64_t n, c
             return fail(RTB_EINVAL, "probe item out of range");
     RenderContext* c = acquire_context(scene);
     uint32_t P = (uint32_t)std::min<int64_t>(std::max<int64_t>((n + 31) / 32 * 32, 1024), 1 << 22);
-    uint32_t SP = params->estimator == RTB_EST_NEE ? P : 2 * P;
+    uint32_t SP = shadow_slots(params->estimator, P);
     rc = ensure_context(scene, c, P, SP, (size_t)n);
     RenderArgs a;
     rtb_stats st{};
@@ -1909,7 +1973,7 @@ int rtb_sample_pixels(rtb_scene* scene, const rtb_params* params, int64_t n, con
     RenderContext* c = acquire_context(scene);
     const uint64_t samples = (uint64_t)n * 4ull * (uint64_t)std::max(1, num_samples);
     const uint32_t P = pool_for(samples, params->pool_paths);
-    const uint32_t SP = params->estimator == RTB_EST_NEE ? P : 2 * P;
+    const uint32_t SP = shadow_slots(params->estimator, P);
     rc = ensure_context(scene, c, P, SP, (size_t)n * 4, requested_bin_bits(scene, params) > 0);
     RenderArgs a;
     rtb_stats st{};
@@ -2083,7 +2147,7 @@ void job_worker(rtb_job* j, int worker) {
     uint64_t band_samples = (uint64_t)band_tile_rows * tiles_x * 1024ull * 4ull * (uint64_t)std::max(1, p.spp / 4);
     if (progressive) band_samples = (band_samples + j->passes - 1) / j->passes;
     const uint32_t P = pool_for(band_samples, p.pool_paths);
-    const uint32_t SP = p.estimator == RTB_EST_NEE ? P : 2 * P;
+    const uint32_t SP = shadow_slots(p.estimator, P);
     RenderContext* c = acquire_context(sc, P);
     auto finish = [&](int rc) {
         if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);   // the pinned frame is no longer written by this worker

@@ -1,6 +1,7 @@
 // scene_host.cpp — see scene_host.hpp.  Reference citations are relative to /root/reference.
 #include "scene_host.hpp"
 
+#include <algorithm>
 #include <array>
 #include <cmath>
 #include <cstring>
@@ -418,6 +419,33 @@ int flatten_scene(const HostScene& hs, FlatScene& fs, std::string& err) {
         fs.light_area = (float)L.surface_area;
         for (double c : L.cumulative_area) fs.light_cdf.push_back((float)c);
     }
+    // RTB_EST_NEE_ALL_LIGHTS: every emitting sphere and mesh, weighted by power (light_rule.cuh, DESIGN §3f).  Planes have no
+    // sampler; they and zero-weight emitters stay out and add their emission wherever a path meets them.
+    double total = 0;
+    for (int i = 0; i < fs.n_objects; ++i) {
+        const HostObject& o = hs.objects[i];
+        if (o.geom == GEOM_PLANE) continue;
+        const double lum = 0.2126 * std::max(o.emitted.x, 0.0) + 0.7152 * std::max(o.emitted.y, 0.0) + 0.0722 * std::max(o.emitted.z, 0.0);
+        FlatLight l;
+        l.obj = i;
+        l.area = 0;
+        if (o.geom == GEOM_SPHERE) {
+            l.area = 4.0 * M_PI * o.r * o.r;
+        } else {
+            for (size_t k = 0; k + 2 < o.indices.size(); k += 3) {
+                const D3 a = o.vertices[o.indices[k]], e1 = sub(o.vertices[o.indices[k + 1]], a), e2 = sub(o.vertices[o.indices[k + 2]], a);
+                l.area += 0.5 * len({e1.y * e2.z - e1.z * e2.y, e1.z * e2.x - e1.x * e2.z, e1.x * e2.y - e1.y * e2.x});
+                l.tri_cdf.push_back(l.area);
+            }
+            for (double& c : l.tri_cdf) c /= l.area;
+        }
+        const double w = lum * l.area;
+        if (!(w > 0) || !std::isfinite(w)) continue;
+        l.prob = w;
+        total += w;
+        fs.lights.push_back(std::move(l));
+    }
+    for (FlatLight& l : fs.lights) l.prob /= total;
     (void)err;
     return RTB_OK;
 }

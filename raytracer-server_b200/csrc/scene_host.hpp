@@ -73,6 +73,15 @@ struct FlatMaterial {  // one per object
     int32_t n_tri;
 };
 
+// one entry of the light table: an emitting sphere or mesh with weight w = lum709(max(emitted, 0)) * area > 0, all in f64
+// after the transforms (a mesh's TRUE area, not Mesh::surface_area)
+struct FlatLight {
+    int32_t obj;
+    double prob;                   // w / sum of w
+    double area;
+    std::vector<double> tri_cdf;   // meshes: cumulative triangle areas / area (the last entry is 1)
+};
+
 struct FlatScene {
     float cam_pos[3], cam_dir[3];
     int32_t n_objects = 0;
@@ -86,6 +95,7 @@ struct FlatScene {
     std::vector<float> light_cdf;     // cumulative areas of the UNTRANSFORMED mesh (reference quirk)
     float light_area = 0;
     int32_t n_planes = 0, n_spheres = 0, n_meshes = 0;
+    std::vector<FlatLight> lights;    // RTB_EST_NEE_ALL_LIGHTS: the light table (light_rule.cuh), in object order
 };
 
 int flatten_scene(const HostScene& hs, FlatScene& out, std::string& err);

@@ -15,6 +15,8 @@
 //           block 4 : {brdf u1, u2, lobe}                            dead-MIS own BRDF sample (:203)
 //   dielectric vertex (DESIGN §3e): block 0 only — russian roulette as for a mirror, reflect iff brdf u1 < Fresnel F;
 //                     no light sample, no block 1
+//   RTB_EST_NEE_ALL_LIGHTS (DESIGN §3f): block 1 z = light-table entry, block 1 y = triangle of a mesh light, block 0 light
+//                     u1, u2 = the point; block 1 is drawn for Phong, more than one light or a mesh light
 #pragma once
 
 #include "device_types.cuh"

@@ -22,6 +22,7 @@
 #include "adaptive_rule.cuh"
 #include "dielectric_rule.cuh"
 #include "intersect.cuh"
+#include "light_rule.cuh"
 #include "octree.cuh"
 #include "shade.cuh"
 
@@ -850,6 +851,35 @@ template <int DIR>
 __device__ __forceinline__ uint32_t seg_slot(uint32_t base, uint32_t k) { return base + (uint32_t)(DIR * (int)k); }
 
 // ---------------------------------------------------------------- k_shade
+// RTB_EST_NEE_ALL_LIGHTS: one entry of the light table by power (u = block 1 z), then a point of it — a sphere uniformly over
+// its surface like the reference's sampler, a mesh by a triangle chosen by true area (block 1 y) and a uniform point of that
+// triangle (light_rule.cuh, DESIGN §3f).  Le receives the entry's emission.  An empty table (the scene's only emitters have
+// zero weight) gives a point at unit distance from the shading point x whose weight is 0.
+__device__ __forceinline__ void light_sample_all(const DevScene& S, const SharedScene& sh, const DevSceneHeader* hdr, float4 xi, float pick_u,
+                                                 float3 x, float3& y, float3& ny, float& pdf, float3& Le) {
+    const int n = hdr->n_lights;
+    if (n == 0) {
+        y = x + f3(1.f, 0.f, 0.f);
+        ny = Le = f3(0.f, 0.f, 0.f);
+        pdf = 1.0f;
+        return;
+    }
+    const char* const base = reinterpret_cast<const char*>(hdr);
+    const float* const cdf = reinterpret_cast<const float*>(base + 256 * (size_t)hdr->off_light_cdf);
+    const DevLight L = reinterpret_cast<const DevLight*>(base + 256 * (size_t)hdr->off_lights)[light_pick(cdf, n, pick_u)];
+    const DevMaterial& m = sh.mats[L.obj];
+    Le = f3(m.emitted);
+    if (L.tri_cdf < 0) {
+        light_sample_sphere(L.sphere, L.pdf_area, xi, y, ny, pdf);
+        return;
+    }
+    const float4* tp = S.tri_orig + (size_t)(m.first_tri + light_pick(cdf + L.tri_cdf, m.n_tri, xi.w)) * 3;
+    const float3 a = f3(__ldg(tp)), b = f3(__ldg(tp + 1)), c = f3(__ldg(tp + 2));
+    y = light_tri_point(a, b, c, xi.x, xi.y);
+    ny = light_tri_normal(a, b, c);
+    pdf = L.pdf_area;
+}
+
 // Everything of reflected_radiance except the mesh traversal, as a PERSISTENT kernel of independent warps (no
 // CTA barrier after the table staging).  A lane keeps its path IN REGISTERS from vertex to vertex for as long as
 // the next nearest hit is already final after the analytic pass (the extension ray cannot reach the mesh box):
@@ -868,7 +898,8 @@ __device__ __forceinline__ uint32_t seg_slot(uint32_t base, uint32_t k) { return
 // light, no probe items; 1 = live NEE estimator, 2 = the dead "MIS" branch.  MODE 0, the general instantiation, keeps
 // every branch at run time (both estimators, Phong, mesh lights, rtb_sample_radiance probes).  MODE 3 is MODE 0 plus the
 // dielectric branch (brdf 3, DESIGN §3e): the host runs it for every scene with a dielectric, so that the other
-// instantiations compile exactly as they did before glass existed.
+// instantiations compile exactly as they did before glass existed.  MODE 4 / 5 are MODE 0 / 3 with next-event estimation over
+// the whole light table (RTB_EST_NEE_ALL_LIGHTS, light_rule.cuh, DESIGN §3f): the host runs them for that estimator only.
 constexpr int SHADE_THREADS_NOMESH = 160;   // the mesh-less instantiation needs 96 registers: 4 CTAs of 160 threads = 20 warps per SM
 // The live-NEE instantiations with a mesh (MODE 1, the bench frame's) fit 96 registers without spills too and run the same
 // shape.  The general and dead-MIS ones need 128 (at 96 they spill 140 bytes) and keep 2 CTAs of SHADE_THREADS.  (3 CTAs of
@@ -882,7 +913,8 @@ constexpr int shade_cta(int mode, bool mesh = true) { return !mesh ? SHADE_THREA
 template <int MODE, int NP = 0, int NS = 0, bool MESH = true, int THREADS = SHADE_THREADS, bool INLINE = false>
 __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_MINB : 640 / THREADS) k_shade(const __grid_constant__ RenderArgs a, int c) {
     constexpr bool FAST = MODE == 1 || MODE == 2;
-    constexpr bool DIEL = MODE == 3;
+    constexpr bool DIEL = MODE == 3 || MODE == 5;
+    constexpr bool ALL = MODE == 4 || MODE == 5;   // RTB_EST_NEE_ALL_LIGHTS
     extern __shared__ __align__(16) unsigned char smem_raw[];
     DevCtrl* C = a.ctrl;
     const DevSceneHeader* hdr = a.S.hdr;
@@ -895,12 +927,13 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
     const PathQueue &Q = a.qin, &N = a.qout;
     const int light_obj = hdr->light_obj;
     const bool light_is_mesh = FAST ? false : hdr->light_geom == 2;
-    const bool mis = MODE == 1 ? false : (MODE == 2 ? true : a.estimator == 1);     // the reference's dead "MIS" branch
+    const bool select_b1 = ALL ? hdr->lights_select != 0 : light_is_mesh;   // a non-Phong vertex draws block 1 for its light choice
+    const bool mis = MODE == 1 || ALL ? false : (MODE == 2 ? true : a.estimator == 1);     // the reference's dead "MIS" branch
     // RTB_EST_MIS_BALANCE (general instantiation only): next-event estimation and the BRDF sample combined with the balance
     // heuristic — what src/scene.rs:187 ("TODO: Do multiple importance sampling properly") asks for.  Diffuse surfaces under
     // a sphere light; Phong surfaces keep plain NEE (the reference's Phong sampler never leaves the local frame, its pdf
     // for a world direction is undefined).  Never used for parity.
-    const bool mis2 = FAST ? false : a.estimator == 2;
+    const bool mis2 = FAST || ALL ? false : a.estimator == 2;
     const bool probe_mode = FAST ? false : a.probe_px != nullptr;
     const float3 Le = f3(sh.mats[light_obj].emitted);
     const int n_prims = a.S.n_prims, n_planes = a.S.n_planes;
@@ -1048,6 +1081,10 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                     } else {
                         beta = beta * f3(pm.k) * inv_pp;
                     }
+                } else if constexpr (ALL) {
+                    // behind a diffuse or Phong vertex: its light sample has counted the emitters of the table, not the others
+                    if (emits && reinterpret_cast<const int32_t*>(reinterpret_cast<const char*>(hdr) + 256 * (size_t)hdr->off_light_of)[hg.obj] < 0)
+                        accum_add(a.accum, acc, beta * emitted);
                 }
                 const float p = depth <= 5u ? 1.0f : 0.9f;  // MAX_BOUNCES / SURVIVAL_PROBABILITY (src/scene.rs:109-110,164-168)
                 const float inv_p = depth <= 5u ? 1.0f : (1.0f / 0.9f);
@@ -1059,10 +1096,12 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                     const VertexRng vr = rng_vertex(rng_pixel, sample, depth, a.keys);
                     // lobe / light-triangle selectors live in block 1 and are only drawn by Phong surfaces / mesh lights
                     float lobe_u = 0.f, select_u = 0.f;
-                    if (!FAST && (mat.brdf == 2 || light_is_mesh) && !(DIEL && mat.brdf == 3)) {
+                    float pick_u = 0.f;
+                    if (!FAST && (mat.brdf == 2 || select_b1) && !(DIEL && mat.brdf == 3)) {
                         const float4 r1 = rng_block(rng_pixel, sample, depth, 1u, a.keys);
                         lobe_u = r1.x;
                         select_u = r1.y;
+                        if constexpr (ALL) pick_u = r1.z;   // which entry of the light table
                     }
                     const float4 r0 = make_float4(vr.light_u1, vr.light_u2, vr.rr, select_u);
                     const float4 rb = make_float4(vr.brdf_u1, vr.brdf_u2, lobe_u, 0.f);
@@ -1093,9 +1132,10 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                         }
                     } else {
                         // ---- direct light
-                        float3 y, ny;
+                        float3 y, ny, Le_y;   // Le_y: the sampled light's emission (ALL)
                         float pdf_a;
                         if (FAST) light_sample_sphere(a.light_sphere, a.light_pdf, r0, y, ny, pdf_a);
+                        else if (ALL) light_sample_all(a.S, sh, hdr, r0, pick_u, hg.pos, y, ny, pdf_a, Le_y);
                         else light_sample<FAST>(a.S, sh.prims, hdr, r0, y, ny, pdf_a);
                         float3 dv = y - hg.pos;
                         float r2 = dot(dv, dv);
@@ -1105,8 +1145,8 @@ __global__ void __launch_bounds__(THREADS, THREADS == SHADE_THREADS ? RTB_SHADE_
                         float3 f = brdf_eval<FAST>(mat, hg.n, ovec, inc);
                         float3 contrib;
                         if (!mis) {  // live NEE, src/scene.rs:217-229 (no cosine is clamped)
-                            float g = __fdividef(dot(hg.n, inc) * dot(ny, -inc), r2 * pdf_a);
-                            contrib = beta * Le * f * g;
+                            float g = ALL ? light_weight(hg.n, ny, inc, r2, pdf_a) : __fdividef(dot(hg.n, inc) * dot(ny, -inc), r2 * pdf_a);
+                            contrib = beta * (ALL ? Le_y : Le) * f * g;
                             if (mis2 && mat.brdf == 0) {   // balance weight of the light sample: pdf_light / (pdf_light + pdf_brdf(inc))
                                 const float pdf_l = pdf_a * r2 / fmaxf(fabsf(dot(ny, -inc)), 1e-20f);
                                 const float pdf_b = fmaxf(dot(hg.n, inc), 0.f) * INV_PI_F;

@@ -13,7 +13,7 @@ import threading
 import numpy as np
 
 from . import _abi
-from ._abi import ACCEL_LBVH, ACCEL_OCTREE_REFERENCE, EST_MIS_BALANCE, EST_MIS_DEAD, EST_NEE, Adaptive, Denoise, ObjectDesc, ObjectInfo, Params, SceneDesc, SceneInfo, Stats
+from ._abi import ACCEL_LBVH, ACCEL_OCTREE_REFERENCE, EST_MIS_BALANCE, EST_MIS_DEAD, EST_NEE, EST_NEE_ALL_LIGHTS, Adaptive, Denoise, ObjectDesc, ObjectInfo, Params, SceneDesc, SceneInfo, Stats
 
 
 class RtbError(RuntimeError):
@@ -210,6 +210,16 @@ class Scene:
             _abi.lib().rtb_scene_triangles(self._h, out.ctypes.data_as(C.POINTER(C.c_float)), n)
         return out
 
+    def lights(self) -> dict:
+        """The light table of EST_NEE_ALL_LIGHTS (rtb_scene_lights): object index int32 [n], selection probability and area
+        float64 [n], in object order."""
+        L = _abi.lib()
+        n = _check(int(L.rtb_scene_lights(self._h, None, None, None, 0)))
+        obj, prob, area = np.zeros(n, np.int32), np.zeros(n, np.float64), np.zeros(n, np.float64)
+        dp = C.POINTER(C.c_double)
+        L.rtb_scene_lights(self._h, obj.ctypes.data_as(C.POINTER(C.c_int32)), prob.ctypes.data_as(dp), area.ctypes.data_as(dp), n)
+        return {"objects": obj, "prob": prob, "area": area}
+
     def octree_stats(self, index: int) -> dict:
         """Octree::build for mesh object `index` on the host (what ACCEL_OCTREE_REFERENCE traverses)."""
         c = (C.c_int64 * 4)()
@@ -328,10 +338,10 @@ class Scene:
 
 
 def sample_pixels(xs, ys_screen, width: int, height: int, samples_per_pixel: int, scene: Scene, *, seed: int = 0,
-                  use_mis: bool = False) -> np.ndarray:
+                  use_mis: bool = False, estimator: int | None = None) -> np.ndarray:
     """sample_pixel for a batch of pixels (x, screen row y; rtb_sample_pixels): float32 [n, 3], the Vec3 of
     src/server.rs:363 per pixel (0..255.5; `as u8` truncates it to the frame's bytes)."""
-    p = make_params(width, height, samples_per_pixel, use_mis=use_mis, seed=seed)
+    p = make_params(width, height, samples_per_pixel, use_mis=use_mis, seed=seed, estimator=estimator)
     px = np.ascontiguousarray(xs, dtype=np.int32).reshape(-1)
     py = np.ascontiguousarray(ys_screen, dtype=np.int32).reshape(-1)
     assert px.size == py.size
@@ -356,13 +366,16 @@ class RenderJob:
     PIXELS_PER_MSG = 60
 
     def __init__(self, scene: Scene, width: int, height: int, samples_per_pixel: int, *, passes: int = 1, seed: int = 0,
-                 use_mis: bool = False, pool_paths: int = 0, accel: int = 0, adaptive: dict | None = None, denoise=None):
+                 use_mis: bool = False, pool_paths: int = 0, accel: int = 0, adaptive: dict | None = None, denoise=None,
+                 estimator: int | None = None):
         """adaptive: dict(target_levels=..., pass_spp=16, min_spp=None) makes this an adaptive job (rtb_job_begin_adaptive):
         samples_per_pixel is the budget, `passes` is ignored and the job re-sends the frame once per pass until every tile
         has converged.  denoise (True / dict of make_denoise keywords / Denoise): every frame the job sends is denoised
-        (rtb_job_begin_denoised); a single-pass job then renders the frame as one band."""
+        (rtb_job_begin_denoised); a single-pass job then renders the frame as one band.  estimator: an EST_* constant
+        (None = EST_MIS_DEAD if use_mis else EST_NEE)."""
         self.scene = scene
-        self.params = make_params(width, height, samples_per_pixel, use_mis=use_mis, seed=seed, pool_paths=pool_paths, accel=accel)
+        self.params = make_params(width, height, samples_per_pixel, use_mis=use_mis, seed=seed, pool_paths=pool_paths, accel=accel,
+                                  estimator=estimator)
         self._h = C.c_void_p()
         # guards the handle: stop() may come from another thread (the server's event loop) while close() frees the job
         self._lock = threading.Lock()

@@ -9,7 +9,8 @@ Protocol (reference `src/server.rs`):
     for adaptive sampling instead — every 32x32 tile stops once its estimated standard error is at most that many 8-bit
     output levels, with "spp" as the budget (rounded down to a multiple of ADAPTIVE_PASS_SPP), and every record is
     re-sent once per pass until all tiles have stopped; "denoise": true sends every frame of the job (either kind, or a
-    plain one) through the edge-aware denoiser.
+    plain one) through the edge-aware denoiser; "all_lights": true lights the scene with every emitting sphere and mesh
+    (EST_NEE_ALL_LIGHTS) instead of the first emitter alone.
   * server -> client, binary, one message per <= 60 pixels of one screen row (:173-190):
         [0] = 0 (message type)   [1] = n   [2..4] = x u16le   [4..6] = y u16le (row 0 = top)   then n x (r, g, b)
     There is no "done" message; the client counts pixels (test-client/app.tsx:69-70).
@@ -45,16 +46,16 @@ ADAPTIVE_MIN_SPP = 64                                      # ... and the least a
 def default_job_factory(scenes: dict, width: int, height: int, accel: int = 0):
     """accel: 0 = LBVH (true nearest hit, the fast path), 1 = the reference's own octrees (ACCEL_OCTREE_REFERENCE: the image the
     Rust binary sends, non-nearest triangles included; 2.4 x slower on flying_unicorn).  `main` reads it from $RTB_ACCEL."""
-    from .host import RenderJob
+    from .host import EST_NEE_ALL_LIGHTS, RenderJob
 
-    def make(scene_name: str, spp: int, passes: int = 1, adaptive: dict | None = None, denoise: bool = False):
+    def make(scene_name: str, spp: int, passes: int = 1, adaptive: dict | None = None, denoise: bool = False, all_lights: bool = False):
         scene = scenes.get(scene_name)
         if scene is None:
             return None
         # spp is an i32 in the reference (`ClientMessage::Render`, :123); `num_samples = spp / 4` makes every spp < 4,
         # negative ones included, an empty sample loop: a black frame is streamed (src/server.rs:332-362)
         return RenderJob(scene, width, height, max(0, spp), passes=passes, seed=random.getrandbits(63), accel=accel,
-                         adaptive=adaptive, denoise=True if denoise else None)
+                         adaptive=adaptive, denoise=True if denoise else None, estimator=EST_NEE_ALL_LIGHTS if all_lights else None)
 
     return make
 
@@ -96,10 +97,10 @@ class Server:
                     try:
                         scene_name, spp, passes = req["scene"], req["spp"], req.get("passes", 1)
                         # serde: `scene: String`, `spp: i32` — a JSON string / float / bool / out-of-range number is a parse error
-                        denoise = req.get("denoise", False)
+                        denoise, all_lights = req.get("denoise", False), req.get("all_lights", False)
                         if not isinstance(scene_name, str) or type(spp) is not int or not -2 ** 31 <= spp < 2 ** 31 or type(passes) is not int:
                             raise TypeError
-                        if type(denoise) is not bool:
+                        if type(denoise) is not bool or type(all_lights) is not bool:
                             raise TypeError
                         passes = max(1, passes)
                         adaptive = self._adaptive_options(req["noise"], spp) if "noise" in req else None
@@ -107,7 +108,9 @@ class Server:
                         await websocket.close(code=1007, reason="failed to parse message")
                         break
                     try:
-                        kw = {"denoise": True} if denoise else {}   # without the field the factory is called as before
+                        kw = {"denoise": True} if denoise else {}   # without the fields the factory is called as before
+                        if all_lights:
+                            kw["all_lights"] = True
                         if adaptive is not None:
                             budget, opts = adaptive
                             job = self.job_factory(scene_name, budget, 1, adaptive=opts, **kw)
