@@ -107,13 +107,14 @@ typedef struct rtb_scene_info {
 
 /* one object as the loader built it (f64, after transforms) — Object / Geometry, src/scene.rs:10-15 */
 typedef struct rtb_object_info {
-    int32_t brdf;          /* 0 diffuse, 1 specular, 2 phong, 3 dielectric */
+    int32_t brdf;          /* 0 diffuse, 1 specular, 2 phong, 3 dielectric, 4 metal */
     int32_t geometry;      /* 0 sphere, 1 plane, 2 mesh (cube / prism / OBJ) */
     int32_t n_triangles;
     int32_t first_triangle; /* global triangle index of the mesh's first triangle, or -1 */
     double emitted[3];
     double k[3];           /* kd | ks | phong {kd, ks, power} | dielectric {ior, orientation sign, 0}: the sign is +1 when the
-                              stored normals point out of the medium (sphere: radial, plane: n, mesh: see rtb_object_desc) */
+                              stored normals point out of the medium (sphere: radial, plane: n, mesh: see rtb_object_desc) |
+                              metal {roughness, GGX alpha = roughness^2, 0}, color_s = F0 */
     double color_d[3];
     double color_s[3];
     double pos[3];
@@ -170,7 +171,11 @@ typedef struct rtb_object_desc {
                                plane's n points to, and for a mesh the outside of the solid it bounds: the loader winds
                                each connected piece consistently and orients it by its signed volume (f64), and keeps
                                the stored normal norm((c-a) x (b-a)) of the first triangle, turning triangles wound
-                               against it around (b <-> c).  Meant for closed meshes; an open one gets an arbitrary side. */
+                               against it around (b <-> c).  Meant for closed meshes; an open one gets an arbitrary side.
+                               4 metal {k = roughness, 0, 0 (finite, in [0.05, 1]); color_s = F0, the reflectance at
+                               normal incidence, each in [0, 1]}: GGX microfacet reflection with alpha = roughness^2, the
+                               height-correlated Smith masking and Schlick's Fresnel term (DESIGN §3g).  Not available
+                               under RTB_EST_MIS_DEAD (RTB_EUNSUPPORTED). */
     int32_t geometry;       /* 0 sphere, 1 plane, 2 mesh */
     double k[3];
     double color_d[3];

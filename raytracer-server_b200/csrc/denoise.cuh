@@ -18,7 +18,7 @@ constexpr int DENOISE_THREADS = 256;
 // of a chain reflects the camera ray's -d).  Per ray: the first non-specular hit's object, facing normal, path length and
 // albedo (times ks of every mirror on the way); an emitter, a miss or an unfinished chain has albedo 1.  Per pixel:
 // A dielectric counts as a specular vertex: the ray follows the refracted direction (the reflected one under total internal
-// reflection) and the albedo takes the tint on transmission.
+// reflection) and the albedo takes the tint on transmission.  A rough metal (brdf 4) is a non-specular first hit of albedo F0.
 // ga = (mean albedo, mean depth over the rays that hit), gn = (renormalised sum of the normals, the object most rays hit,
 // ties to the lowest sub-pixel; -1 = miss).
 __global__ void __launch_bounds__(WF_THREADS) k_gbuffer(DevScene S, const Camera cam, int width, int height, int accel,
@@ -75,7 +75,8 @@ __global__ void __launch_bounds__(WF_THREADS) k_gbuffer(DevScene S, const Camera
                     continue;
                 }
                 const bool emits = m.emitted.x != 0.f || m.emitted.y != 0.f || m.emitted.z != 0.f;
-                if (m.brdf != 1 && m.brdf != 3 && !emits)
+                if (m.brdf == 4 && !emits) a = thr * f3(m.color_s);   // rough metal: F0
+                else if (m.brdf != 1 && m.brdf != 3 && !emits)
                     a = thr * (m.brdf == 0 ? f3(m.k) : f3(m.color_d) * m.k.x + f3(m.color_s) * m.k.y);
                 nrm = nrm + hg.n;
                 depth += path;

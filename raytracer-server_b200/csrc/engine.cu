@@ -553,6 +553,8 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
         CU_TRY(cudaFuncSetAttribute(k_shade<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_shade<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_shade<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        CU_TRY(cudaFuncSetAttribute(k_shade_metal<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        CU_TRY(cudaFuncSetAttribute(k_shade_metal<7>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaFuncSetAttribute(k_generate<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         const int smem_tail = (int)shared_scene_bytes(MAX_OBJECTS, MAX_OBJECTS, SHADE_THREADS);
         const int smem_tail_nee = (int)shared_scene_bytes(MAX_OBJECTS, MAX_OBJECTS, SHADE_THREADS_NEE);
@@ -562,6 +564,8 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
         CU_TRY(cudaFuncSetAttribute(k_shade<3, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         CU_TRY(cudaFuncSetAttribute(k_shade<4, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         CU_TRY(cudaFuncSetAttribute(k_shade<5, 0, 0, true, SHADE_THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
+        CU_TRY(cudaFuncSetAttribute(k_shade_metal<6, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
+        CU_TRY(cudaFuncSetAttribute(k_shade_metal<7, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_tail));
         int b = 0;
         CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_traverse<false>, WF_THREADS, smem_stack));
         c->grid_ext = std::max(1, b) * prop.multiProcessorCount;
@@ -582,7 +586,7 @@ int ensure_context(rtb_scene* sc, RenderContext* c, uint32_t P, uint32_t SP, siz
         };
         if (int e = shade_grid({(const void*)k_shade<0>, (const void*)k_shade<2>, (const void*)k_shade<2, 8, 0>, (const void*)k_shade<2, 5, 1>,
                                 (const void*)k_shade<2, 5, 2>, (const void*)k_shade<2, 5, 3>, (const void*)k_shade<3>, (const void*)k_shade<4>,
-                                (const void*)k_shade<5>}, SHADE_THREADS, c->grid_shade)) return e;
+                                (const void*)k_shade<5>, (const void*)k_shade_metal<6>, (const void*)k_shade_metal<7>}, SHADE_THREADS, c->grid_shade)) return e;
         if (int e = shade_grid({(const void*)k_shade<1, 0, 0, true, SHADE_THREADS_NEE>, (const void*)k_shade<1, 8, 0, true, SHADE_THREADS_NEE>,
                                 (const void*)k_shade<1, 5, 1, true, SHADE_THREADS_NEE>, (const void*)k_shade<1, 5, 2, true, SHADE_THREADS_NEE>,
                                 (const void*)k_shade<1, 5, 3, true, SHADE_THREADS_NEE>}, SHADE_THREADS_NEE, c->grid_shade_nee)) return e;
@@ -835,6 +839,8 @@ static void launch_shade(int mode, int n_planes, int n_spheres, int grid, size_t
         else if (mode == 3) k_shade<3, 0, 0, true, shade_cta(3), true><<<grid, shade_cta(3), smem_t, st>>>(a, cur);
         else if (mode == 4) k_shade<4, 0, 0, true, shade_cta(4), true><<<grid, shade_cta(4), smem_t, st>>>(a, cur);
         else if (mode == 5) k_shade<5, 0, 0, true, shade_cta(5), true><<<grid, shade_cta(5), smem_t, st>>>(a, cur);
+        else if (mode == 6) k_shade_metal<6, true><<<grid, SHADE_THREADS, smem_t, st>>>(a, cur);
+        else if (mode == 7) k_shade_metal<7, true><<<grid, SHADE_THREADS, smem_t, st>>>(a, cur);
         else k_shade<0, 0, 0, true, shade_cta(0), true><<<grid, shade_cta(0), smem_t, st>>>(a, cur);
         return;
     }
@@ -854,6 +860,8 @@ static void launch_shade(int mode, int n_planes, int n_spheres, int grid, size_t
     else if (mode == 3) RTB_SHADE(3, 0, 0);
     else if (mode == 4) RTB_SHADE(4, 0, 0);
     else if (mode == 5) RTB_SHADE(5, 0, 0);
+    else if (mode == 6) k_shade_metal<6><<<grid, SHADE_THREADS, smem, st>>>(a, cur);
+    else if (mode == 7) k_shade_metal<7><<<grid, SHADE_THREADS, smem, st>>>(a, cur);
     else RTB_SHADE(0, 0, 0);
 #undef RTB_SHADE
 }
@@ -890,13 +898,17 @@ int run_wavefront(rtb_scene* sc, RenderContext* c, RenderArgs& a, uint32_t ks_be
     if (a.estimator == RTB_EST_MIS_BALANCE && sc->fs.light_geom != GEOM_SPHERE)
         return fail(RTB_EUNSUPPORTED, "RTB_EST_MIS_BALANCE needs a sphere light (the reference's mesh-light sampler does not return points of the mesh, src/geometry.rs:622-628)");
     // a scene with a dielectric always runs the general kernel with the dielectric branch (MODE 3), probes included
-    bool dielectric = false;
+    bool dielectric = false, metal = false;
     for (const FlatMaterial& m : sc->fs.materials) dielectric = dielectric || m.brdf == BRDF_DIELECTRIC;
+    for (const FlatMaterial& m : sc->fs.materials) metal = metal || m.brdf == BRDF_METAL;
+    if (metal && a.estimator == RTB_EST_MIS_DEAD)
+        return fail(RTB_EUNSUPPORTED, "RTB_EST_MIS_DEAD is the reference's dead branch and has no meaning for a rough metal (brdf 4), which the reference lacks");
     bool fast_shade = !a.probe_px && a.estimator != RTB_EST_MIS_BALANCE && sc->fs.light_geom == GEOM_SPHERE && !getenv("RTB_NO_FAST_SHADE");
-    for (const FlatMaterial& m : sc->fs.materials) fast_shade = fast_shade && m.brdf != BRDF_PHONG;
+    for (const FlatMaterial& m : sc->fs.materials) fast_shade = fast_shade && m.brdf != BRDF_PHONG && m.brdf != BRDF_METAL;
     // RTB_EST_NEE_ALL_LIGHTS: the general kernel with next-event estimation over the whole light table (MODE 4), or MODE 3's
-    // dielectric kernel with it (MODE 5), probes included
-    const int shade_mode = a.estimator == RTB_EST_NEE_ALL_LIGHTS ? (dielectric ? 5 : 4)
+    // dielectric kernel with it (MODE 5), probes included.  A scene with a metal runs MODE 3 / 5 plus the metal branch (MODE 6 / 7).
+    const int shade_mode = metal ? (a.estimator == RTB_EST_NEE_ALL_LIGHTS ? 7 : 6)
+                         : a.estimator == RTB_EST_NEE_ALL_LIGHTS ? (dielectric ? 5 : 4)
                                                                  : (dielectric ? 3 : (!fast_shade ? 0 : (a.estimator == 0 ? 1 : 2)));
     // the CTA shape of k_shade depends on the instantiation: so do its grid and warp count (static first chunks, k_prepare)
     const bool nomesh = shade_is_nomesh(shade_mode, a);
@@ -1376,7 +1388,7 @@ int rtb_scene_create(const rtb_scene_desc* desc, int device, rtb_scene** out) {
         const rtb_object_desc& d = desc->objects[i];
         HostObject o;
         o.emitted = {d.emitted[0], d.emitted[1], d.emitted[2]};
-        if (d.brdf < 0 || d.brdf > 3 || d.geometry < 0 || d.geometry > 2) { rc = RTB_EPARSE; err = "object " + std::to_string(i) + ": unknown brdf / geometry kind"; break; }
+        if (d.brdf < 0 || d.brdf > 4 || d.geometry < 0 || d.geometry > 2) { rc = RTB_EPARSE; err = "object " + std::to_string(i) + ": unknown brdf / geometry kind"; break; }
         o.brdf = d.brdf;
         if (d.brdf == BRDF_PHONG) {
             if (d.k[2] < 0) { rc = RTB_EPARSE; err = "phong power must be >= 0"; break; }
@@ -1390,6 +1402,13 @@ int rtb_scene_create(const rtb_scene_desc* desc, int device, rtb_scene** out) {
             if (!tint_ok) { rc = RTB_EPARSE; err = "object " + std::to_string(i) + ": dielectric tint (color_d) components must lie in [0, 1]"; break; }
             o.k = {d.k[0], 0, 0};
             o.color_d = {d.color_d[0], d.color_d[1], d.color_d[2]};
+        } else if (d.brdf == BRDF_METAL) {
+            if (!std::isfinite(d.k[0]) || !(d.k[0] >= METAL_MIN_ROUGHNESS && d.k[0] <= 1)) { rc = RTB_EPARSE; err = "object " + std::to_string(i) + ": metal roughness (k[0]) must be a finite number in [0.05, 1]"; break; }
+            bool f0_ok = true;
+            for (int c = 0; c < 3; ++c) f0_ok = f0_ok && d.color_s[c] >= 0 && d.color_s[c] <= 1;
+            if (!f0_ok) { rc = RTB_EPARSE; err = "object " + std::to_string(i) + ": metal color (color_s, F0) components must lie in [0, 1]"; break; }
+            o.k = {d.k[0], 0, 0};
+            o.color_s = {d.color_s[0], d.color_s[1], d.color_s[2]};
         } else {
             o.k = {d.k[0], d.k[1], d.k[2]};
         }
@@ -1595,6 +1614,9 @@ int rtb_scene_object(const rtb_scene* scene, int32_t index, rtb_object_info* out
     } else if (o.brdf == BRDF_DIELECTRIC) {
         out->k[0] = o.k.x; out->k[1] = scene->fs.materials[index].k[1];   // ior, orientation sign
         out->color_d[0] = o.color_d.x; out->color_d[1] = o.color_d.y; out->color_d[2] = o.color_d.z;
+    } else if (o.brdf == BRDF_METAL) {
+        out->k[0] = o.k.x; out->k[1] = o.k.x * o.k.x;   // roughness, GGX alpha
+        out->color_s[0] = o.color_s.x; out->color_s[1] = o.color_s.y; out->color_s[2] = o.color_s.z;
     } else {
         out->k[0] = o.k.x; out->k[1] = o.k.y; out->k[2] = o.k.z;
     }

@@ -209,8 +209,19 @@ void build_object(const Value& spec, const std::string& assets_dir, HostObject& 
             for (double c : {o.color_d.x, o.color_d.y, o.color_d.z})
                 if (!(c >= 0 && c <= 1)) bad("dielectric tint components must lie in [0, 1]");
         }
+    } else if (bt == "metal") {
+        o.brdf = BRDF_METAL;
+        const double rough = num(need(b, "roughness", "brdf"), "roughness");
+        if (!std::isfinite(rough) || !(rough >= METAL_MIN_ROUGHNESS && rough <= 1)) bad("metal roughness must be a finite number in [0.05, 1]");
+        o.k = {rough, 0, 0};
+        o.color_s = {1, 1, 1};
+        if (const Value* c = b.find("color")) {
+            o.color_s = vec3(*c, "color");
+            for (double v : {o.color_s.x, o.color_s.y, o.color_s.z})
+                if (!(v >= 0 && v <= 1)) bad("metal color components must lie in [0, 1]");
+        }
     } else {
-        bad("unknown variant `" + bt + "`, expected one of `diffuse`, `specular`, `phong`, `dielectric`");
+        bad("unknown variant `" + bt + "`, expected one of `diffuse`, `specular`, `phong`, `dielectric`, `metal`");
     }
     const Value& g = need(spec, "geometry", "object");
     if (g.kind != Value::Table) bad("geometry must be a table");
@@ -336,6 +347,9 @@ int flatten_scene(const HostScene& hs, FlatScene& fs, std::string& err) {
             m.k[0] = (float)o.k.x;
             m.k[1] = 1.0f;   // spheres and planes; meshes below
             m.color_d[0] = (float)o.color_d.x; m.color_d[1] = (float)o.color_d.y; m.color_d[2] = (float)o.color_d.z;
+        } else if (o.brdf == BRDF_METAL) {   // microfacet_rule.cuh: k.x = GGX alpha, color_s = F0
+            m.k[0] = (float)(o.k.x * o.k.x);
+            m.color_s[0] = (float)o.color_s.x; m.color_s[1] = (float)o.color_s.y; m.color_s[2] = (float)o.color_s.z;
         } else {
             m.k[0] = (float)o.k.x; m.k[1] = (float)o.k.y; m.k[2] = (float)o.k.z;
         }

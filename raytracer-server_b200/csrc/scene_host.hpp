@@ -17,15 +17,16 @@ struct D3 {
 };
 
 enum GeomKind : int { GEOM_SPHERE = 0, GEOM_PLANE = 1, GEOM_MESH = 2 };
-enum BrdfKind : int { BRDF_DIFFUSE = 0, BRDF_SPECULAR = 1, BRDF_PHONG = 2, BRDF_DIELECTRIC = 3 };
+enum BrdfKind : int { BRDF_DIFFUSE = 0, BRDF_SPECULAR = 1, BRDF_PHONG = 2, BRDF_DIELECTRIC = 3, BRDF_METAL = 4 };
+constexpr double METAL_MIN_ROUGHNESS = 0.05;   // rough metal: roughness in [0.05, 1], GGX alpha = roughness^2
 
 struct HostObject {
     D3 emitted;
     int brdf = BRDF_DIFFUSE;
-    D3 k;                      // kd (diffuse) / ks (specular) / {ior, 0, 0} (dielectric)
+    D3 k;                      // kd (diffuse) / ks (specular) / {ior, 0, 0} (dielectric) / {roughness, 0, 0} (metal)
     double phong_kd = 0, phong_ks = 0;
     int phong_power = 0;
-    D3 color_d, color_s;       // phong colours; dielectric: color_d = transmission tint
+    D3 color_d, color_s;       // phong colours; dielectric: color_d = transmission tint; metal: color_s = F0
     int geom = GEOM_SPHERE;
     D3 pos;                    // sphere centre / plane point
     double r = 0;
@@ -64,9 +65,9 @@ struct FlatPrim {      // analytic primitive, in object order
 
 struct FlatMaterial {  // one per object
     float emitted[4];  // rgb, -
-    float k[4];        // diffuse kd / specular ks rgb; phong: kd, ks, power, -; dielectric: ior, orientation sign, -
+    float k[4];        // diffuse kd / specular ks rgb; phong: kd, ks, power, -; dielectric: ior, orientation sign, -; metal: alpha, -, -
     float color_d[4];  // phong colour_d; dielectric: tint
-    float color_s[4];
+    float color_s[4];  // phong colour_s; metal: F0
     int32_t brdf;
     int32_t geom;
     int32_t first_tri;  // meshes: first global triangle index, else -1

@@ -17,6 +17,8 @@
 //                     no light sample, no block 1
 //   RTB_EST_NEE_ALL_LIGHTS (DESIGN §3f): block 1 z = light-table entry, block 1 y = triangle of a mesh light, block 0 light
 //                     u1, u2 = the point; block 1 is drawn for Phong, more than one light or a mesh light
+//   metal vertex (DESIGN §3g): block 0 only — light u1, u2, russian roulette as for a diffuse vertex, brdf u1, u2 = the visible
+//                     normal; block 1 only where a diffuse vertex would draw it for its light sample
 #pragma once
 
 #include "device_types.cuh"

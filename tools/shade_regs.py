@@ -11,6 +11,7 @@ import os, re, shutil, subprocess, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OBJ = os.path.join(ROOT, "raytracer-server_b200", "build", "engine.o")
 KERNELS = ("k_shade<", "k_traverse<", "k_generate<")
+METAL_KERNELS = ("k_shade_metal<",)   # k_shade's MODE 6 / 7 for scenes with a rough metal, a kernel of their own
 CUOBJDUMP = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
 WIDTH = {"U8": 1, "S8": 1, "U16": 2, "S16": 2, "64": 8, "128": 16}
 
@@ -51,21 +52,23 @@ def local_bytes(obj):
     return acc
 
 
-def table(obj=OBJ):
-    """[(kernel, registers, stack bytes, spill store bytes, spill load bytes)], sorted by kernel"""
+def table(obj=OBJ, kernels=KERNELS):
+    """[(kernel, registers, stack bytes, spill store bytes, spill load bytes)] of the kernels whose names start with one of
+    `kernels`, sorted by kernel"""
     usage, spills = resource_usage(obj), local_bytes(obj)
     names = demangle(list(usage))
     rows = []
     for fn, (reg, stack) in usage.items():
         name = names[fn].replace("rtb::", "").removeprefix("void ").split("(")[0]
-        if name.startswith(KERNELS):
+        if name.startswith(kernels):
             st, ld = spills.get(fn, (0, 0))
             rows.append((name, reg, stack, st, ld))
     return sorted(rows)
 
 
 def main():
-    rows = table(sys.argv[1] if len(sys.argv) > 1 else OBJ)
+    obj = sys.argv[1] if len(sys.argv) > 1 else OBJ
+    rows = table(obj) + table(obj, METAL_KERNELS)
     w = max(len(r[0]) for r in rows)
     print(f"{'kernel':<{w}}  {'regs':>4}  {'stack':>5}  {'spill st':>8}  {'spill ld':>8}")
     for name, reg, stack, st, ld in rows:
